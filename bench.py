@@ -7,6 +7,7 @@ per-kernel tensor-core / HBM roofline of the dominant CRF kernel and the host-CP
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --steps K --warmup W     # the reference's CPU path (oracle port), host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR   # also write what the timed step computes (.npy)
 
 A "step" is one iteration of the reference training loop (src/train.py:86-114): forward, SSIM + 0.1 L1 loss,
 backward, Adam.  Data is synthetic (rand image / depth of NYU shape), weights are random-init (no network).
@@ -82,7 +83,16 @@ def parse_args():
                     help="N>1: exchange the gradient buckets in bf16 (90 MB instead of 180 MB per step); off by default")
     ap.add_argument("--memory-format", default="channels_last", choices=["contiguous", "channels_last"],
                     help="memory format of the model and the images (host-side choice; math is identical)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed regions, run the timed step twice from the seeded initial model and "
+                         "optimizer state and write its losses and first gradients to DIR/<name>.npy (dump_outputs), "
+                         "so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def load_peaks():
@@ -140,6 +150,46 @@ class ClockSampler:
             except Exception:
                 pass
         return out
+
+
+DUMP_SAMPLE = 1 << 20   # elements of the gradient sample: 4 MB in float32
+
+
+def reset_state(model, optimizer, state0):
+    """Put the model back into `state0` (a clone of its state_dict) and the optimizer into the state a fresh Adam starts
+    from (moments and step counters at zero), in place: a captured CUDA graph keeps reading the same tensors."""
+    import torch
+    with torch.no_grad():
+        for k, t in model.state_dict().items():
+            t.copy_(state0[k])
+        for st in optimizer.state.values():
+            for t in st.values():
+                if torch.is_tensor(t):
+                    t.zero_()
+
+
+def grad_sample(model):
+    """A fixed sample (seeded, DUMP_SAMPLE elements) of the model's gradients, float32 on the host, flattened in
+    model.named_parameters() order and in logical element order, so it does not depend on the memory format."""
+    import numpy as np
+    import torch
+    params = [p for _, p in model.named_parameters() if p.requires_grad]
+    n = sum(p.numel() for p in params)
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    flat = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1) for p in params])
+    return flat[torch.from_numpy(idx).to(flat.device)].float().cpu().numpy()
+
+
+def dump_outputs(out_dir, losses, grads):
+    """`loss.npy`: the losses train_step returned (float64), `grads.npy`: a grad_sample (float32).
+
+    Two runs of the same build (`--steps 10 --warmup 3`, B200 at its 1000 W power limit) agreed to rel 6e-7 in the
+    losses and rel-L2 1.7e-3 in the gradient sample (every element within rtol 1e-2, atol 1e-6): the bf16 path's
+    rounding under a varying summation order."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array(losses, dtype=np.float64))
+    np.save(os.path.join(out_dir, "grads.npy"), grads)
 
 
 # --------------------------------------------------------------------------------------------------------------
@@ -249,6 +299,8 @@ def run_ours(args):
         opt = LibAdam([p for p in model.parameters() if p.requires_grad], 1e-4)
     else:
         opt = torch.optim.Adam(model.parameters(), 1e-4, fused=True, capturable=use_graph)
+    # --dump-outputs: the state the dumped steps start from (taken after DDP gave every rank rank 0's parameters)
+    state0 = {k: t.detach().clone() for k, t in model.state_dict().items()} if args.dump_outputs else None
 
     image_h = torch.rand(B, 3, H, W).contiguous(memory_format=mf).pin_memory()
     depth_h = torch.rand(B, 1, H, W).pin_memory()
@@ -307,11 +359,13 @@ def run_ours(args):
             graph = None
             torch.cuda.synchronize()
 
+    resident_loss = [static_loss]
+
     def step_resident():
         if graph is not None:
             graph.replay()
         else:
-            step_eager()
+            resident_loss[0] = step_eager()
 
     last_loss = [0.0]
     # End-to-end input pipeline (what a pinned-memory loader with prefetch does): every step's image + depth are copied
@@ -368,6 +422,19 @@ def run_ours(args):
     if graph is not None:
         launches = launches_per_replay * args.steps  # replayed from the graph: counted once at capture time
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # The state reached after the timed regions differs from run to run (float atomics in the library and cuDNN's
+        # convolutions vary the summation order, and the Adam steps amplify that), so the timed step runs twice more
+        # from the seeded initial state, on every rank (a DDP step all-reduces): rank 0 writes both losses and the
+        # first step's gradients.  With the same arguments, these depend on the arguments only, up to rounding.
+        reset_state(model, opt, state0)
+        step_resident()
+        losses, grads = [resident_loss[0].detach().item()], grad_sample(model)
+        step_resident()
+        losses.append(resident_loss[0].detach().item())
+        if rank == 0:
+            dump_outputs(args.dump_outputs, losses, grads)
+        state0 = None
 
     for _ in range(args.steps):   # one full untimed region (keeps the prefetch phase aligned with the step counter)
         step_e2e()

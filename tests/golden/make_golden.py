@@ -11,12 +11,14 @@ time with rate 0 (newcrf_layers.py:6,107,184,187), so a stub module is injected 
 import os
 import sys
 import types
+import zlib
 
 import numpy as np
 import torch
 import torch.nn as nn
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 REF_SRC = "/root/reference/src"
 
 
@@ -43,17 +45,36 @@ def import_reference():
 
 def randomize(module, gen):
     """Replace default-initialised parameters (zero biases, unit LN weights) by non-trivial values so that every
-    parameter influences the output and receives a non-trivial gradient."""
+    parameter influences the output and receives a non-trivial gradient (tests.helpers.draw_layer_param, which the
+    tests use to draw the same values again from the fixture's seed)."""
+    from tests.helpers import draw_layer_param
     with torch.no_grad():
         for name, p in module.named_parameters():
-            if name.endswith("norm1.weight") or name.endswith("norm2.weight"):
-                p.copy_(1.0 + 0.1 * torch.randn(p.shape, generator=gen))
-            elif name.endswith(".bias"):
-                p.copy_(0.1 * torch.randn(p.shape, generator=gen))
-            elif name.endswith("relative_position_bias_table"):
-                p.copy_(0.2 * torch.randn(p.shape, generator=gen))
-            else:
-                p.copy_(torch.randn(p.shape, generator=gen) * p.shape[-1] ** -0.5)
+            p.copy_(draw_layer_param(name, p.shape, gen))
+
+
+# Gradients stored as a fixed half-sample of their elements, so that every fixture stays below 1 MB.
+SAMPLED_GRADS = {"block_14x21_c128": ("blocks.0.mlp.fc1.weight", "blocks.0.mlp.fc2.weight")}
+
+
+def write_layer_fixture(name, seed, meta, inputs, sd, outputs, grads):
+    """A layer fixture holds the reference's outputs (y, dx, dv, `grad.<param>`) and what draws its inputs again
+    (tests.helpers.layer_inputs_from_seed): the seed, the state_dict keys in order with their shapes, and the CRC32 of
+    the inputs (x, v, dy, then the state_dict) the reference was run on."""
+    crc = 0
+    for t in [inputs["x"], inputs["v"], inputs["dy"]] + list(sd.values()):
+        crc = zlib.crc32(np.ascontiguousarray(t).tobytes(), crc)
+    blob = {"meta": meta, "seed": np.array([seed], dtype=np.int64), "sd_keys": np.array(list(sd)),
+            "inputs_crc32": np.array([crc], dtype=np.int64)}
+    blob.update({"shape." + k: np.array(t.shape, dtype=np.int64) for k, t in sd.items()})
+    blob.update(outputs)
+    blob.update({"grad." + k: g for k, g in grads.items()})
+    rng = np.random.default_rng(seed)
+    for k in SAMPLED_GRADS.get(name, ()):
+        keep = rng.random(grads[k].size) < 0.5
+        blob["mask.grad." + k] = np.packbits(keep)
+        blob["grad." + k] = grads[k].reshape(-1)[keep]
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), **blob)
 
 
 def layer_case(ref, name, B, H, W, C, nH, depth, seed, strided):
@@ -73,14 +94,11 @@ def layer_case(ref, name, B, H, W, C, nH, depth, seed, strided):
     y = out[0]
     assert out[1] == H and out[2] == W and out[3] is y
     y.backward(dy)
-    blob = {"meta": np.array([B, H, W, C, nH, depth, int(strided)], dtype=np.int64),
-            "x": x.detach().contiguous().numpy(), "v": v.detach().contiguous().numpy(), "dy": dy.numpy(),
-            "y": y.detach().numpy(), "dx": x.grad.contiguous().numpy(), "dv": v.grad.contiguous().numpy()}
-    for k, t in layer.state_dict().items():
-        blob["sd." + k] = t.numpy()
-    for k, p in layer.named_parameters():
-        blob["grad." + k] = p.grad.numpy()
-    np.savez_compressed(os.path.join(HERE, name + ".npz"), **blob)
+    write_layer_fixture(name, seed, np.array([B, H, W, C, nH, depth, int(strided)], dtype=np.int64),
+                        {"x": x.detach().contiguous().numpy(), "v": v.detach().contiguous().numpy(), "dy": dy.numpy()},
+                        {k: t.numpy() for k, t in layer.state_dict().items()},
+                        {"y": y.detach().numpy(), "dx": x.grad.contiguous().numpy(), "dv": v.grad.contiguous().numpy()},
+                        {k: p.grad.numpy() for k, p in layer.named_parameters()})
     print(name, "y", tuple(y.shape), "abs-mean", float(y.abs().mean()))
 
 
@@ -156,7 +174,6 @@ def model_case(name):
     of a dozen small parameters.  Weights come from tests.helpers.fill_by_name (seeded by parameter NAME), so the oracle
     and the product rebuild exactly the same model without a checkpoint.  Import shims (SURVEY.md Appendix A):
     matplotlib is absent (utils.py imports it for colour maps only) and `pretrained=True` needs the network."""
-    sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
     from tests.helpers import MODEL_GRAD_KEYS, fill_by_name
     for m in ("matplotlib", "matplotlib.cm"):
         sys.modules.setdefault(m, types.ModuleType(m))

@@ -1,5 +1,6 @@
 """Shared test helpers: golden-fixture loading and error metrics."""
 import os
+import zlib
 
 import numpy as np
 import torch
@@ -11,7 +12,63 @@ HEAD_CASES = ["layer_8x13_c64_hd64", "layer_8x13_c64_hd16"]   # head widths othe
 
 def load_golden(name):
     z = np.load(os.path.join(GOLDEN, name + ".npz"))
-    return {k: z[k] for k in z.files}
+    g = {k: z[k] for k in z.files}
+    if "seed" in g:
+        g.update(layer_inputs_from_seed(g))
+    return g
+
+
+def draw_layer_param(name, shape, gen):
+    """One parameter of a layer fixture: non-trivial values (no zero biases or unit LN weights) so that every
+    parameter influences the output and receives a non-trivial gradient."""
+    if name.endswith("norm1.weight") or name.endswith("norm2.weight"):
+        return 1.0 + 0.1 * torch.randn(shape, generator=gen)
+    if name.endswith(".bias"):
+        return 0.1 * torch.randn(shape, generator=gen)
+    if name.endswith("relative_position_bias_table"):
+        return 0.2 * torch.randn(shape, generator=gen)
+    return torch.randn(shape, generator=gen) * shape[-1] ** -0.5
+
+
+def layer_inputs_from_seed(g):
+    """The inputs of a layer fixture (x, v, dy and the state_dict as `sd.<key>`), drawn from the fixture's seed in the
+    order tests/golden/make_golden.py drew them for the reference: the parameters in state_dict order, then x, v, dy.
+    A layer fixture stores only the seed, the reference's state_dict keys and shapes, and the reference's outputs;
+    `inputs_crc32` pins the redrawn inputs to the ones the reference saw."""
+    B, H, W, C, nH, depth, strided = [int(t) for t in g["meta"]]
+    gen = torch.Generator().manual_seed(int(g["seed"][0]))
+    out = {}
+    for k in g["sd_keys"].tolist():
+        shape = tuple(int(s) for s in g["shape." + k])
+        if k.endswith("relative_position_index"):   # a buffer, not drawn: the reference's own index map
+            idx = np.load(os.path.join(GOLDEN, "index_maps.npz"))["relative_position_index"]
+            assert idx.shape == shape, (k, idx.shape, shape)
+            out["sd." + k] = idx
+        else:
+            out["sd." + k] = draw_layer_param(k, shape, gen).numpy()
+    if strided:   # drawn as NCHW maps, the layouts NewCRF.forward hands over (newcrf_layers.py:426-427)
+        x = torch.randn(B, C, H, W, generator=gen).flatten(2).transpose(1, 2)
+        v = torch.randn(B, C, H, W, generator=gen).transpose(1, 2).transpose(2, 3)
+    else:
+        x = torch.randn(B, H * W, C, generator=gen)
+        v = torch.randn(B, H, W, C, generator=gen)
+    out["x"], out["v"] = x.contiguous().numpy(), v.contiguous().numpy()
+    out["dy"] = torch.randn(B, H * W, C, generator=gen).numpy()
+    crc = 0
+    for k in ["x", "v", "dy"] + ["sd." + k for k in g["sd_keys"].tolist()]:
+        crc = zlib.crc32(np.ascontiguousarray(out[k]).tobytes(), crc)
+    assert crc == int(g["inputs_crc32"][0]), "the redrawn inputs differ from the ones the reference was run on"
+    return out
+
+
+def golden_rel_l2(g, key, t):
+    """rel_l2 of `t` against the fixture's `g[key]`.  Where the fixture stores a fixed sample of a large tensor
+    (`mask.<key>`: np.packbits of a boolean mask over the flattened tensor), on the sampled elements."""
+    if "mask." + key not in g:
+        return rel_l2(t, g[key])
+    t = torch.as_tensor(t).detach().reshape(-1).cpu()
+    keep = np.unpackbits(g["mask." + key])[: t.numel()].astype(bool)
+    return rel_l2(t[torch.from_numpy(keep)], g[key])
 
 
 def rel_l2(a, b):
@@ -48,7 +105,6 @@ def fill_by_name(module):
     each tensor is drawn from a generator seeded by the CRC32 of its state_dict name.  The reference model (in the build
     container, tests/golden/make_golden.py), the oracle model and the product model therefore get identical weights
     from their NAMES alone -- no 180 MB checkpoint has to travel to the GPU box."""
-    import zlib
     with torch.no_grad():
         for name, t in list(module.named_parameters()) + list(module.named_buffers()):
             if name.endswith("relative_position_index") or name.endswith("num_batches_tracked"):

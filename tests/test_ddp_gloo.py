@@ -42,8 +42,10 @@ def _data(n):
 
 
 def _worker(rank, world, port, out_path, grad_dtype=None):
+    # the CPU / gloo path also on a host with GPUs: this spawned process has not initialised CUDA yet, so hiding the
+    # devices here makes init_distributed() choose the CPU (with GPUs it would take cuda:<local rank> and NCCL)
     os.environ.update({"RANK": str(rank), "LOCAL_RANK": str(rank), "WORLD_SIZE": str(world),
-                       "MASTER_ADDR": "127.0.0.1", "MASTER_PORT": str(port)})
+                       "MASTER_ADDR": "127.0.0.1", "MASTER_PORT": str(port), "CUDA_VISIBLE_DEVICES": ""})
     torch.set_num_threads(1)
     r, lr, w, device = T.init_distributed()
     assert (r, w, device.type) == (rank, world, "cpu")

@@ -5,7 +5,7 @@ import pytest
 import torch
 
 from oracle import crf_oracle as O
-from tests.helpers import HEAD_CASES, LAYER_CASES, golden_layer_inputs, load_golden, rel_l2
+from tests.helpers import HEAD_CASES, LAYER_CASES, golden_layer_inputs, golden_rel_l2, load_golden, rel_l2
 
 
 def test_index_maps_bit_exact():
@@ -53,7 +53,7 @@ def test_layer_forward_backward_matches_reference(name):
     assert rel_l2(v.grad, g["dv"]) < 1e-5
     for i, p in enumerate(blocks):
         for k, t in p.items():
-            assert rel_l2(t.grad, g[f"grad.blocks.{i}.{k}"]) < 2e-5, (i, k)
+            assert golden_rel_l2(g, f"grad.blocks.{i}.{k}", t.grad) < 2e-5, (i, k)
 
 
 def test_loss_matches_reference_golden():
