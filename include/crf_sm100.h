@@ -45,7 +45,7 @@ enum { CRF_DT_F32 = 0, CRF_DT_BF16 = 1 };
 typedef struct crf_block_desc {
   int32_t B, H, W, C;
   int32_t num_heads;
-  int32_t window;   /* 7 */
+  int32_t window;   /* 2..8 (the reference's default 7) */
   int32_t shift;    /* 0 or window/2 */
   int32_t training; /* 1: keep everything backward needs in `saved` */
   int32_t device;   /* CUDA device ordinal that owns every pointer */
@@ -66,7 +66,7 @@ typedef struct crf_block_params {
   const float* norm1_b;  /* (C)      */
   const float* qk_w;     /* (2C, C)  blocks.i.attn.qk.weight : first C rows -> q, last C rows -> k */
   const float* qk_b;     /* (2C)     */
-  const float* rpb_table;/* (169,nH) blocks.i.attn.relative_position_bias_table */
+  const float* rpb_table;/* ((2w-1)^2,nH), w = window: blocks.i.attn.relative_position_bias_table */
   const float* proj_w;   /* (C, C)   */
   const float* proj_b;   /* (C)      */
   const float* norm2_w;  /* (C)      */
@@ -78,7 +78,7 @@ typedef struct crf_block_params {
   float qk_scale;        /* head_dim^-0.5 unless overridden (newcrf_layers.py:83) */
   float ln_eps;          /* 1e-5 */
   const float* ext_mask; /* NULL: the shifted-window mask of BasicCRFLayer.forward (newcrf_layers.py:332-350), evaluated
-                          * in closed form.  Otherwise an additive (ext_mask_windows, 49, 49) f32 mask that REPLACES it
+                          * in closed form.  Otherwise an additive (ext_mask_windows, N, N) f32 mask, N = window^2, that REPLACES it
                           * (CRFBlock.forward's mask_matrix argument, :195,236): window w of every image uses
                           * ext_mask[w mod ext_mask_windows]. */
   int32_t ext_mask_windows;
@@ -318,12 +318,12 @@ int crf_cast_bf16(const float* src, void* dst, int64_t n, int device, void* stre
  *   o    bf16 (T, C)   attention output in token order (window_reverse + un-roll + crop applied)
  *   lse  f32 (B*nW, nH, 64) row log-sum-exp (saved for backward)
  *   qk_bias f32 (2C): q/k of zero-padded tokens are their bias (newcrf_layers.py:215,118) */
-/*   mask  optional additive mask f32 (mask_windows, 49, 49) applied to window (global index % mask_windows), as
+/*   mask  optional additive mask f32 (mask_windows, N, N), N = window^2, applied to window (global index % mask_windows), as
  *         WindowAttention.forward's `mask` argument (newcrf_layers.py:129-133); NULL / 0 for none */
 int crf_attn_fwd(const crf_block_desc* d, const void* qk, const void* vb, const float* qk_bias, float scale,
                  const float* rpb_table, const float* mask, int mask_windows, void* o, float* lse, void* stream);
 /*   dout bf16 (T, C); dqk bf16 (T, 2C) (dq includes the scale factor); dv f32 (T, C) (= or +=);
- *   d_table f32 (169, nH) +=;  d_qk_bias f32 (2C) += (only the k half receives pad-token gradient) */
+ *   d_table f32 ((2w-1)^2, nH) +=;  d_qk_bias f32 (2C) += (only the k half receives pad-token gradient) */
 int crf_attn_bwd(const crf_block_desc* d, const void* qk, const void* vb, const float* qk_bias, float scale,
                  const float* rpb_table, const float* mask, int mask_windows, const float* lse, const void* dout,
                  void* dqk, float* dv, int dv_accumulate, float* d_table, float* d_qk_bias, void* stream);

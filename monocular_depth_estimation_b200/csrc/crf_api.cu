@@ -113,7 +113,8 @@ int check_desc(const crf_block_desc* d) {
   CRF_CHECK(d->C % 64 == 0 && d->C >= 64 && d->C <= 1024, "C=%d must be a multiple of 64 in [64,1024]", d->C);
   CRF_CHECK(d->num_heads > 0 && d->C % d->num_heads == 0 && head_dim_supported(d->C / d->num_heads),
             "head_dim must be 16, 32, 64 or 128 (C=%d, heads=%d)", d->C, d->num_heads);
-  CRF_CHECK(d->window == 7, "window must be 7 (got %d)", d->window);
+  CRF_CHECK(d->window >= kMinWindow && d->window <= kMaxWindow, "window must be in [%d, %d] (got %d)", kMinWindow,
+            kMaxWindow, d->window);
   CRF_CHECK(d->shift >= 0 && d->shift < d->window, "shift_size must in 0-window_size");
   CRF_CHECK(static_cast<int64_t>(d->B) * d->H * d->W * 4 * d->C < (int64_t(1) << 31) * 4,
             "problem too large for 32-bit token indexing");

@@ -18,7 +18,8 @@ bool head_dim_supported(int hd) { return hd == 16 || hd == 32 || hd == 64 || hd 
 int fill_attn_params(AttnParams& P, const crf_block_desc& d) {
   CRF_CHECK(d.num_heads > 0 && d.C % d.num_heads == 0 && head_dim_supported(d.C / d.num_heads),
             "attention core: head_dim must be 16, 32, 64 or 128 (C=%d, heads=%d)", d.C, d.num_heads);
-  CRF_CHECK(d.window == 7, "attention core: window must be 7 (got %d)", d.window);
+  CRF_CHECK(d.window >= kMinWindow && d.window <= kMaxWindow, "attention core: window must be in [%d, %d] (got %d)",
+            kMinWindow, kMaxWindow, d.window);
   CRF_CHECK(d.shift >= 0 && d.shift < d.window, "shift_size must in 0-window_size");
   P.gm = WindowGeom(d.H, d.W, d.window, d.shift);
   P.B = d.B;

@@ -4,8 +4,9 @@
 // relative-position-bias gather, the shifted-window mask, softmax, attn @ v, window_reverse, the reverse roll and
 // the crop (newcrf_layers.py:121-146, :212-249, :332-350).
 //
-// Work decomposition: a CTA owns one head and loops over PAIRS of windows.  The two 49-token windows of a pair are
-// stacked into one 128-row UMMA tile (rows 0..48 = window A, 64..112 = window B, the rest zero):
+// Work decomposition: a CTA owns one head and loops over PAIRS of windows.  The two N-token windows of a pair
+// (N = ws^2 <= 64; the kernels are instantiated per window size 2..8, and the prose below uses ws = 7, N = 49) are
+// stacked into one 128-row UMMA tile (rows 0..N-1 = window A, 64..64+N-1 = window B, the rest zero):
 //   S  [128 x 128] = bias + Q[128 x hd] * [K_A ; K_B]^T     -- row r only uses the 64 columns of its own window
 //   O  [128 x 2hd] = P~[128 x 64] * [V_A | V_B]             -- row r reads the hd columns of its window
 // Token rows are gathered straight from the token-major q/k/v tensors with the closed-form pad+roll index map
@@ -63,14 +64,27 @@ constexpr uint32_t kFwdMisc = kFwdTiles + 2 * 16384;
 constexpr uint32_t kBwdTiles = 4 * kSlot;               // P | dS tiles: 2 lanes x (16 + 16) KB
 constexpr uint32_t kBwdMisc = kBwdTiles + 2 * 32768;
 constexpr int kBiasStride = 68;                         // floats per bias row (272 B: conflict-free LDS.128 per quarter warp)
-constexpr uint32_t kMiscTbl = 0;                        // tbl[176] f32
-constexpr uint32_t kMiscBias = 704;                     // bias rows [49][68] f32
-constexpr uint32_t kMiscScratch = kMiscBias + kNTok * kBiasStride * 4;   // 8 compute warps x (32 rows x 80 B)
 constexpr uint32_t kScratchWarp = 32 * 80;
-constexpr uint32_t kMiscBar = kMiscScratch + 8 * kScratchWarp;         // 16 mbarriers
-constexpr uint32_t kMiscTmem = kMiscBar + 16 * 8;
-constexpr uint32_t kMiscBytes = kMiscTmem + 16;
-static_assert(kMiscBar % 8 == 0, "mbarrier alignment");
+
+// The misc region behind the tiles, for window size WS (N = WS^2 tokens per window):
+//   tbl[rpb_table_padded(WS)] f32 | bias rows [N][68] f32 | 8 compute warps x (32 rows x 80 B) scratch | 16 mbarriers |
+//   TMEM address.  At WS = 7: tbl[176], bias rows [49][68].
+// The WS = 8 backward keeps no bias rows: its 196 KB of tiles plus 64 rows of 272 B would exceed the 227 KB a CTA may
+// use, so it pre-loads the bias straight from the table (64 scalar LDS per row and pair instead of 16 LDS.128).
+template <int WS, bool BWD>
+struct Misc {
+  static constexpr int kN = WS * WS;
+  static constexpr bool kBiasRows = !(BWD && WS == 8);
+  static constexpr int kTblFloats = rpb_table_padded(WS);
+  static constexpr uint32_t kTbl = 0;
+  static constexpr uint32_t kBias = kTblFloats * 4;
+  static constexpr uint32_t kScratch = kBias + (kBiasRows ? kN * kBiasStride * 4 : 0);
+  static constexpr uint32_t kBar = kScratch + 8 * kScratchWarp;
+  static constexpr uint32_t kTmem = kBar + 16 * 8;
+  static constexpr uint32_t kBytes = kTmem + 16;
+  static_assert(kBias % 16 == 0 && kBar % 8 == 0, "bias-row / mbarrier alignment");
+  static_assert(WS >= kMinWindow && WS <= kMaxWindow, "a window's N = WS^2 tokens must fit 64 tile rows");
+};
 
 struct Bars {
   uint32_t base;
@@ -110,45 +124,49 @@ struct WinPos {
   int b, wh, ww;
   bool hsplit, wsplit;  // the window straddles the roll seam in h / w (shifted-window mask separates positions)
 };
+template <int WS>
 __device__ __forceinline__ WinPos window_pos(const AttnParams& P, int wg) {
   WinPos w;
   w.b = fast_div(wg, P.gm.nW, P.rcp_nW);
   const int win = wg - w.b * P.gm.nW;
   w.wh = fast_div(win, P.gm.nWw, P.rcp_nWw);
   w.ww = win - w.wh * P.gm.nWw;
-  w.hsplit = P.gm.shift > 0 && (w.wh + 1) * 7 == P.gm.Hp;
+  w.hsplit = P.gm.shift > 0 && (w.wh + 1) * WS == P.gm.Hp;
   w.wsplit = P.gm.shift > 0 && (w.ww + 1) == P.gm.nWw;
   return w;
 }
 // Closed-form geometry of tile position (pi, pj) of a window (newcrf_layers.py:212-233 folded): token index (>= 0),
 // or -1 for a zero-pad position.
+template <int WS>
 __device__ __forceinline__ int window_token(const AttnParams& P, const WinPos& w, int pi, int pj) {
-  int hh = w.wh * 7 + pi + P.gm.shift, wx = w.ww * 7 + pj + P.gm.shift;
+  int hh = w.wh * WS + pi + P.gm.shift, wx = w.ww * WS + pj + P.gm.shift;
   if (hh >= P.gm.Hp) hh -= P.gm.Hp;
   if (wx >= P.gm.Wp) wx -= P.gm.Wp;
   return (hh < P.gm.H && wx < P.gm.W) ? (w.b * P.gm.H + hh) * P.gm.W + wx : -1;
 }
 
-// Per-row view a compute thread needs: token (-2 dead row), global window, and the 49-bit set of key positions j the
+// Per-row view a compute thread needs: token (-2 dead row), global window, and the N-bit set of key positions j the
 // shifted-window mask separates from this row (region(i) != region(j)  <=>  they lie on different sides of a seam).
 struct RowView {
   int tok, wg;
   uint32_t m_lo, m_hi;
 };
+template <int WS>
 __device__ __forceinline__ RowView row_view(const AttnParams& P, int pair, int half, int pos, int pi, int pj,
                                             uint64_t far_h, uint64_t far_w) {
+  constexpr int kN = WS * WS;
   RowView v;
   v.wg = 2 * pair + half;
   v.tok = -2;
   v.m_lo = v.m_hi = 0u;
-  if (pos < kNTok && v.wg < P.total_windows) {
-    const WinPos w = window_pos(P, v.wg);
-    v.tok = window_token(P, w, pi, pj);
-    const int lo = 7 - P.gm.shift;
+  if (pos < kN && v.wg < P.total_windows) {
+    const WinPos w = window_pos<WS>(P, v.wg);
+    v.tok = window_token<WS>(P, w, pi, pj);
+    const int lo = WS - P.gm.shift;
     uint64_t m = 0;
     if (w.hsplit) m |= (pi >= lo) ? ~far_h : far_h;
     if (w.wsplit) m |= (pj >= lo) ? ~far_w : far_w;
-    m &= (1ull << kNTok) - 1;
+    m &= kN < 64 ? (1ull << (kN & 63)) - 1 : ~0ull;  // (a shift by 64 would be undefined)
     if (P.ext_replaces) m = 0;
     v.m_lo = static_cast<uint32_t>(m);
     v.m_hi = static_cast<uint32_t>(m >> 32);
@@ -157,28 +175,32 @@ __device__ __forceinline__ RowView row_view(const AttnParams& P, int pair, int h
 }
 #define CRF_MASKED(v, j) ((((j) < 32 ? (v).m_lo >> ((j) & 31) : (v).m_hi >> ((j) & 31)) & 1u) != 0u)
 
-// key positions on the far side of the seam: rows i >= 7 - shift (far_h), columns j >= 7 - shift (far_w)
+// key positions on the far side of the seam: rows i >= WS - shift (far_h), columns j >= WS - shift (far_w)
+template <int WS>
 __device__ __forceinline__ void seam_sets(int shift, uint64_t& far_h, uint64_t& far_w) {
   far_h = far_w = 0;
-  const int lo = 7 - shift;
+  const int lo = WS - shift;
 #pragma unroll
-  for (int j = 0; j < kNTok; ++j) {
-    if (j / 7 >= lo) far_h |= 1ull << j;
-    if (j % 7 >= lo) far_w |= 1ull << j;
+  for (int j = 0; j < WS * WS; ++j) {
+    if (j / WS >= lo) far_h |= 1ull << j;
+    if (j % WS >= lo) far_w |= 1ull << j;
   }
 }
 
-// bias rows: brow[i][j] = table[relative_position_index[i][j], h] (newcrf_layers.py:124-127), 0 for j >= 49
+// bias rows: brow[i][j] = table[relative_position_index[i][j], h] (newcrf_layers.py:124-127), 0 for j >= N
+template <int WS>
 __device__ __forceinline__ void build_bias_rows(float* brow, const float* tbl) {
-  for (int idx = threadIdx.x; idx < kNTok * 64; idx += kThreads) {
+  constexpr int kN = WS * WS;
+  for (int idx = threadIdx.x; idx < kN * 64; idx += kThreads) {
     const int i = idx >> 6, j = idx & 63;
-    brow[i * kBiasStride + j] = j < kNTok ? tbl[rpb_base(i) - rpb_col(j)] : 0.f;
+    brow[i * kBiasStride + j] = j < kN ? tbl[rpb_base<WS>(i) - rpb_col<WS>(j)] : 0.f;
   }
 }
 // Write this thread's bias row into the 64 S columns of its TMEM lane (whole warp; dead rows write row 0's values,
 // which nobody reads), so that the next S MMA accumulates Q K^T on top of it.
+template <int WS>
 __device__ __forceinline__ void preload_bias(const float* brow, int pos, uint32_t taddr) {
-  const float4* src = reinterpret_cast<const float4*>(brow + (pos < kNTok ? pos : 0) * kBiasStride);
+  const float4* src = reinterpret_cast<const float4*>(brow + (pos < WS * WS ? pos : 0) * kBiasStride);
 #pragma unroll
   for (int hlf = 0; hlf < 2; ++hlf) {
     uint32_t v[32];
@@ -191,6 +213,29 @@ __device__ __forceinline__ void preload_bias(const float* brow, int pos, uint32_
     tmem_st32(taddr + hlf * 32, v);
   }
   tmem_st_wait();
+}
+// The same row gathered from the table itself (the WS = 8 backward, which has no room for bias rows).  Every column
+// j < N of a live row gets its bias; the columns j >= N of this N = 64 window do not exist.
+template <int WS>
+__device__ __forceinline__ void preload_bias_from_table(const float* tbl, int pos, uint32_t taddr) {
+  constexpr int kN = WS * WS;
+  const int bi = rpb_base<WS>(pos < kN ? pos : 0);
+#pragma unroll
+  for (int hlf = 0; hlf < 2; ++hlf) {
+    uint32_t v[32];
+#pragma unroll
+    for (int c = 0; c < 32; ++c) {
+      const int j = hlf * 32 + c;
+      v[c] = j < kN ? __float_as_uint(tbl[bi - rpb_col<WS>(j)]) : 0u;
+    }
+    tmem_st32(taddr + hlf * 32, v);
+  }
+  tmem_st_wait();
+}
+template <int WS, bool BWD>
+__device__ __forceinline__ void preload_row_bias(const float* brow, const float* tbl, int pos, uint32_t taddr) {
+  if constexpr (Misc<WS, BWD>::kBiasRows) preload_bias<WS>(brow, pos, taddr);
+  else preload_bias_from_table<WS>(tbl, pos, taddr);
 }
 
 // Loaders: FOUR threads per tile row (thread t: 16-byte chunk t & 3 of rows (t >> 2) + 32 k), so one warp-level
@@ -226,14 +271,16 @@ __device__ __forceinline__ void load_chunk(const AttnParams& P, int tok, int r, 
   }
 }
 
-template <bool BWD>
+template <int WS, bool BWD>
 __device__ __forceinline__ void loader_loop(const AttnParams& P, const Bars& bars, uint32_t base, uint8_t* gen, int h,
                                             int niter) {
+  constexpr int kN = WS * WS;
   const int t = threadIdx.x - 256;
   const int c = t & 3, rb = t >> 2;           // rows rb, rb + 32 (window A) and rb + 64, rb + 96 (window B)
-  const int pi0 = rb / 7, pj0 = rb % 7;       // position rb (always a live position)
-  const int pi1 = (rb + 32) / 7, pj1 = (rb + 32) % 7;
-  const bool live1 = rb + 32 < kNTok;
+  const int pi0 = rb / WS, pj0 = rb % WS;     // position rb (always live when N > 32)
+  const int pi1 = (rb + 32) / WS, pj1 = (rb + 32) % WS;
+  const bool live0 = kN > 32 || rb < kN;      // dead rows (-2) are written as zeros
+  const bool live1 = rb + 32 < kN;
   int pair = blockIdx.x;
   const bool prof = P.prof && blockIdx.x == 0 && blockIdx.y == 0 && t == 0;
   long long t_wait = 0, t_begin = prof ? clock64() : 0;
@@ -245,9 +292,9 @@ __device__ __forceinline__ void loader_loop(const AttnParams& P, const Bars& bar
       const int wg = 2 * pair + half;
       tok[2 * half] = tok[2 * half + 1] = -2;
       if (wg < P.total_windows) {
-        const WinPos w = window_pos(P, wg);
-        tok[2 * half] = window_token(P, w, pi0, pj0);
-        if (live1) tok[2 * half + 1] = window_token(P, w, pi1, pj1);
+        const WinPos w = window_pos<WS>(P, wg);
+        if (live0) tok[2 * half] = window_token<WS>(P, w, pi0, pj0);
+        if (live1) tok[2 * half + 1] = window_token<WS>(P, w, pi1, pj1);
       }
     }
     const long long t0 = prof ? clock64() : 0;
@@ -301,18 +348,21 @@ __device__ __forceinline__ void warp_store_rows64(uint8_t* scratch, int lane, co
 // =====================================================================================================
 // forward
 // =====================================================================================================
+template <int WS>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_fwd_async_kernel(const AttnParams P) {
+  using M = Misc<WS, false>;
+  constexpr int kNTok = WS * WS;
   pdl_launch_dependents();   // (the relative-position table below is a parameter: read before pdl_wait)
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
   uint8_t* misc = gen + kFwdMisc;
-  float* tbl = reinterpret_cast<float*>(misc + kMiscTbl);
-  float* brow = reinterpret_cast<float*>(misc + kMiscBias);
-  const Bars bars{base + kFwdMisc + kMiscBar};
-  const uint32_t tmem_ptr_addr = base + kFwdMisc + kMiscTmem;
-  volatile uint32_t* tmem_ptr_gen = reinterpret_cast<volatile uint32_t*>(misc + kMiscTmem);
+  float* tbl = reinterpret_cast<float*>(misc + M::kTbl);
+  float* brow = reinterpret_cast<float*>(misc + M::kBias);
+  const Bars bars{base + kFwdMisc + M::kBar};
+  const uint32_t tmem_ptr_addr = base + kFwdMisc + M::kTmem;
+  volatile uint32_t* tmem_ptr_gen = reinterpret_cast<volatile uint32_t*>(misc + M::kTmem);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int h = blockIdx.y;
@@ -325,9 +375,10 @@ attn_fwd_async_kernel(const AttnParams P) {
     tmem_alloc(tmem_ptr_addr, 256);
     tmem_relinquish();
   }
-  for (int i = threadIdx.x; i < 176; i += kThreads) tbl[i] = i < 169 ? __ldg(P.table + i * P.nH + h) : 0.f;
+  for (int i = threadIdx.x; i < M::kTblFloats; i += kThreads)
+    tbl[i] = i < rpb_table_size(WS) ? __ldg(P.table + i * P.nH + h) : 0.f;
   __syncthreads();
-  build_bias_rows(brow, tbl);
+  build_bias_rows<WS>(brow, tbl);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -370,26 +421,26 @@ attn_fwd_async_kernel(const AttnParams P) {
     }
   } else if (warp >= 8) {
     reg_dealloc<56>();
-    loader_loop<false>(P, bars, base, gen, h, niter);
+    loader_loop<WS, false>(P, bars, base, gen, h, niter);
   } else {
     // ================= compute groups =================
     reg_alloc<200>();
     const int g = warp >> 2;
     const int r = threadIdx.x & 127;
     const int half = r >> 6, pos = r & 63;
-    const int pi = pos / 7, pj = pos % 7;
+    const int pi = pos / WS, pj = pos % WS;
     const uint32_t t0 = tmem + g * 128 + (static_cast<uint32_t>((warp & 3) * 32) << 16);
     uint8_t* Ps_g = gen + kFwdTiles + g * 16384;
-    uint8_t* scratch = misc + kMiscScratch + warp * kScratchWarp;
+    uint8_t* scratch = misc + M::kScratch + warp * kScratchWarp;
     uint64_t far_h, far_w;
-    seam_sets(P.gm.shift, far_h, far_w);
+    seam_sets<WS>(P.gm.shift, far_h, far_w);
     CRF_PROF_DECL(8);
 
-    preload_bias(brow, pos, t0 + half * 64);
+    preload_bias<WS>(brow, pos, t0 + half * 64);
     tc_fence_before();
     mbar_arrive(bars.t_free(g));
 
-    RowView rv = row_view(P, blockIdx.x + g * gridDim.x, half, pos, pi, pj, far_h, far_w);
+    RowView rv = row_view<WS>(P, blockIdx.x + g * gridDim.x, half, pos, pi, pj, far_h, far_w);
     for (int i = g, n = 0; i < niter; i += 2, ++n) {
       const int pair = blockIdx.x + i * gridDim.x;
       const float* xmask = (P.ext_mask != nullptr && rv.tok != -2)
@@ -451,7 +502,7 @@ attn_fwd_async_kernel(const AttnParams P) {
       CRF_PROF_MARK(4);
       if (P.lse != nullptr && rv.tok != -2) P.lse[(static_cast<int64_t>(rv.wg) * P.nH + h) * 64 + pos] = lse;
       // geometry of this lane's next pair, computed while the tensor core works on O
-      const RowView rv_next = row_view(P, pair + 2 * gridDim.x, half, pos, pi, pj, far_h, far_w);
+      const RowView rv_next = row_view<WS>(P, pair + 2 * gridDim.x, half, pos, pi, pj, far_h, far_w);
 
       mbar_wait(bars.o_done(g), n & 1);
       CRF_PROF_MARK(5);
@@ -459,7 +510,7 @@ attn_fwd_async_kernel(const AttnParams P) {
       uint32_t o[32];
       tmem_ld32(t0 + half * HD, o);
       tmem_ld_wait();
-      preload_bias(brow, pos, t0 + half * 64);  // the next S of this lane accumulates on top of the bias
+      preload_bias<WS>(brow, pos, t0 + half * 64);  // the next S of this lane accumulates on top of the bias
       tc_fence_before();
       mbar_arrive(bars.t_free(g));
       CRF_PROF_MARK(6);
@@ -496,18 +547,21 @@ attn_fwd_async_kernel(const AttnParams P) {
 // =====================================================================================================
 // backward
 // =====================================================================================================
+template <int WS>
 __global__ void __launch_bounds__(kThreads, 1)
 attn_bwd_async_kernel(const AttnParams P) {
+  using M = Misc<WS, true>;
+  constexpr int kNTok = WS * WS;
   pdl_launch_dependents();   // (the relative-position table below is a parameter: read before pdl_wait)
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
   uint8_t* misc = gen + kBwdMisc;
-  float* tbl = reinterpret_cast<float*>(misc + kMiscTbl);
-  float* brow = reinterpret_cast<float*>(misc + kMiscBias);
-  const Bars bars{base + kBwdMisc + kMiscBar};
-  const uint32_t tmem_ptr_addr = base + kBwdMisc + kMiscTmem;
-  volatile uint32_t* tmem_ptr_gen = reinterpret_cast<volatile uint32_t*>(misc + kMiscTmem);
+  float* tbl = reinterpret_cast<float*>(misc + M::kTbl);
+  float* brow = reinterpret_cast<float*>(misc + M::kBias);
+  const Bars bars{base + kBwdMisc + M::kBar};
+  const uint32_t tmem_ptr_addr = base + kBwdMisc + M::kTmem;
+  volatile uint32_t* tmem_ptr_gen = reinterpret_cast<volatile uint32_t*>(misc + M::kTmem);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int h = blockIdx.y;
@@ -520,9 +574,10 @@ attn_bwd_async_kernel(const AttnParams P) {
     tmem_alloc(tmem_ptr_addr, 512);
     tmem_relinquish();
   }
-  for (int i = threadIdx.x; i < 176; i += kThreads) tbl[i] = i < 169 ? __ldg(P.table + i * P.nH + h) : 0.f;
+  for (int i = threadIdx.x; i < M::kTblFloats; i += kThreads)
+    tbl[i] = i < rpb_table_size(WS) ? __ldg(P.table + i * P.nH + h) : 0.f;
   __syncthreads();
-  build_bias_rows(brow, tbl);
+  if constexpr (M::kBiasRows) build_bias_rows<WS>(brow, tbl);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -583,41 +638,41 @@ attn_bwd_async_kernel(const AttnParams P) {
     }
   } else if (warp >= 8) {
     reg_dealloc<56>();
-    loader_loop<true>(P, bars, base, gen, h, niter);
+    loader_loop<WS, true>(P, bars, base, gen, h, niter);
   } else {
     // ================= compute groups =================
     reg_alloc<200>();
     const int g = warp >> 2;
     const int r = threadIdx.x & 127;
     const int half = r >> 6, pos = r & 63;
-    const int pi = pos / 7, pj = pos % 7;
+    const int pi = pos / WS, pj = pos % WS;
     // second-stage results (M = 64 per window): this thread's TMEM lane holds row epos of window ehalf
     const int ehalf = lane >> 4, epos = 16 * (warp & 3) + (lane & 15);
-    const int epi_i = epos / 7, epi_j = epos % 7;
+    const int epi_i = epos / WS, epi_j = epos % WS;
     const uint32_t t0 = tmem + g * 256 + (static_cast<uint32_t>((warp & 3) * 32) << 16);
     uint8_t* Pb_g = gen + kBwdTiles + g * 32768;
     uint8_t* Db_g = Pb_g + 16384;
-    uint8_t* scratch = misc + kMiscScratch + warp * kScratchWarp;
-    const int bi = rpb_base(pos < kNTok ? pos : 0);
+    uint8_t* scratch = misc + M::kScratch + warp * kScratchWarp;
+    const int bi = rpb_base<WS>(pos < kNTok ? pos : 0);
     uint64_t far_h, far_w;
-    seam_sets(P.gm.shift, far_h, far_w);
+    seam_sets<WS>(P.gm.shift, far_h, far_w);
     float dtab[kNTok];
 #pragma unroll
     for (int j = 0; j < kNTok; ++j) dtab[j] = 0.f;
     CRF_PROF_DECL(8);
 
-    preload_bias(brow, pos, t0 + half * 64);
+    preload_row_bias<WS, true>(brow, tbl, pos, t0 + half * 64);
     tc_fence_before();
     mbar_arrive(bars.t_free(g));
 
     // per-pair row state, always computed one pair ahead (while the tensor core runs the second stage)
     auto row_state = [&](int pr, RowView& v, float& l, int& et) {
-      v = row_view(P, pr, half, pos, pi, pj, far_h, far_w);
+      v = row_view<WS>(P, pr, half, pos, pi, pj, far_h, far_w);
       l = 0.f;
       if (v.tok >= 0) l = __ldg(P.lse + (static_cast<int64_t>(v.wg) * P.nH + h) * 64 + pos);
       et = -2;
       const int ewg = 2 * pr + ehalf;
-      if (epos < kNTok && ewg < P.total_windows) et = window_token(P, window_pos(P, ewg), epi_i, epi_j);
+      if (epos < kNTok && ewg < P.total_windows) et = window_token<WS>(P, window_pos<WS>(P, ewg), epi_i, epi_j);
     };
     RowView rv;
     float lse;
@@ -744,7 +799,7 @@ attn_bwd_async_kernel(const AttnParams P) {
         }
         // dv and dk are on their way (64 of the 96 result registers are dead): pre-load the bias and hand the TMEM
         // columns back BEFORE the last store, so the next first-stage MMAs of this lane run under it
-        preload_bias(brow, pos, t0 + half * 64);
+        preload_row_bias<WS, true>(brow, tbl, pos, t0 + half * 64);
         tc_fence_before();
         mbar_arrive(bars.t_free(g));
         const float sc = P.scale;  // d(xW+b) = dq * scale because q was stored pre-scaled
@@ -768,14 +823,14 @@ attn_bwd_async_kernel(const AttnParams P) {
 
     // relative-position-bias gradient: dTable[idx(i,j), h] += sum over my pairs of dS[i][j]
     named_bar_sync(1, 256);  // both compute groups are past their last read of tbl
-    if (threadIdx.x < 176) tbl[threadIdx.x] = 0.f;
+    if (threadIdx.x < M::kTblFloats) tbl[threadIdx.x] = 0.f;
     named_bar_sync(1, 256);
     if (pos < kNTok) {
 #pragma unroll
-      for (int j = 0; j < kNTok; ++j) atomicAdd(tbl + bi - rpb_col(j), dtab[j]);
+      for (int j = 0; j < kNTok; ++j) atomicAdd(tbl + bi - rpb_col<WS>(j), dtab[j]);
     }
     named_bar_sync(1, 256);
-    if (threadIdx.x < 169) atomicAdd(P.d_table + threadIdx.x * P.nH + h, tbl[threadIdx.x]);
+    if (threadIdx.x < rpb_table_size(WS)) atomicAdd(P.d_table + threadIdx.x * P.nH + h, tbl[threadIdx.x]);
   }
 
   tc_fence_before();
@@ -792,30 +847,46 @@ int grid_x(const AttnParams& P, const crf_block_desc& d) {
   return gx < 1 ? 1 : gx;
 }
 
-}  // namespace
-
-int launch_attn_fwd_async(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
-  const size_t smem = kFwdMisc + kMiscBytes + 1024;
-  CRF_CUDA(cudaFuncSetAttribute(attn_fwd_async_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+template <int WS>
+int launch_fwd(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
+  constexpr size_t smem = kFwdMisc + Misc<WS, false>::kBytes + 1024;
+  static_assert(smem <= 232448, "shared-memory plan exceeds 227 KB");
+  CRF_CUDA(cudaFuncSetAttribute(attn_fwd_async_kernel<WS>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   const double TC = static_cast<double>(d.B) * d.H * d.W * d.C;
-  KernelTimer tm(st, 4.0 * 49 * 49 * d.C * P.total_windows, 8.0 * TC, "attn_fwd_B%d_%dx%d_C%d_s%d", d.B, d.H, d.W, d.C,
+  const double N = WS * WS;
+  KernelTimer tm(st, 4.0 * N * N * d.C * P.total_windows, 8.0 * TC, "attn_fwd_B%d_%dx%d_C%d_s%d", d.B, d.H, d.W, d.C,
                  d.shift);
-  launch_pdl(attn_fwd_async_kernel, dim3(grid_x(P, d), P.nH), kThreads, smem, st, P);
+  launch_pdl(attn_fwd_async_kernel<WS>, dim3(grid_x(P, d), P.nH), kThreads, smem, st, P);
   CRF_CUDA(cudaGetLastError());
   note_launch();
   return 0;
 }
 
-int launch_attn_bwd_async(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
-  const size_t smem = kBwdMisc + kMiscBytes + 1024;
-  CRF_CUDA(cudaFuncSetAttribute(attn_bwd_async_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+template <int WS>
+int launch_bwd(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
+  constexpr size_t smem = kBwdMisc + Misc<WS, true>::kBytes + 1024;
+  static_assert(smem <= 232448, "shared-memory plan exceeds 227 KB");
+  CRF_CUDA(cudaFuncSetAttribute(attn_bwd_async_kernel<WS>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   const double TC = static_cast<double>(d.B) * d.H * d.W * d.C;
-  KernelTimer tm(st, 10.0 * 49 * 49 * d.C * P.total_windows, 16.0 * TC, "attn_bwd_B%d_%dx%d_C%d_s%d", d.B, d.H, d.W,
+  const double N = WS * WS;
+  KernelTimer tm(st, 10.0 * N * N * d.C * P.total_windows, 16.0 * TC, "attn_bwd_B%d_%dx%d_C%d_s%d", d.B, d.H, d.W,
                  d.C, d.shift);
-  launch_pdl(attn_bwd_async_kernel, dim3(grid_x(P, d), P.nH), kThreads, smem, st, P);
+  launch_pdl(attn_bwd_async_kernel<WS>, dim3(grid_x(P, d), P.nH), kThreads, smem, st, P);
   CRF_CUDA(cudaGetLastError());
   note_launch();
   return 0;
+}
+
+}  // namespace
+
+int launch_attn_fwd_async(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
+  const int rc = with_window(P.gm.ws, [&](auto w) { return launch_fwd<decltype(w)::value>(P, d, st); });
+  return rc >= 0 ? rc : set_error("attention core: no kernel for window %d", P.gm.ws);
+}
+
+int launch_attn_bwd_async(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
+  const int rc = with_window(P.gm.ws, [&](auto w) { return launch_bwd<decltype(w)::value>(P, d, st); });
+  return rc >= 0 ? rc : set_error("attention core: no kernel for window %d", P.gm.ws);
 }
 
 }  // namespace crf

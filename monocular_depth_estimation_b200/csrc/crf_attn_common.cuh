@@ -7,8 +7,6 @@
 
 namespace crf {
 
-constexpr int kNTok = 49;
-
 struct AttnParams {
   WindowGeom gm;
   int B, C, nH;
@@ -18,9 +16,9 @@ struct AttnParams {
   const __nv_bfloat16* qk;   // (T, 2C)
   const __nv_bfloat16* vb;   // (T, C)
   const float* qk_bias;      // (2C)
-  const float* table;        // (169, nH)
+  const float* table;        // ((2ws-1)^2, nH)
   float scale;
-  const float* ext_mask;     // optional additive mask (nwm, 49, 49) f32, window index = global window % nwm; or nullptr
+  const float* ext_mask;     // optional additive mask (nwm, N, N) f32 (N = ws^2), window index = global window % nwm; or nullptr
   int ext_mask_nw;
   int ext_replaces;          // 1: ext_mask REPLACES the closed-form shift mask (CRFBlock.forward's mask_matrix); 0: added on top
   // forward
@@ -31,15 +29,11 @@ struct AttnParams {
   __nv_bfloat16* dqk;        // (T, 2C)
   float* dv;                 // (T, C)
   int dv_acc;
-  float* d_table;            // (169, nH)
+  float* d_table;            // ((2ws-1)^2, nH)
   float* d_qk_bias;          // (2C)
   float rcp_nW, rcp_nWw;     // 1 / windows per image, 1 / windows per row (fast exact division in the kernels)
   int prof;                  // development: block (0,0) prints per-phase cycle counts (CRF_ATTN_PROF=1)
 };
-
-// relative_position_index[i][j] = (yi - yj + 6) * 13 + (xi - xj + 6)   (newcrf_layers.py:90-99)
-__device__ __forceinline__ int rpb_base(int pos) { return (pos / 7) * 13 + (pos % 7) + 84; }
-__host__ __device__ constexpr int rpb_col(int j) { return (j / 7) * 13 + (j % 7); }
 
 // register re-balancing between warp-specialised roles (whole warpgroups execute these)
 template <int N>

@@ -32,11 +32,12 @@ constexpr int kWideThreads = 160;  // warps 0-3: one thread per tile row; warp 4
 constexpr int kTile = 8192;        // one 128-row x 64-byte SW64 slice tile
 
 // Token index of tile row r of a window pair: >= 0 real token, -1 zero-pad token, -2 dead row.
+template <int WS>
 __device__ __forceinline__ int row_token(const AttnParams& P, int pair, int r, int& window_global, int& pos) {
   const int half = r >> 6;
   pos = r & 63;
   window_global = 2 * pair + half;
-  if (pos >= kNTok || window_global >= P.total_windows) return -2;
+  if (pos >= WS * WS || window_global >= P.total_windows) return -2;
   const int b = window_global / P.gm.nW;
   const int win = window_global - b * P.gm.nW;
   const int src = P.gm.source(win, pos);
@@ -62,34 +63,36 @@ __device__ __forceinline__ void bias_row64(uint8_t* tile_gen, int r, const float
   }
 }
 
-template <int NS>
+template <int NS, int WS>
 struct WideFwd {
   static constexpr int kQ = 0, kK = NS * kTile, kV = 2 * NS * kTile, kP = 3 * NS * kTile;  // P: 128 x 128 B SW128
   static constexpr int kMisc = kP + 16384;                                                  // tbl | rid | bars | tmem ptr
+  static constexpr int kTbl = rpb_table_padded(WS);                                         // 176 floats at WS = 7
   static constexpr int kTmemCols = NS == 2 ? 256 : 512;  // S [0,128) + O_s [128 + 64 s, 128 + 64 s + 64)
   // head_dim 64: pad the request to 80 KB so that at most two CTAs (2 x 256 TMEM columns) share an SM
-  static constexpr int kSmem = (kMisc + 176 * 4 + 128 + 32 + 1024) < 81920 ? 81920 : (kMisc + 176 * 4 + 128 + 32 + 1024);
+  static constexpr int kSmem = (kMisc + kTbl * 4 + 128 + 32 + 1024) < 81920 ? 81920 : (kMisc + kTbl * 4 + 128 + 32 + 1024);
 };
 
 // ------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------
-template <int NS>
+template <int NS, int WS>
 __global__ void __launch_bounds__(kWideThreads)
 attn_fwd_wide_kernel(const AttnParams P) {
-  using L = WideFwd<NS>;
+  using L = WideFwd<NS, WS>;
+  constexpr int kNTok = WS * WS;
   constexpr int HD = 32 * NS;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
   const uint32_t Qs = base + L::kQ, Ks = base + L::kK, Vs = base + L::kV, Ps = base + L::kP;
   uint8_t* Ps_gen = gen + L::kP;
-  float* tbl = reinterpret_cast<float*>(gen + L::kMisc);  // 176 floats
-  uint8_t* rid = gen + L::kMisc + 176 * 4;                // 128 bytes
-  const uint32_t bar_s = base + L::kMisc + 176 * 4 + 128;
+  float* tbl = reinterpret_cast<float*>(gen + L::kMisc);  // L::kTbl floats
+  uint8_t* rid = gen + L::kMisc + L::kTbl * 4;                // 128 bytes
+  const uint32_t bar_s = base + L::kMisc + L::kTbl * 4 + 128;
   const uint32_t bar_o = bar_s + 8;
   const uint32_t tmem_ptr_addr = bar_s + 16;
-  volatile uint32_t* tmem_ptr_gen = reinterpret_cast<volatile uint32_t*>(gen + L::kMisc + 176 * 4 + 128 + 16);
+  volatile uint32_t* tmem_ptr_gen = reinterpret_cast<volatile uint32_t*>(gen + L::kMisc + L::kTbl * 4 + 128 + 16);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int h = blockIdx.y;
@@ -105,7 +108,7 @@ attn_fwd_wide_kernel(const AttnParams P) {
     tmem_alloc(tmem_ptr_addr, L::kTmemCols);
     tmem_relinquish();
   }
-  for (int i = threadIdx.x; i < 169; i += kWideThreads) tbl[i] = __ldg(P.table + i * P.nH + h);
+  for (int i = threadIdx.x; i < rpb_table_size(WS); i += kWideThreads) tbl[i] = __ldg(P.table + i * P.nH + h);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -120,7 +123,7 @@ attn_fwd_wide_kernel(const AttnParams P) {
     const int r = threadIdx.x;
     // ---- phase 0: gather the NS slices of this head's Q, K, V rows ----
     if (warp < 4) {
-      tok = row_token(P, pair, r, wg, pos);
+      tok = row_token<WS>(P, pair, r, wg, pos);
       if (tok >= 0) {
         const __nv_bfloat16* qrow = P.qk + static_cast<int64_t>(tok) * 2 * C + h * HD;
         const __nv_bfloat16* vrow = P.vb + static_cast<int64_t>(tok) * C + h * HD;
@@ -176,7 +179,7 @@ attn_fwd_wide_kernel(const AttnParams P) {
       tmem_ld_wait();
       float p[64];
       if (tok != -2) {
-        const int bi = rpb_base(pos);
+        const int bi = rpb_base<WS>(pos);
         const uint8_t* rrow = rid + half * 64;
         const int my_region = rrow[pos];
         const bool masked = P.gm.shift > 0 && !P.ext_replaces;
@@ -186,7 +189,7 @@ attn_fwd_wide_kernel(const AttnParams P) {
         float mx = -INFINITY;
 #pragma unroll
         for (int j = 0; j < kNTok; ++j) {
-          float s = __uint_as_float(j < 32 ? s0[j & 31] : s1[j & 31]) + tbl[bi - rpb_col(j)];
+          float s = __uint_as_float(j < 32 ? s0[j & 31] : s1[j & 31]) + tbl[bi - rpb_col<WS>(j)];
           if (masked && rrow[j] != my_region) s += -100.0f;
           if (xmask != nullptr) s += __ldg(xmask + j);
           p[j] = s;
@@ -269,34 +272,36 @@ attn_fwd_wide_kernel(const AttnParams P) {
 // ------------------------------------------------------------------------------------------------
 // backward
 // ------------------------------------------------------------------------------------------------
-template <int NS>
+template <int NS, int WS>
 struct WideBwd {
   // Q, K, V, dO: NS slice tiles each; Pbd, dSbd: 2 x 16 KB each (two SW128 column chunks of 128 rows)
   static constexpr int kQ = 0, kK = NS * kTile, kV = 2 * NS * kTile, kG = 3 * NS * kTile;
   static constexpr int kPb = 4 * NS * kTile, kDb = kPb + 32768;
   static constexpr int kMisc = kDb + 32768;
+  static constexpr int kTbl = rpb_table_padded(WS);      // 176 floats at WS = 7
   static constexpr int kTmemCols = NS == 2 ? 256 : 512;  // S [0,128), dP [128,256); then dV_s | dK_s | dQ_s at 96 s
-  static constexpr int kSmem = kMisc + 176 * 4 + 128 + 32 + 1024;
+  static constexpr int kSmem = kMisc + kTbl * 4 + 128 + 32 + 1024;
   static_assert(kSmem <= 232448, "shared-memory plan exceeds 227 KB");
   static_assert(96 * NS <= kTmemCols, "second-stage results do not fit the TMEM allocation");
 };
 
-template <int NS>
+template <int NS, int WS>
 __global__ void __launch_bounds__(kWideThreads)
 attn_bwd_wide_kernel(const AttnParams P) {
-  using L = WideBwd<NS>;
+  using L = WideBwd<NS, WS>;
+  constexpr int kNTok = WS * WS;
   constexpr int HD = 32 * NS;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (base - smem_u32(smem_raw));
   const uint32_t Qs = base + L::kQ, Ks = base + L::kK, Vs = base + L::kV, Gs = base + L::kG;
   const uint32_t Pb = base + L::kPb, Db = base + L::kDb;
-  float* tbl = reinterpret_cast<float*>(gen + L::kMisc);  // 176 floats
-  uint8_t* rid = gen + L::kMisc + 176 * 4;                // 128 bytes
-  const uint32_t bar_s = base + L::kMisc + 176 * 4 + 128;
+  float* tbl = reinterpret_cast<float*>(gen + L::kMisc);  // L::kTbl floats
+  uint8_t* rid = gen + L::kMisc + L::kTbl * 4;                // 128 bytes
+  const uint32_t bar_s = base + L::kMisc + L::kTbl * 4 + 128;
   const uint32_t bar_o = bar_s + 8;
   const uint32_t tmem_ptr_addr = bar_s + 16;
-  volatile uint32_t* tmem_ptr_gen = reinterpret_cast<volatile uint32_t*>(gen + L::kMisc + 176 * 4 + 128 + 16);
+  volatile uint32_t* tmem_ptr_gen = reinterpret_cast<volatile uint32_t*>(gen + L::kMisc + L::kTbl * 4 + 128 + 16);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int h = blockIdx.y;
@@ -312,7 +317,7 @@ attn_bwd_wide_kernel(const AttnParams P) {
     tmem_alloc(tmem_ptr_addr, L::kTmemCols);
     tmem_relinquish();
   }
-  for (int i = threadIdx.x; i < 169; i += kWideThreads) tbl[i] = __ldg(P.table + i * P.nH + h);
+  for (int i = threadIdx.x; i < rpb_table_size(WS); i += kWideThreads) tbl[i] = __ldg(P.table + i * P.nH + h);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -332,7 +337,7 @@ attn_bwd_wide_kernel(const AttnParams P) {
     int tok = -2, wg = 0, pos = 0;
     const int r = threadIdx.x;
     if (warp < 4) {
-      tok = row_token(P, pair, r, wg, pos);
+      tok = row_token<WS>(P, pair, r, wg, pos);
       if (tok >= 0) {
         const __nv_bfloat16* qrow = P.qk + static_cast<int64_t>(tok) * 2 * C + h * HD;
         const __nv_bfloat16* vrow = P.vb + static_cast<int64_t>(tok) * C + h * HD;
@@ -399,7 +404,7 @@ attn_bwd_wide_kernel(const AttnParams P) {
         tmem_ld_wait();
         if (tok >= 0) {
           const float lse = __ldg(P.lse + (static_cast<int64_t>(wg) * P.nH + h) * 64 + pos);
-          const int bi = rpb_base(pos);
+          const int bi = rpb_base<WS>(pos);
           const uint8_t* rrow = rid + half * 64;
           const int my_region = rrow[pos];
           const bool masked = P.gm.shift > 0 && !P.ext_replaces;
@@ -408,7 +413,7 @@ attn_bwd_wide_kernel(const AttnParams P) {
                                    : nullptr;
 #pragma unroll
           for (int j = 0; j < kNTok; ++j) {
-            float s = __uint_as_float(j < 32 ? s0[j & 31] : s1[j & 31]) + tbl[bi - rpb_col(j)];
+            float s = __uint_as_float(j < 32 ? s0[j & 31] : s1[j & 31]) + tbl[bi - rpb_col<WS>(j)];
             if (masked && rrow[j] != my_region) s += -100.0f;
             if (xmask != nullptr) s += __ldg(xmask + j);
             p[j] = __expf(s - lse);
@@ -537,15 +542,15 @@ attn_bwd_wide_kernel(const AttnParams P) {
   // flush the relative-position-bias gradient: dTable[idx(i,j), h] += sum_windows dS[i][j]
   __syncthreads();
   float* dt = tbl;  // reuse as the CTA-level accumulator
-  for (int i = threadIdx.x; i < 176; i += kWideThreads) dt[i] = 0.f;
+  for (int i = threadIdx.x; i < L::kTbl; i += kWideThreads) dt[i] = 0.f;
   __syncthreads();
   if (warp < 4 && my_pos < kNTok) {
-    const int bi = rpb_base(my_pos);
+    const int bi = rpb_base<WS>(my_pos);
 #pragma unroll
-    for (int j = 0; j < kNTok; ++j) atomicAdd(dt + bi - rpb_col(j), dtab[j]);
+    for (int j = 0; j < kNTok; ++j) atomicAdd(dt + bi - rpb_col<WS>(j), dtab[j]);
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < 169; i += kWideThreads) atomicAdd(P.d_table + i * P.nH + h, dt[i]);
+  for (int i = threadIdx.x; i < rpb_table_size(WS); i += kWideThreads) atomicAdd(P.d_table + i * P.nH + h, dt[i]);
 
   tc_fence_before();
   __syncthreads();
@@ -561,13 +566,14 @@ int wide_grid_x(const AttnParams& P, const crf_block_desc& d, int ctas_per_sm) {
   return gx < 1 ? 1 : gx;
 }
 
-template <int NS>
+template <int NS, int WS>
 int launch_fwd(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
-  auto kern = attn_fwd_wide_kernel<NS>;
-  constexpr int smem = WideFwd<NS>::kSmem;
+  auto kern = attn_fwd_wide_kernel<NS, WS>;
+  constexpr int smem = WideFwd<NS, WS>::kSmem;
+  const double N = WS * WS;
   CRF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   const double TC = static_cast<double>(d.B) * d.H * d.W * d.C;
-  KernelTimer tm(st, 4.0 * 49 * 49 * d.C * P.total_windows, 8.0 * TC, "attn_fwd_wide_B%d_%dx%d_C%d_h%d_s%d", d.B, d.H,
+  KernelTimer tm(st, 4.0 * N * N * d.C * P.total_windows, 8.0 * TC, "attn_fwd_wide_B%d_%dx%d_C%d_h%d_s%d", d.B, d.H,
                  d.W, d.C, P.nH, d.shift);
   kern<<<dim3(wide_grid_x(P, d, NS == 2 ? 2 : 1), P.nH), kWideThreads, smem, st>>>(P);
   CRF_CUDA(cudaGetLastError());
@@ -575,13 +581,14 @@ int launch_fwd(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
   return 0;
 }
 
-template <int NS>
+template <int NS, int WS>
 int launch_bwd(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
-  auto kern = attn_bwd_wide_kernel<NS>;
-  constexpr int smem = WideBwd<NS>::kSmem;
+  auto kern = attn_bwd_wide_kernel<NS, WS>;
+  constexpr int smem = WideBwd<NS, WS>::kSmem;
+  const double N = WS * WS;
   CRF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   const double TC = static_cast<double>(d.B) * d.H * d.W * d.C;
-  KernelTimer tm(st, 10.0 * 49 * 49 * d.C * P.total_windows, 16.0 * TC, "attn_bwd_wide_B%d_%dx%d_C%d_h%d_s%d", d.B,
+  KernelTimer tm(st, 10.0 * N * N * d.C * P.total_windows, 16.0 * TC, "attn_bwd_wide_B%d_%dx%d_C%d_h%d_s%d", d.B,
                  d.H, d.W, d.C, P.nH, d.shift);
   kern<<<dim3(wide_grid_x(P, d, 1), P.nH), kWideThreads, smem, st>>>(P);
   CRF_CUDA(cudaGetLastError());
@@ -592,15 +599,19 @@ int launch_bwd(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
 }  // namespace
 
 int launch_attn_fwd_wide(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
-  if (P.hd == 64) return launch_fwd<2>(P, d, st);
-  if (P.hd == 128) return launch_fwd<4>(P, d, st);
-  return set_error("wide attention core: head_dim must be 64 or 128 (got %d)", P.hd);
+  if (P.hd != 64 && P.hd != 128) return set_error("wide attention core: head_dim must be 64 or 128 (got %d)", P.hd);
+  const int rc = with_window(P.gm.ws, [&](auto w) {
+    return P.hd == 64 ? launch_fwd<2, decltype(w)::value>(P, d, st) : launch_fwd<4, decltype(w)::value>(P, d, st);
+  });
+  return rc >= 0 ? rc : set_error("wide attention core: no kernel for window %d", P.gm.ws);
 }
 
 int launch_attn_bwd_wide(const AttnParams& P, const crf_block_desc& d, cudaStream_t st) {
-  if (P.hd == 64) return launch_bwd<2>(P, d, st);
-  if (P.hd == 128) return launch_bwd<4>(P, d, st);
-  return set_error("wide attention core: head_dim must be 64 or 128 (got %d)", P.hd);
+  if (P.hd != 64 && P.hd != 128) return set_error("wide attention core: head_dim must be 64 or 128 (got %d)", P.hd);
+  const int rc = with_window(P.gm.ws, [&](auto w) {
+    return P.hd == 64 ? launch_bwd<2, decltype(w)::value>(P, d, st) : launch_bwd<4, decltype(w)::value>(P, d, st);
+  });
+  return rc >= 0 ? rc : set_error("wide attention core: no kernel for window %d", P.gm.ws);
 }
 
 }  // namespace crf

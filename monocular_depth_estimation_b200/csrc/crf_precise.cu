@@ -25,9 +25,6 @@ namespace crf {
 
 namespace {
 
-constexpr int kN = 49;   // tokens per window (window 7)
-constexpr int kPS = 50;  // row stride of the 49 x 49 score tiles in shared memory
-
 inline size_t align_up(size_t v) { return (v + 255) & ~static_cast<size_t>(255); }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -105,8 +102,8 @@ struct AttnF32 {
   int v_bf16;
   int64_t vsb, vsh, vsw, vsc;
   const float* qk_bias;   // (2C): q / k of a zero-pad token (LayerNorm output is padded with zeros AFTER the norm)
-  const float* table;     // (169, nH)
-  const float* ext_mask;  // (ext_nw, 49, 49) additive or nullptr (closed-form shift mask)
+  const float* table;     // ((2ws-1)^2, nH)
+  const float* ext_mask;  // (ext_nw, N, N) additive or nullptr (closed-form shift mask), N = ws^2
   int ext_nw;
   float scale;
   int B, H, W, C, nH, hd;
@@ -118,7 +115,7 @@ struct AttnF32 {
   float* dqk;             // (T, 2C)
   float* dv;              // (B, H, W, C) contiguous
   int dv_acc;
-  float* d_table;         // (169, nH), +=
+  float* d_table;         // ((2ws-1)^2, nH), +=
   float* d_qk_bias;       // (2C), += (pad keys)
 };
 
@@ -127,17 +124,23 @@ __device__ __forceinline__ float load_v(const AttnF32& P, int b, int tok, int c)
   const int64_t off = b * P.vsb + h * P.vsh + w * P.vsw + c * P.vsc;
   return P.v_bf16 ? __bfloat162float(static_cast<const __nv_bfloat16*>(P.v)[off]) : static_cast<const float*>(P.v)[off];
 }
-__device__ __forceinline__ int rel_index(int i, int j) {  // newcrf_layers.py:90-100
-  return (i / 7 - j / 7 + 6) * 13 + (i % 7 - j % 7 + 6);
-}
+// Per window size WS: kN = WS^2 tokens per window, kPS = kN + 1 the row stride of the kN x kN score tiles in shared
+// memory, kTbl floats for a head's relative-position table (49 / 50 / 176 at WS = 7).
+template <int WS>
+struct Win {
+  static constexpr int kN = WS * WS;
+  static constexpr int kPS = kN + 1;
+  static constexpr int kTbl = rpb_table_padded(WS);
+};
 
 // Gathers the window's q (scaled), k, v (and dO) rows of one head into shared memory; tok[n] = token index or -1.
-template <bool BWD>
+template <int WS, bool BWD>
 __device__ void attn_gather(const AttnF32& P, int b, int win, int head, float* q, float* k, float* v, float* dO, int* tok,
                             float* tb) {
+  constexpr int kN = Win<WS>::kN;
   const int hd = P.hd, hs = hd + 1, C = P.C;
   for (int n = threadIdx.x; n < kN; n += blockDim.x) tok[n] = P.gm.source(win, n);
-  for (int t = threadIdx.x; t < 169; t += blockDim.x) tb[t] = P.table[t * P.nH + head];
+  for (int t = threadIdx.x; t < rpb_table_size(WS); t += blockDim.x) tb[t] = P.table[t * P.nH + head];
   __syncthreads();
   for (int idx = threadIdx.x; idx < kN * hd; idx += blockDim.x) {
     const int n = idx / hd, d = idx - n * hd, c = head * hd + d;
@@ -163,8 +166,10 @@ __device__ void attn_gather(const AttnF32& P, int b, int win, int head, float* q
 }
 
 // scores of query row i -> p[i][.] = softmax_j(q_i . k_j + bias + mask)
+template <int WS>
 __device__ void attn_softmax_row(const AttnF32& P, int wg, int win, int i, const float* q, const float* k, const float* tb,
                                  float* p) {
+  constexpr int kN = Win<WS>::kN, kPS = Win<WS>::kPS;
   const int hd = P.hd, hs = hd + 1;
   const float* xmask = P.ext_mask != nullptr ? P.ext_mask + (static_cast<int64_t>(wg % P.ext_nw) * kN + i) * kN : nullptr;
   const int ri = (P.gm.shift > 0 && xmask == nullptr) ? P.gm.region(win, i) : 0;
@@ -172,7 +177,7 @@ __device__ void attn_softmax_row(const AttnF32& P, int wg, int win, int i, const
   for (int j = 0; j < kN; ++j) {
     float s = 0.f;
     for (int d = 0; d < hd; ++d) s = fmaf(q[i * hs + d], k[j * hs + d], s);
-    s += tb[rel_index(i, j)];
+    s += tb[rel_position_index<WS>(i, j)];
     if (xmask != nullptr) s += xmask[j];
     else if (P.gm.shift > 0 && P.gm.region(win, j) != ri) s += -100.0f;  // newcrf_layers.py:350
     p[i * kPS + j] = s;
@@ -188,8 +193,10 @@ __device__ void attn_softmax_row(const AttnF32& P, int wg, int win, int i, const
   for (int j = 0; j < kN; ++j) p[i * kPS + j] *= inv;
 }
 
+template <int WS>
 __global__ void __launch_bounds__(64)
 attn_fwd_f32_kernel(const AttnF32 P) {
+  constexpr int kN = Win<WS>::kN, kPS = Win<WS>::kPS;
   extern __shared__ float sm[];
   const int hd = P.hd, hs = hd + 1;
   float* q = sm;
@@ -197,13 +204,13 @@ attn_fwd_f32_kernel(const AttnF32 P) {
   float* v = k + kN * hs;
   float* p = v + kN * hs;
   float* tb = p + kN * kPS;
-  int* tok = reinterpret_cast<int*>(tb + 176);
+  int* tok = reinterpret_cast<int*>(tb + Win<WS>::kTbl);
   const int wg = blockIdx.x, head = blockIdx.y;
   const int b = wg / P.gm.nW, win = wg - b * P.gm.nW;
-  attn_gather<false>(P, b, win, head, q, k, v, nullptr, tok, tb);
+  attn_gather<WS, false>(P, b, win, head, q, k, v, nullptr, tok, tb);
   const int i = threadIdx.x;
   if (i < kN) {
-    attn_softmax_row(P, wg, win, i, q, k, tb, p);
+    attn_softmax_row<WS>(P, wg, win, i, q, k, tb, p);
     if (tok[i] >= 0) {  // pad queries are dropped by the crop (newcrf_layers.py:248-249)
       float* o = P.out + (static_cast<int64_t>(b) * P.H * P.W + tok[i]) * P.C + head * hd;
       for (int d = 0; d < hd; ++d) {
@@ -215,8 +222,10 @@ attn_fwd_f32_kernel(const AttnF32 P) {
   }
 }
 
+template <int WS>
 __global__ void __launch_bounds__(64)
 attn_bwd_f32_kernel(const AttnF32 P) {
+  constexpr int kN = Win<WS>::kN, kPS = Win<WS>::kPS;
   extern __shared__ float sm[];
   const int hd = P.hd, hs = hd + 1, C = P.C;
   float* q = sm;
@@ -226,15 +235,15 @@ attn_bwd_f32_kernel(const AttnF32 P) {
   float* p = dO + kN * hs;
   float* ds = p + kN * kPS;
   float* tb = ds + kN * kPS;
-  float* tg = tb + 176;
-  int* tok = reinterpret_cast<int*>(tg + 176);
+  float* tg = tb + Win<WS>::kTbl;
+  int* tok = reinterpret_cast<int*>(tg + Win<WS>::kTbl);
   const int wg = blockIdx.x, head = blockIdx.y;
   const int b = wg / P.gm.nW, win = wg - b * P.gm.nW;
-  for (int t = threadIdx.x; t < 169; t += blockDim.x) tg[t] = 0.f;
-  attn_gather<true>(P, b, win, head, q, k, v, dO, tok, tb);
+  for (int t = threadIdx.x; t < rpb_table_size(WS); t += blockDim.x) tg[t] = 0.f;
+  attn_gather<WS, true>(P, b, win, head, q, k, v, dO, tok, tb);
   const int i = threadIdx.x;
   if (i < kN) {
-    attn_softmax_row(P, wg, win, i, q, k, tb, p);
+    attn_softmax_row<WS>(P, wg, win, i, q, k, tb, p);
     // dP = dO V^T ; dS = P o (dP - sum_j P dP)
     float dot = 0.f;
     for (int j = 0; j < kN; ++j) {
@@ -246,7 +255,7 @@ attn_bwd_f32_kernel(const AttnF32 P) {
     for (int j = 0; j < kN; ++j) {
       const float g = p[i * kPS + j] * (ds[i * kPS + j] - dot);
       ds[i * kPS + j] = g;
-      if (g != 0.f) atomicAdd(&tg[rel_index(i, j)], g);
+      if (g != 0.f) atomicAdd(&tg[rel_position_index<WS>(i, j)], g);
     }
     if (tok[i] >= 0) {  // dq = scale * dS K   (gradient of the UNSCALED q the qk projection produced)
       float* dq = P.dqk + (static_cast<int64_t>(b) * P.H * P.W + tok[i]) * 2 * C + head * hd;
@@ -278,13 +287,15 @@ attn_bwd_f32_kernel(const AttnF32 P) {
       }
     }
   }
-  for (int t = threadIdx.x; t < 169; t += blockDim.x)
+  for (int t = threadIdx.x; t < rpb_table_size(WS); t += blockDim.x)
     if (tg[t] != 0.f) atomicAdd(P.d_table + t * P.nH + head, tg[t]);
 }
 
+template <int WS>
 size_t attn_smem(int hd, bool bwd) {
+  constexpr int kN = Win<WS>::kN, kPS = Win<WS>::kPS, kTbl = Win<WS>::kTbl;
   const size_t rows = static_cast<size_t>(kN) * (hd + 1);
-  return ((bwd ? 4 : 3) * rows + (bwd ? 2 : 1) * kN * kPS + (bwd ? 352 : 176) + 64) * sizeof(float);
+  return ((bwd ? 4 : 3) * rows + (bwd ? 2 : 1) * kN * kPS + (bwd ? 2 * kTbl : kTbl) + 64) * sizeof(float);
 }
 
 AttnF32 attn_params(const crf_block_desc& d, const crf_block_params& p, const float* qk, const void* v) {
@@ -303,33 +314,44 @@ AttnF32 attn_params(const crf_block_desc& d, const crf_block_params& p, const fl
   return P;
 }
 
+template <int WS>
+int attn_fwd_f32(const crf_block_desc& d, const AttnF32& P, cudaStream_t st) {
+  const size_t smem = attn_smem<WS>(P.hd, false);
+  CRF_CUDA(cudaFuncSetAttribute(attn_fwd_f32_kernel<WS>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  const double T = static_cast<double>(d.B) * d.H * d.W, N = WS * WS;
+  KernelTimer tm(st, 4.0 * N * N * d.C * d.B * P.gm.nW, T * d.C * 16.0, "attn_fwd_f32_B%d_%dx%d_C%d_s%d", d.B, d.H, d.W, d.C,
+                 d.shift);
+  attn_fwd_f32_kernel<WS><<<dim3(d.B * P.gm.nW, d.num_heads), 64, smem, st>>>(P);
+  CRF_CUDA(cudaGetLastError());
+  note_launch();
+  return 0;
+}
+template <int WS>
+int attn_bwd_f32(const crf_block_desc& d, const AttnF32& P, cudaStream_t st) {
+  const size_t smem = attn_smem<WS>(P.hd, true);
+  CRF_CUDA(cudaFuncSetAttribute(attn_bwd_f32_kernel<WS>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  const double T = static_cast<double>(d.B) * d.H * d.W, N = WS * WS;
+  KernelTimer tm(st, 10.0 * N * N * d.C * d.B * P.gm.nW, T * d.C * 32.0, "attn_bwd_f32_B%d_%dx%d_C%d_s%d", d.B, d.H, d.W, d.C,
+                 d.shift);
+  attn_bwd_f32_kernel<WS><<<dim3(d.B * P.gm.nW, d.num_heads), 64, smem, st>>>(P);
+  CRF_CUDA(cudaGetLastError());
+  note_launch();
+  return 0;
+}
+
 int launch_attn_fwd_f32(const crf_block_desc& d, const crf_block_params& p, const float* qk, const void* v, float* out,
                         cudaStream_t st) {
   AttnF32 P = attn_params(d, p, qk, v);
   P.out = out;
-  const size_t smem = attn_smem(P.hd, false);
-  CRF_CUDA(cudaFuncSetAttribute(attn_fwd_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  const double T = static_cast<double>(d.B) * d.H * d.W;
-  KernelTimer tm(st, 4.0 * 49 * 49 * d.C * d.B * P.gm.nW, T * d.C * 16.0, "attn_fwd_f32_B%d_%dx%d_C%d_s%d", d.B, d.H, d.W, d.C,
-                 d.shift);
-  attn_fwd_f32_kernel<<<dim3(d.B * P.gm.nW, d.num_heads), 64, smem, st>>>(P);
-  CRF_CUDA(cudaGetLastError());
-  note_launch();
-  return 0;
+  const int rc = with_window(d.window, [&](auto w) { return attn_fwd_f32<decltype(w)::value>(d, P, st); });
+  return rc >= 0 ? rc : set_error("fp32 attention: no kernel for window %d", d.window);
 }
 int launch_attn_bwd_f32(const crf_block_desc& d, const crf_block_params& p, const float* qk, const void* v, const float* dout,
                         float* dqk, float* dv, int dv_acc, float* d_table, float* d_qk_bias, cudaStream_t st) {
   AttnF32 P = attn_params(d, p, qk, v);
   P.dout = dout; P.dqk = dqk; P.dv = dv; P.dv_acc = dv_acc; P.d_table = d_table; P.d_qk_bias = d_qk_bias;
-  const size_t smem = attn_smem(P.hd, true);
-  CRF_CUDA(cudaFuncSetAttribute(attn_bwd_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  const double T = static_cast<double>(d.B) * d.H * d.W;
-  KernelTimer tm(st, 10.0 * 49 * 49 * d.C * d.B * P.gm.nW, T * d.C * 32.0, "attn_bwd_f32_B%d_%dx%d_C%d_s%d", d.B, d.H, d.W, d.C,
-                 d.shift);
-  attn_bwd_f32_kernel<<<dim3(d.B * P.gm.nW, d.num_heads), 64, smem, st>>>(P);
-  CRF_CUDA(cudaGetLastError());
-  note_launch();
-  return 0;
+  const int rc = with_window(d.window, [&](auto w) { return attn_bwd_f32<decltype(w)::value>(d, P, st); });
+  return rc >= 0 ? rc : set_error("fp32 attention: no kernel for window %d", d.window);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

@@ -138,8 +138,8 @@ def crf_block(x, v, H, W, params, num_heads, *, window=7, shift=0, qk_scale=None
 
     x: (B, H*W, C) fp32/bf16, any strides (the reference hands over a view of NCHW); v: (B, H, W, C);
     params: 13 fp32 tensors in PARAM_KEYS order; v_bf16: optional result of convert_v(v) shared between blocks;
-    mask: None = the shifted-window mask of BasicCRFLayer.forward in closed form, else an additive (nW, 49, 49) mask that
-    replaces it; precision: "bf16" | "fp32" | None (process default, ops.set_precision).
+    window: 2..8; mask: None = the shifted-window mask of BasicCRFLayer.forward in closed form, else an additive
+    (nW, N, N) mask (N = window^2) that replaces it; precision: "bf16" | "fp32" | None (process default, ops.set_precision).
     Returns (B, H*W, C) fp32.  Mirrors the reference's error behaviour (newcrf_layers.py:205,143,180).
     """
     assert x.dim() == 3 and v.dim() == 4
@@ -398,7 +398,7 @@ def pixel_shuffle2(x):
 
 class _WindowAttentionFn(torch.autograd.Function):
     """Stand-alone WindowAttention.forward (newcrf_layers.py:110-149) on already-partitioned windows, built from the
-    stage-level entry points: qk GEMM -> attention core (each window = a 7x7 image, no pad, no shift) -> proj GEMM."""
+    stage-level entry points: qk GEMM -> attention core (each window = a ws x ws image, no pad, no shift) -> proj GEMM."""
 
     @staticmethod
     def forward(ctx, x, v, mask, num_heads, scale, qk_w, qk_b, table, proj_w, proj_b):
@@ -412,7 +412,8 @@ class _WindowAttentionFn(torch.autograd.Function):
         qkb, pb = qk_b.detach().contiguous(), proj_b.detach().contiguous()
         tab = table.detach().contiguous()
         m = None if mask is None else mask.detach().float().contiguous()
-        desc = make_desc(B_, 7, 7, Cd, num_heads, 0, device=dev.index)
+        ws = _window_of(N)
+        desc = make_desc(B_, ws, ws, Cd, num_heads, 0, window=ws, device=dev.index)
         qk = torch.empty(T, 2 * Cd, dtype=torch.bfloat16, device=dev)
         ops.gemm(xb, wqk, T, 2 * Cd, Cd, epilogue=L.EPI_STORE_BF16, out0=qk, bias=qkb, scale=scale, scale_cols=Cd)
         o, lse = ops.attn_fwd(desc, qk, vb, qkb, scale, tab, want_lse=True, mask=m)
@@ -428,7 +429,8 @@ class _WindowAttentionFn(torch.autograd.Function):
         xb, vb, wqk, wp, qkb, tab, qk, o, lse, m = ctx.saved_tensors
         B_, N, Cd, num_heads, scale, has_mask = ctx.meta
         T, dev = B_ * N, xb.device
-        desc = make_desc(B_, 7, 7, Cd, num_heads, 0, device=dev.index)
+        ws = _window_of(N)
+        desc = make_desc(B_, ws, ws, Cd, num_heads, 0, window=ws, device=dev.index)
         dob = ops.cast_bf16(dout.contiguous().float().reshape(T, Cd))
         d_o = torch.empty(T, Cd, dtype=torch.bfloat16, device=dev)
         ops.gemm(dob, wp, T, Cd, Cd, b_major=1, epilogue=L.EPI_STORE_BF16, out0=d_o)
@@ -442,9 +444,20 @@ class _WindowAttentionFn(torch.autograd.Function):
         return (dx.view(B_, N, Cd), dv.view(B_, N, Cd), None, None, None, d_wqk, d_qkb, d_tab, d_wp, d_pb)
 
 
+MIN_WINDOW, MAX_WINDOW = 2, 8   # window sizes the attention kernels implement (N = ws^2 <= 64 tokens per window)
+
+
+def _window_of(N):
+    """The window size ws of an N = ws * ws token window, or None."""
+    ws = int(round(N ** 0.5))
+    return ws if ws * ws == N and MIN_WINDOW <= ws <= MAX_WINDOW else None
+
+
 def window_attention(x, v, qk_w, qk_b, table, proj_w, proj_b, num_heads, scale, mask=None):
-    """WindowAttention.forward(x, v, mask): x, v (num_windows*B, 49, C); mask (nW, 49, 49) or None -> (B_, 49, C) fp32."""
-    assert x.dim() == 3 and x.shape[1] == 49, "window attention expects (num_windows*B, 49, C) windows of 7x7 tokens"
+    """WindowAttention.forward(x, v, mask): x, v (num_windows*B, N, C) windows of ws x ws tokens (N = ws^2, ws in 2..8);
+    mask (nW, N, N) or None -> (B_, N, C) fp32."""
+    assert x.dim() == 3 and _window_of(x.shape[1]) is not None, \
+        f"window attention expects (num_windows*B, ws*ws, C) windows with ws in {MIN_WINDOW}..{MAX_WINDOW}"
     assert x.shape[-1] == v.shape[-1], "self.dim != v.shape[-1]"
     if not x.is_cuda:
         raise RuntimeError("monocular_depth_estimation_b200 runs on CUDA (sm_100a) only; there is no CPU path")

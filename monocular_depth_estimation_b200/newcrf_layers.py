@@ -28,6 +28,12 @@ def _pair(v):
     return v if isinstance(v, tuple) else (v, v)
 
 
+def _require_window(window_size):
+    if not CF.MIN_WINDOW <= window_size <= CF.MAX_WINDOW:
+        raise NotImplementedError(f"window_size={window_size}: the sm_100a attention kernels implement window sizes "
+                                  f"{CF.MIN_WINDOW} to {CF.MAX_WINDOW} (a window's ws*ws tokens fill at most 64 tile rows)")
+
+
 def _require_zero(name, rate):
     if rate != 0.0:
         raise NotImplementedError(f"{name}={rate}: the fused sm_100a CRF block implements the reference's "
@@ -82,7 +88,7 @@ class WindowAttention(nn.Module):
         self.softmax = nn.Softmax(dim=-1)
 
     def forward(self, x, v, mask=None):
-        """x, v: (num_windows*B, 49, C) pre-partitioned windows; mask: (nW, 49, 49) additive or None.
+        """x, v: (num_windows*B, N, C) pre-partitioned windows, N = ws*ws; mask: (nW, N, N) additive or None.
         The fused CRFBlock never materialises windows and does not call this; it exists for drop-in use of the class
         on its own (qk GEMM -> attention core -> proj GEMM through the stage-level entry points)."""
         return CF.window_attention(x, v, self.qk.weight, self.qk.bias, self.relative_position_bias_table,
@@ -94,6 +100,7 @@ class CRFBlock(nn.Module):
                  drop=0., attn_drop=0., drop_path=0., act_layer=nn.GELU, norm_layer=nn.LayerNorm):
         super().__init__()
         _require_zero("drop_path", drop_path)
+        _require_window(window_size)
         if norm_layer is not nn.LayerNorm:
             raise NotImplementedError("only nn.LayerNorm is implemented")
         assert 0 <= shift_size < window_size, "shift_size must in 0-window_size"
@@ -140,7 +147,7 @@ class CRFBlock(nn.Module):
 
     def forward(self, x, v, mask_matrix=None, v_bf16=None):
         """x: (B, H*W, C); v: (B, H, W, C); self.H / self.W set by the caller (as BasicCRFLayer does).
-        mask_matrix: the (nW, 49, 49) additive mask of a shifted block.  The standard one (what BasicCRFLayer.forward
+        mask_matrix: the (nW, N, N) additive mask of a shifted block (N = window_size^2).  The standard one (what BasicCRFLayer.forward
         builds) is recognised and evaluated in closed form inside the kernels; any other mask is honoured as given."""
         H, W = self.H, self.W
         B, Ltok, _ = x.shape
@@ -157,6 +164,7 @@ class BasicCRFLayer(nn.Module):
         super().__init__()
         if downsample is not None:
             raise NotImplementedError("downsample is always None in the reference (newcrf_layers.py:411)")
+        _require_window(window_size)
         self.window_size = window_size
         self.shift_size = window_size // 2
         self.depth = depth

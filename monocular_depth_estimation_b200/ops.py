@@ -214,8 +214,9 @@ def shift_mask(H, W, window, shift, device):
 
 def attn_fwd(desc, qk, vb, qk_bias, scale, table, want_lse=True, mask=None):
     T, Cd = vb.shape
-    Hp, Wp = -(-desc.H // 7) * 7, -(-desc.W // 7) * 7
-    nW = (Hp // 7) * (Wp // 7)
+    ws = desc.window
+    Hp, Wp = -(-desc.H // ws) * ws, -(-desc.W // ws) * ws
+    nW = (Hp // ws) * (Wp // ws)
     o = torch.zeros(T, Cd, dtype=torch.bfloat16, device=vb.device)
     lse = torch.zeros(desc.B * nW, desc.num_heads, 64, dtype=torch.float32, device=vb.device) if want_lse else None
     L.check(L.lib().crf_attn_fwd(C.byref(desc), _ptr(qk), _ptr(vb), _ptr(qk_bias), scale, _ptr(table), _ptr(mask),
