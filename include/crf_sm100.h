@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define CRF_ABI_VERSION 3
+#define CRF_ABI_VERSION 4
 enum { CRF_PREC_BF16 = 0, CRF_PREC_FP32 = 1 };
 
 enum { CRF_DT_F32 = 0, CRF_DT_BF16 = 1 };
@@ -206,7 +206,8 @@ typedef struct crf_gemm_args {
   int64_t ld_out;          /* row stride (elements) of out0/out1/aux1 */
   float scale; int32_t scale_cols;
   int32_t device;
-  void* workspace;         /* CRF_EPI_SPLITK_F32: fp32 partial tiles (crf_gemm_workspace_bytes) or NULL */
+  void* workspace;         /* CRF_EPI_SPLITK_F32 with CRF_WGRAD_DETERMINISTIC=1: fp32 partial tiles
+                            * (crf_gemm_workspace_bytes) or NULL.  Not read by any other GEMM. */
   size_t workspace_bytes;
   float* colsum;           /* MN-major A only: colsum[m] += sum_k A(m,k) (bias gradient fused into wgrad), or NULL */
   int32_t split3;          /* 1: split-operand fp32 emulation.  A and B hold fp32 values as two bf16 terms side by side,
@@ -216,10 +217,6 @@ typedef struct crf_gemm_args {
 int crf_gemm(const crf_gemm_args* a, void* stream);
 /* workspace a CRF_EPI_SPLITK_F32 GEMM of this shape wants (0 when it runs as a single split) */
 size_t crf_gemm_workspace_bytes(int M, int N, int K, int device);
-/* Scratch (flags + one 256 x 256 fp32 partial tile per SM pair) that lets the fprop / dgrad GEMMs of the wide decoder
- * scales (N % 256 == 0, K >= 512: the CTA-pair kernel) run STREAM-K: pass it as crf_gemm_args.workspace with a
- * non-split-K epilogue.  Without it those GEMMs run whole tiles in rounds of (SMs / 2).  Contents are scratch. */
-size_t crf_gemm_streamk_bytes(int device);
 
 /* The MLP half of a block in ONE kernel (C = 128 or 256):  y = x1 + fc2(GELU(fc1(LayerNorm(x1))))
  * (replaces `x + self.mlp(self.norm2(x))`, /root/reference/src/newcrf_layers.py:255, Mlp.forward :21-27).

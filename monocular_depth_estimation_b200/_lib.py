@@ -27,7 +27,7 @@ EPI_SPLITK_F32 = 5
 EXPORTED_SYMBOLS = (
     "crf_last_error", "crf_abi_version", "crf_kernel_launches", "crf_timing_enable", "crf_timing_report", "crf_block_sizes", "crf_block_fwd", "crf_block_bwd", "crf_convert_v",
     "crf_layer_sizes", "crf_layer_fwd", "crf_layer_bwd",
-    "crf_window_gather", "crf_window_scatter", "crf_shift_mask", "crf_gemm", "crf_mlp_fwd", "crf_gemm_workspace_bytes", "crf_gemm_streamk_bytes", "crf_ln_fwd", "crf_ln_bwd", "crf_dgrad_ln_bwd",
+    "crf_window_gather", "crf_window_scatter", "crf_shift_mask", "crf_gemm", "crf_mlp_fwd", "crf_gemm_workspace_bytes", "crf_ln_fwd", "crf_ln_bwd", "crf_dgrad_ln_bwd",
     "crf_layernorm_fwd", "crf_layernorm_bwd", "crf_layernorm_ps_fwd", "crf_layernorm_ps_bwd", "crf_depth_loss_fwd", "crf_depth_loss_bwd", "crf_pixel_shuffle_nhwc",
     "crf_colsum_bf16", "crf_cast_bf16", "crf_attn_fwd", "crf_attn_bwd", "crf_adam_step",
 )
@@ -121,8 +121,6 @@ def _declare(lib):
     lib.crf_mlp_fwd.argtypes = [C.POINTER(MlpArgs), vp]
     lib.crf_gemm_workspace_bytes.restype = sz
     lib.crf_gemm_workspace_bytes.argtypes = [i32, i32, i32, i32]
-    lib.crf_gemm_streamk_bytes.restype = sz
-    lib.crf_gemm_streamk_bytes.argtypes = [i32]
     lib.crf_ln_fwd.argtypes = [vp, i32, i64, i64, i64, i32, i32, i32, vp, vp, f32, vp, vp, vp, i32, vp]
     lib.crf_ln_bwd.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]
     lib.crf_dgrad_ln_bwd.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]
@@ -139,8 +137,7 @@ def _declare(lib):
     lib.crf_attn_fwd.argtypes = [C.POINTER(BlockDesc), vp, vp, vp, f32, vp, vp, i32, vp, vp, vp]
     lib.crf_attn_bwd.argtypes = [C.POINTER(BlockDesc), vp, vp, vp, f32, vp, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp]
     for name in EXPORTED_SYMBOLS:
-        if name not in ("crf_last_error", "crf_kernel_launches", "crf_timing_report", "crf_gemm_workspace_bytes",
-                        "crf_gemm_streamk_bytes"):
+        if name not in ("crf_last_error", "crf_kernel_launches", "crf_timing_report", "crf_gemm_workspace_bytes"):
             getattr(lib, name).restype = i32
     lib.crf_kernel_launches.restype = C.c_longlong
     lib.crf_kernel_launches.argtypes = []

@@ -1,7 +1,5 @@
 // extern "C" entry points of libcrf_sm100.so (see include/crf_sm100.h) and the per-block orchestration:
 // which kernels run, in what order, on which slices of the caller-provided `saved` / workspace buffers.
-#include <stdlib.h>
-
 #include "crf_host.h"
 #include "crf_window.cuh"
 
@@ -12,30 +10,12 @@ inline size_t align_up(size_t v) { return (v + 255) & ~static_cast<size_t>(255);
 
 // Layout of the `saved` buffer (forward products backward needs) -- offsets in bytes.
 struct SavedLayout {
-  size_t xc, stats1, xn1, qk, vb, lse, attn_o, x1, stats2, xn2, pre, act, wb_qk, wb_proj, wb_fc1, wb_fc2, sk, sk_bytes, total;
+  size_t xc, stats1, xn1, qk, vb, lse, attn_o, x1, stats2, xn2, pre, act, wb_qk, wb_proj, wb_fc1, wb_fc2, total;
 };
 // Layout of the backward workspace.
 struct BwdLayout {
   size_t dyb, dhpre, dxn, dx1, dx1b, dob, dqk, partials, partials_bytes, total;
 };
-
-bool fused_mlp_enabled() {
-  static const bool on = [] { const char* e = getenv("CRF_FUSED_MLP"); return e == nullptr || e[0] != '0'; }();
-  return on;
-}
-
-// stream-K scratch for the CTA-pair GEMMs: measured not to pay (crf_gemm_pair.cu), so only on request
-bool streamk_enabled() {
-  static const bool on = [] { const char* e = getenv("CRF_GEMM_STREAMK"); return e != nullptr && e[0] == '1'; }();
-  return on;
-}
-
-// d fc1 / d qk GEMM with the LayerNorm backward in its epilogue (crf_dgrad_lnbwd.cu); CRF_FUSED_LNBWD=0 restores the
-// GEMM + ln_bwd kernel pairs
-bool fused_lnbwd_enabled() {
-  static const bool on = [] { const char* e = getenv("CRF_FUSED_LNBWD"); return e == nullptr || e[0] != '0'; }();
-  return on;
-}
 
 // v already is what the attention kernels read: bf16 rows, token-major, contiguous (the channels-last output of the
 // proj_v convolution under bf16 autocast) -- the layer then uses it in place instead of making the bf16 copy
@@ -72,9 +52,6 @@ SavedLayout saved_layout(const crf_block_desc& d) {
   L.wb_proj = take(C * C * 2);
   L.wb_fc1 = take(4 * C * C * 2);
   L.wb_fc2 = take(4 * C * C * 2);
-  // stream-K partial tiles of the CTA-pair GEMMs (C >= 512: the projections that run on crf_gemm_pair.cu); scratch only
-  L.sk_bytes = (C >= 512 && streamk_enabled()) ? gemm_pair_streamk_bytes(d.device) : 0;
-  L.sk = take(L.sk_bytes);
   L.total = o;
   return L;
 }
@@ -100,7 +77,6 @@ BwdLayout bwd_layout(const crf_block_desc& d) {
     const size_t b = gemm_splitk_workspace_bytes(s[0], s[1], Ti, d.device, nullptr);
     if (b > pb) pb = b;
   }
-  if (Ci >= 512 && streamk_enabled() && gemm_pair_streamk_bytes(d.device) > pb) pb = gemm_pair_streamk_bytes(d.device);
   L.partials_bytes = pb;
   L.partials = take(pb);
   L.total = o;
@@ -122,10 +98,8 @@ int check_desc(const crf_block_desc* d) {
 }
 
 int gemm_fprop(const void* A, const void* W, int M, int N, int K, int epi, void* out0, void* out1, const float* bias,
-               const void* aux1, float scale, int scale_cols, int device, cudaStream_t st, void* ws = nullptr,
-               size_t ws_bytes = 0) {
+               const void* aux1, float scale, int scale_cols, int device, cudaStream_t st) {
   crf_gemm_args a{};
-  a.workspace = ws; a.workspace_bytes = ws_bytes;
   a.A = A; a.B = W; a.a_major = 0; a.b_major = 0;
   a.M = M; a.N = N; a.K = K; a.epilogue = epi; a.split_k = 1;
   a.out0 = out0; a.out1 = out1; a.bias = bias; a.aux1 = aux1; a.ld_out = N;
@@ -134,9 +108,8 @@ int gemm_fprop(const void* A, const void* W, int M, int N, int K, int epi, void*
 }
 // dX[M=T, N=Cin] = dY[T, K=Cout] * W[Cout, Cin]
 int gemm_dgrad(const void* dY, const void* W, int M, int N, int K, int epi, void* out0, const void* aux1, int device,
-               cudaStream_t st, void* ws = nullptr, size_t ws_bytes = 0) {
+               cudaStream_t st) {
   crf_gemm_args a{};
-  a.workspace = ws; a.workspace_bytes = ws_bytes;
   a.A = dY; a.B = W; a.a_major = 0; a.b_major = 1;
   a.M = M; a.N = N; a.K = K; a.epilogue = epi; a.split_k = 1;
   a.out0 = out0; a.aux1 = aux1; a.ld_out = N; a.scale = 1.f; a.scale_cols = 0; a.device = device;
@@ -224,7 +197,7 @@ static int block_fwd_impl(const crf_block_desc* d, const crf_block_params* p, co
   }
   // q (scaled) and k
   if (gemm_fprop(S + L.xn1, S + L.wb_qk, T, 2 * C, C, CRF_EPI_STORE_BF16, S + L.qk, nullptr, p->qk_b, nullptr,
-                 p->qk_scale, C, d->device, st, S + L.sk, L.sk_bytes))
+                 p->qk_scale, C, d->device, st))
     return 1;
   // window attention core
   if (launch_attn_fwd(*d, S + L.qk, vb, p->qk_b, p->qk_scale, p->rpb_table, p->ext_mask, p->ext_mask_windows,
@@ -232,11 +205,10 @@ static int block_fwd_impl(const crf_block_desc* d, const crf_block_params* p, co
     return 1;
   // x1 = x + proj(attn)
   if (gemm_fprop(S + L.attn_o, S + L.wb_proj, T, C, C, CRF_EPI_BIAS_RES_F32, S + L.x1, nullptr, p->proj_b, x_tok, 1.f,
-                 0, d->device, st, S + L.sk, L.sk_bytes))
+                 0, d->device, st))
     return 1;
-  // LN2 + MLP + residual in one kernel where the fused kernel exists (C = 128, 256; CRF_FUSED_MLP=0 restores the
-  // three-kernel path below)
-  if (mlp_fused_supported(C) && fused_mlp_enabled()) {
+  // LN2 + MLP + residual in one kernel where the fused kernel exists (C = 128, 256), else the three kernels below
+  if (mlp_fused_supported(C)) {
     crf_mlp_args m{};
     m.x1 = reinterpret_cast<const float*>(S + L.x1); m.y = y;
     m.w1_bf16 = S + L.wb_fc1; m.w2_bf16 = S + L.wb_fc2;
@@ -252,10 +224,10 @@ static int block_fwd_impl(const crf_block_desc* d, const crf_block_params* p, co
     return 1;
   // MLP
   if (gemm_fprop(S + L.xn2, S + L.wb_fc1, T, 4 * C, C, CRF_EPI_BIAS_GELU, d->training ? S + L.pre : nullptr, S + L.act,
-                 p->fc1_b, nullptr, 1.f, 0, d->device, st, S + L.sk, L.sk_bytes))
+                 p->fc1_b, nullptr, 1.f, 0, d->device, st))
     return 1;
   if (gemm_fprop(S + L.act, S + L.wb_fc2, T, C, 4 * C, CRF_EPI_BIAS_RES_F32, y, nullptr, p->fc2_b, S + L.x1, 1.f, 0,
-                 d->device, st, S + L.sk, L.sk_bytes))
+                 d->device, st))
     return 1;
   return 0;
 }
@@ -288,24 +260,22 @@ static int block_bwd_impl(const crf_block_desc* d, const crf_block_params* p, co
   float* dxn = reinterpret_cast<float*>(Wk + W.dxn);
   float* dx1 = reinterpret_cast<float*>(Wk + W.dx1);
 
-  void* sk_ws = streamk_enabled() ? static_cast<void*>(Wk + W.partials) : nullptr;
-  const size_t sk_bytes = streamk_enabled() ? W.partials_bytes : 0;
   // ---- MLP ----
   const void* dyb = dy_bf16;
   if (dyb == nullptr) {
     if (launch_cast_bf16(dy, Wk + W.dyb, static_cast<int64_t>(T) * C, st)) return 1;
     dyb = Wk + W.dyb;
   }
-  if (gemm_dgrad(dyb, S + L.wb_fc2, T, 4 * C, C, CRF_EPI_MUL_DGELU, Wk + W.dhpre, S + L.pre, dev, st, sk_ws, sk_bytes)) return 1;
+  if (gemm_dgrad(dyb, S + L.wb_fc2, T, 4 * C, C, CRF_EPI_MUL_DGELU, Wk + W.dhpre, S + L.pre, dev, st)) return 1;
   if (gemm_wgrad(dyb, S + L.act, C, 4 * C, T, g->fc2_w, g->fc2_b, Wk + W.partials, W.partials_bytes, dev, st)) return 1;
-  const bool fuse_ln = fused_lnbwd_enabled() && dgrad_lnbwd_supported(C, 2 * C);
+  const bool fuse_ln = dgrad_lnbwd_supported(C, 2 * C);
   if (fuse_ln) {  // dx1 = dy + LN2'(dhpre W1) straight from the GEMM's accumulator rows
     if (launch_dgrad_lnbwd(Wk + W.dhpre, S + L.wb_fc1, 4 * C, reinterpret_cast<const float*>(S + L.x1),
                            reinterpret_cast<const float*>(S + L.stats2), p->norm2_w, dy, dx1, Wk + W.dx1b, g->norm2_w,
                            g->norm2_b, T, C, dev, st))
       return 1;
   } else {
-    if (gemm_dgrad(Wk + W.dhpre, S + L.wb_fc1, T, C, 4 * C, CRF_EPI_STORE_F32, dxn, nullptr, dev, st, sk_ws, sk_bytes)) return 1;
+    if (gemm_dgrad(Wk + W.dhpre, S + L.wb_fc1, T, C, 4 * C, CRF_EPI_STORE_F32, dxn, nullptr, dev, st)) return 1;
   }
   if (gemm_wgrad(Wk + W.dhpre, S + L.xn2, 4 * C, C, T, g->fc1_w, g->fc1_b, Wk + W.partials, W.partials_bytes, dev, st)) return 1;
   if (!fuse_ln &&
@@ -313,7 +283,7 @@ static int block_bwd_impl(const crf_block_desc* d, const crf_block_params* p, co
                     p->norm2_w, dy, dx1, Wk + W.dx1b, g->norm2_w, g->norm2_b, T, C, st))
     return 1;
   // ---- attention ----
-  if (gemm_dgrad(Wk + W.dx1b, S + L.wb_proj, T, C, C, CRF_EPI_STORE_BF16, Wk + W.dob, nullptr, dev, st, sk_ws, sk_bytes)) return 1;
+  if (gemm_dgrad(Wk + W.dx1b, S + L.wb_proj, T, C, C, CRF_EPI_STORE_BF16, Wk + W.dob, nullptr, dev, st)) return 1;
   if (gemm_wgrad(Wk + W.dx1b, S + L.attn_o, C, C, T, g->proj_w, g->proj_b, Wk + W.partials, W.partials_bytes, dev, st)) return 1;
   if (launch_attn_bwd(*d, S + L.qk, vb, p->qk_b, p->qk_scale, p->rpb_table, p->ext_mask, p->ext_mask_windows,
                       reinterpret_cast<const float*>(S + L.lse),
@@ -324,7 +294,7 @@ static int block_bwd_impl(const crf_block_desc* d, const crf_block_params* p, co
                            dx1, dx, dx_bf16, g->norm1_w, g->norm1_b, T, C, dev, st))
       return 1;
   } else {
-    if (gemm_dgrad(Wk + W.dqk, S + L.wb_qk, T, C, 2 * C, CRF_EPI_STORE_F32, dxn, nullptr, dev, st, sk_ws, sk_bytes)) return 1;
+    if (gemm_dgrad(Wk + W.dqk, S + L.wb_qk, T, C, 2 * C, CRF_EPI_STORE_F32, dxn, nullptr, dev, st)) return 1;
   }
   if (gemm_wgrad(Wk + W.dqk, S + L.xn1, 2 * C, C, T, g->qk_w, g->qk_b, Wk + W.partials, W.partials_bytes, dev, st)) return 1;
   if (!fuse_ln &&
@@ -575,8 +545,6 @@ int crf_dgrad_ln_bwd(const void* dy_bf16, const void* w_bf16, int K, const float
   return launch_dgrad_lnbwd(dy_bf16, w_bf16, K, x, stats, gamma, dres, dx, dx_bf16, dgamma, dbeta, T, C, device,
                             static_cast<cudaStream_t>(stream));
 }
-
-size_t crf_gemm_streamk_bytes(int device) { return gemm_pair_streamk_bytes(device); }
 
 int crf_gemm(const crf_gemm_args* a, void* stream) {
   CRF_CHECK(a && a->A && a->B && (a->out0 || a->out1), "crf_gemm: null pointer");

@@ -24,9 +24,6 @@
 // follows the output stores in pass 2).
 //
 // Algorithmic bytes per token: 2K (dY) + 4C (x) + 4C (dres) + 4C (dx) + 2C (bf16 twin); flops 2 K C.
-#include <stdio.h>
-#include <stdlib.h>
-
 #include "crf_host.h"
 #include "crf_ptx.cuh"
 #include "crf_sched.h"
@@ -39,7 +36,7 @@ constexpr int TM = 128, BK = 64;
 constexpr int kThreads = 352;   // 8 epilogue warps, A/B producer, MMA issuer, slab producer
 constexpr int kSlab = TM * 128;     // 16 KB: 128 rows x 32 fp32 (or x 64 bf16)
 
-// Shared-memory plan (runtime stage counts: n_ring A/B stages, n_slab slab stages; CRF_LNBWD_STAGES=ring,slab overrides)
+// Shared-memory plan (runtime stage counts: n_ring A/B stages, n_slab slab stages)
 constexpr int kMaxStages = 6;
 template <int C>
 struct LnPlan {
@@ -381,11 +378,7 @@ int launch_c(const void* dY, const void* W, int K, const float* x, const float* 
   // so that the tiles fill whole rounds of the persistent grid (T = 38400: 300 tiles of 128 rows are 2.03 rounds on 148
   // SMs, i.e. 3; 437 tiles of 88 rows are 2.95 rounds of a shorter tile: -31 % row-time).
   const int sms = num_sms(device);
-  int tm = balanced_tile_rows(T, sms);
-  {
-    static const bool fixed = getenv("CRF_LNBWD_TM128") != nullptr;
-    if (fixed) tm = TM;
-  }
+  const int tm = balanced_tile_rows(T, sms);
   if (make_tmap_bf16(&tmA, dY, T, K, tm)) return 1;
   if (make_tmap_bf16(&tmB, W, K, C, 64)) return 1;
   if (make_tmap_f32(&tmX, x, T, C, tm)) return 1;
@@ -395,15 +388,7 @@ int launch_c(const void* dY, const void* W, int K, const float* x, const float* 
   if (dx_bf16 != nullptr && make_tmap_bf16(&tmDxb, dx_bf16, T, C, tm)) return 1;
   auto kern = dgrad_lnbwd_kernel<C>;
   // stages (measured: the counts hardly matter once >= 2): 96 KB of A/B ring + 4 slab stages
-  int n_ring = C <= 128 ? 3 : 2, n_slab = 4;
-  if (const char* e = getenv("CRF_LNBWD_STAGES")) {
-    int r_ = 0, s_ = 0;
-    if (sscanf(e, "%d,%d", &r_, &s_) == 2 && r_ >= 2 && r_ <= kMaxStages && s_ >= 2 && s_ <= kMaxStages &&
-        PL::bytes(r_, s_) <= 232448) {
-      n_ring = r_;
-      n_slab = s_;
-    }
-  }
+  const int n_ring = C <= 128 ? 3 : 2, n_slab = 4;
   const int smem_bytes = PL::bytes(n_ring, n_slab);
   CRF_CHECK(smem_bytes <= 232448, "dgrad_lnbwd: shared-memory plan exceeds 227 KB");
   CRF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));

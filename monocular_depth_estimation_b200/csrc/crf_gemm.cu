@@ -273,7 +273,6 @@ int launch_one(const Launch& L, const crf_gemm_args& a, cudaStream_t st) {
   // conversions, HBM stores), so favour residency: 128-wide tiles with a 2-stage ring = 3 CTAs per SM whose
   // main loops and epilogues interleave (measured: -0.5 ms per training step vs 256-wide tiles, 2 CTAs per SM).
   int stages = a.a_major == 1 ? ((L.cps >= 8) ? (BN == 256 ? 4 : 6) : (BN == 256 ? 2 : 3)) : 2;
-  if (const char* e = getenv("CRF_GEMM_STAGES")) stages = atoi(e);  // development knob
   if (stages > L.cps) stages = L.cps < 2 ? 2 : L.cps;
   size_t ring = static_cast<size_t>(stages) * kStageBytes;
   if (ring < 4u * kSlabBytes) ring = 4u * kSlabBytes;
@@ -343,21 +342,14 @@ int launch_gemm(const crf_gemm_args& a, cudaStream_t st) {
   CRF_CHECK(a.a_major == 1 || a.K % 8 == 0, "crf_gemm: K-major A needs K %% 8 == 0 (K=%d)", a.K);
   CRF_CHECK(a.a_major == 0 || a.M % 8 == 0, "crf_gemm: MN-major A needs M %% 8 == 0 (M=%d)", a.M);
   CRF_CHECK(a.ld_out == a.N, "crf_gemm: outputs must be dense (ld_out == N)");
-  {  // token-major projections with N % 128 == 0 run on the persistent kernel (crf_gemm_persist.cu)
-    static const bool persist = !(getenv("CRF_GEMM_PERSIST") && atoi(getenv("CRF_GEMM_PERSIST")) == 0);
-    if (persist && !a.split3) {
-      const int rc2 = launch_gemm_pair(a, st);
-      if (rc2 >= 0) return rc2;
-      const int rc = launch_gemm_persistent(a, st);
-      if (rc >= 0) return rc;
-    }
+  if (!a.split3) {  // token-major projections: CTA-pair kernel, else the persistent kernel where the shape is eligible
+    const int rc2 = launch_gemm_pair(a, st);
+    if (rc2 >= 0) return rc2;
+    const int rc = launch_gemm_persistent(a, st);
+    if (rc >= 0) return rc;
   }
   int BN = (a.N % 256 == 0) ? 256 : (a.N % 128 == 0 ? 128 : 64);
   if (a.a_major == 0 && BN > 128) BN = 128;
-  if (const char* e = getenv("CRF_GEMM_BN")) {  // development knob: cap the tile width
-    const int cap = atoi(e);
-    if (a.epilogue != CRF_EPI_SPLITK_F32 && (cap == 64 || cap == 128) && cap < BN) BN = cap;
-  }
 
   Launch L{};
   const int dup = a.split3 ? 2 : 1;  // split-operand matrices are twice as wide: [hi | lo]

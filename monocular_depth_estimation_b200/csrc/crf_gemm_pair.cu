@@ -14,10 +14,7 @@
 //   both CTAs    warps 0-7  epilogue, two groups of four warps (column halves), thread = accumulator row, the same slab
 //                         epilogues as the single-CTA kernel (crf_gemm_epi.cuh); TMEM hand-back = one remote mbarrier
 //                         arrival per warp on the leader's `tmem_empty` barrier
-#include <stdlib.h>
-
 #include "crf_gemm_epi.cuh"
-#include "crf_sched.h"
 
 namespace crf {
 
@@ -35,31 +32,12 @@ constexpr int kNumBars = 2 * kStages + 2 + 2 + 2;       // full, empty, tmem_ful
 constexpr int kSmemBytes = kBarOff + 8 * kNumBars + 16 + 1024;
 static_assert(kSmemBytes <= 232448, "shared-memory plan exceeds 227 KB");
 
-// ---- work decomposition -------------------------------------------------------------------------------------------
-// classic : pair p takes whole tiles p, p + npairs, ...  (rounds of 74 tiles: 40 / 76 / 80 / 152 / 160 tiles quantise badly)
-// stream-K: the tiles x K-chunks sequence (tile-major) is cut into npairs equal contiguous ranges.  A range starts with
-//           the TAIL of a tile another pair began (a "contributor" piece: the fp32 partial accumulator goes to this pair's
-//           workspace slot, then a flag is released), continues with whole tiles and ends with the HEAD of a tile (an
-//           "owner" piece: after its own K chunks the pair adds the partials of the pairs that hold the rest of the tile,
-//           then runs the ordinary epilogue).  A contributor piece is always the FIRST piece of its pair and waits for
-//           nothing, an owner piece is the LAST of its pair, so the flags are long set when they are needed and no pair
-//           ever waits on a pair that waits (CTAs are dispatched in index order; all 74 pairs are resident).
-// (Piece, PieceIter, sk_bound, sk_contributors: crf_sched.h -- compiled on the host by tests/test_sched_host.py)
-__device__ __forceinline__ uint32_t ld_acquire_gpu(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void st_release_gpu(uint32_t* p, uint32_t v) {
-  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
+// Pair p takes whole tiles p, p + npairs, ... in the producer, the MMA issuer and the epilogue alike.
 template <int EPI>
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmO0, const __grid_constant__ CUtensorMap tmO1,
-                 const __grid_constant__ CUtensorMap tmAux, int M, int N, int K, int b_major, EpiParams ep, int streamk,
-                 int snap, float* sk_ws, uint32_t* sk_flags) {
+                 const __grid_constant__ CUtensorMap tmAux, int M, int N, int K, int b_major, EpiParams ep) {
   pdl_launch_dependents();
   using TR = EpiTraits<EPI>;
   constexpr int kSlabCols = TR::kSlabCols;
@@ -115,13 +93,10 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     // ===== TMA producer (both CTAs): A rows [m0 + 128 rank, +128), B columns [n0 + 128 rank, +128) =====
     if (lane == 0) {
       int it = 0;
-      PieceIter pit(nk_all, total_tiles, pair, npairs, streamk, snap);
-      Piece pc;
-      while (pit.next(pc)) {
-        const int t = pc.t;
+      for (int t = pair; t < total_tiles; t += npairs) {
         const int m0 = (t / n_tiles) * PM + 128 * static_cast<int>(rank);
         const int n0 = (t % n_tiles) * PN + 128 * static_cast<int>(rank);
-        for (int kc = pc.kc0; kc < pc.kc1; ++kc, ++it) {
+        for (int kc = 0; kc < nk_all; ++kc, ++it) {
           const int s = it % kStages;
           if (it >= kStages) mbar_wait(empty_bar(s), ((it / kStages) - 1) & 1);
           const uint32_t a_dst = base + s * kStage, b_dst = a_dst + kATile;
@@ -141,17 +116,14 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     if (lane == 0 && rank == 0) {
       const uint32_t idesc = make_idesc(1u, 0u, static_cast<uint32_t>(b_major), PM, PN);
       int it = 0;
-      PieceIter pit(nk_all, total_tiles, pair, npairs, streamk, snap);
-      Piece pc;
-      for (int i = 0; pit.next(pc); ++i) {
+      for (int t = pair, i = 0; t < total_tiles; t += npairs, ++i) {
         const int a = i & 1;
         if (i >= 2) {
           mbar_wait(tempty_bar(a), ((i >> 1) - 1) & 1);   // both CTAs' epilogues have drained this accumulator
           tc_fence_after();
         }
         const uint32_t d_tmem = tmem_base + a * PN;
-        const int kc0 = pc.kc0, kc1 = pc.kc1;
-        for (int kc = kc0; kc < kc1; ++kc, ++it) {
+        for (int kc = 0; kc < nk_all; ++kc, ++it) {
           const int s = it % kStages;
           mbar_wait(full_bar(s), (it / kStages) & 1);
           tc_fence_after();
@@ -161,7 +133,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             const uint64_t ad = make_smem_desc(a_src + ks * 32, 16, 1024, kSwizzle128);
             const uint64_t bd = (b_major == 0) ? make_smem_desc(b_src + ks * 32, 16, 1024, kSwizzle128)
                                                : make_smem_desc(b_src + ks * 2048, 8192, 1024, kSwizzle128);
-            umma_bf16_2sm(d_tmem, ad, bd, idesc, (kc > kc0 || ks > 0) ? 1u : 0u);
+            umma_bf16_2sm(d_tmem, ad, bd, idesc, (kc > 0 || ks > 0) ? 1u : 0u);
           }
           umma_commit_2sm(empty_bar(s), 3);   // frees the stage in both CTAs
         }
@@ -177,66 +149,22 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     uint8_t* xb = o0 + kSlab;
     const uint32_t lane_base = static_cast<uint32_t>((warp & 3) * 32) << 16;
     int aux_cnt = 0;
-    // stream-K partial slots: [pair][rank][group] x (32 column quads x 128 rows x float4) -- a warp's accesses are contiguous
-    constexpr int kSlotFloats = 128 * 128;
-    PieceIter pit(nk_all, total_tiles, pair, npairs, streamk, snap);
-    Piece pc;
-    for (int i = 0; pit.next(pc); ++i) {
-      const int t = pc.t;
-      const bool emits = pc.kc0 == 0;                  // this pair owns the tile: it runs the real epilogue
-      const bool head = emits && pc.kc1 < nk_all;      // ... after adding the partials of the pairs that finish the tile
+    for (int t = pair, i = 0; t < total_tiles; t += npairs, ++i) {
       const int a = i & 1;
       const int m0 = (t / n_tiles) * PM + 128 * static_cast<int>(rank);
       const int n0 = (t % n_tiles) * PN + 128 * e;
       const uint32_t taddr = tmem_base + a * PN + e * 128 + lane_base;
-      if (TR::kHasAux && emits && r == 0) {
+      if (TR::kHasAux && r == 0) {
         mbar_expect_tx(aux_bar(e), kSlab);
         tma_load_2d(x_s, &tmAux, aux_bar(e), n0, m0);
       }
-      // contributors of an owner piece: the pairs whose (first) piece covers the rest of this tile
-      int n_contrib = 0;
-      const float* contrib[kMaxContrib];
-      if (head) {
-        int q[kMaxContrib];
-        n_contrib = sk_contributors(pair, npairs, total_tiles, nk_all, snap, t, pc.kc1, q);
-        if (n_contrib < 0) n_contrib = 0;   // (the host only selects stream-K for shapes where this cannot happen)
-        for (int k = 0; k < n_contrib; ++k) {
-          const int slot = (q[k] * 2 + static_cast<int>(rank)) * 2 + e;
-          if (r == 0) {
-            while (ld_acquire_gpu(sk_flags + slot) == 0u) __nanosleep(64);
-          }
-          contrib[k] = sk_ws + static_cast<size_t>(slot) * kSlotFloats;
-        }
-      }
       mbar_wait(tfull_bar(a), (i >> 1) & 1);
       tc_fence_after();
-      if (!emits) {
-        // ---- contributor piece: bare fp32 partial accumulator -> this pair's workspace slot, then release the flag ----
-        const int slot = (pair * 2 + static_cast<int>(rank)) * 2 + e;
-        float4* dst = reinterpret_cast<float4*>(sk_ws + static_cast<size_t>(slot) * kSlotFloats) + r;
-#pragma unroll 1
-        for (int c = 0; c < 4; ++c) {
-          uint32_t acc[32];
-          tmem_ld32(taddr + c * 32, acc);
-          tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 8; ++j)
-            __stcg(dst + (c * 8 + j) * 128, make_float4(__uint_as_float(acc[4 * j]), __uint_as_float(acc[4 * j + 1]),
-                                                        __uint_as_float(acc[4 * j + 2]), __uint_as_float(acc[4 * j + 3])));
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(tempty_bar(a), 0);
-        __threadfence();
-        named_bar_sync(1 + e, 128);
-        if (r == 0) st_release_gpu(sk_flags + slot, 1u);
-        continue;
-      }
 #pragma unroll 1
       for (int s = 0; s < kNumSlabs; ++s) {
         const int nc = n0 + s * kSlabCols;
         if (r == 0) bulk_wait_read<0>();
-        named_bar_sync(1 + e, 128);   // (also publishes thread 0's flag acquires of an owner piece to the group)
+        named_bar_sync(1 + e, 128);
         if (TR::kHasAux) {
           mbar_wait(aux_bar(e), aux_cnt & 1);
           ++aux_cnt;
@@ -246,20 +174,6 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           uint32_t acc[32];
           tmem_ld32(taddr + s * kSlabCols + half * 32, acc);
           tmem_ld_wait();
-          if (head) {
-            const int c4 = (s * kSlabCols + half * 32) / 4;
-            for (int k = 0; k < n_contrib; ++k) {
-              const float4* src = reinterpret_cast<const float4*>(contrib[k]) + r;
-#pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                const float4 pv = __ldcg(src + (c4 + j) * 128);
-                acc[4 * j + 0] = __float_as_uint(__uint_as_float(acc[4 * j + 0]) + pv.x);
-                acc[4 * j + 1] = __float_as_uint(__uint_as_float(acc[4 * j + 1]) + pv.y);
-                acc[4 * j + 2] = __float_as_uint(__uint_as_float(acc[4 * j + 2]) + pv.z);
-                acc[4 * j + 3] = __float_as_uint(__uint_as_float(acc[4 * j + 3]) + pv.w);
-              }
-            }
-          }
           epi_group32<EPI>(acc, ep, nc + half * 32, r, half, o0, xb);
         }
         if (s == kNumSlabs - 1) {  // this warp has read its part of the accumulator: one arrival per warp on the leader
@@ -298,29 +212,8 @@ int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMa
   CRF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
   const int tiles = ((a.M + PM - 1) / PM) * (a.N / PN);
   const int max_pairs = num_sms(a.device) / 2;
-  const int nk = (a.K + BK - 1) / BK;
   int pairs = max_pairs;
   if (pairs > tiles) pairs = tiles;
-  // Stream-K (see the kernel) runs when the caller hands over the partial-tile workspace (gemm_pair_streamk_bytes) and
-  // a pair's share is at least a quarter of a tile's K loop (<= 5 contributors per tile).  MEASURED on B200 (round 2,
-  // profiles/r02_gemm_streamk.md): bit-stable and correct, but NOT faster -- with all 74 pairs busy the time per K chunk
-  // doubles (0.45 -> 0.8 us): these GEMMs are bound by a chip-wide resource on the operand path (tiles x K chunks x 64 KB
-  // of TMA fills at ~5 TB/s either way), not by how the tiles pack into rounds.  So the block orchestration passes the workspace only with
-  // CRF_GEMM_STREAMK=1; through the C ABI (crf_gemm) the workspace itself is the switch.
-  int streamk = 0, snap = 1;
-  float* sk_ws = nullptr;
-  uint32_t* sk_flags = nullptr;
-  if (a.workspace != nullptr && a.workspace_bytes >= gemm_pair_streamk_bytes(a.device)) {
-    const double per_pair = static_cast<double>(tiles) * nk / max_pairs;
-    if (per_pair * 4.0 >= nk && per_pair >= 4.0) {
-      streamk = 1;
-      pairs = max_pairs;
-      snap = nk / 8 < 1 ? 1 : (nk / 8 > 4 ? 4 : nk / 8);
-      sk_flags = reinterpret_cast<uint32_t*>(a.workspace);
-      sk_ws = reinterpret_cast<float*>(static_cast<uint8_t*>(a.workspace) + 4096);
-      CRF_CUDA(cudaMemsetAsync(sk_flags, 0, 4096, st));
-    }
-  }
   EpiParams ep{a.bias, a.scale, a.scale_cols, 0, a.out0 != nullptr ? 1 : 0, nullptr, 0};
   const double mn = static_cast<double>(a.M) * a.N;
   const double out_bytes = EPI == CRF_EPI_STORE_BF16 ? 2 * mn
@@ -328,7 +221,7 @@ int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMa
                            : EPI == CRF_EPI_BIAS_GELU ? (a.out0 != nullptr ? 4 * mn : 2 * mn)
                            : 4 * mn;
   KernelTimer tm(st, 2.0 * mn * a.K, 2.0 * (static_cast<double>(a.M) + a.N) * a.K + out_bytes,
-                 "gemm2%s_%s_epi%d_M%d_N%d_K%d", streamk ? "sk" : "", a.b_major ? "dgrad" : "fprop", EPI, a.M, a.N, a.K);
+                 "gemm2_%s_epi%d_M%d_N%d_K%d", a.b_major ? "dgrad" : "fprop", EPI, a.M, a.N, a.K);
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(2 * pairs);
   cfg.blockDim = dim3(kThreads);
@@ -340,28 +233,20 @@ int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMa
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // see launch_pdl (crf_host.h)
-  attr[1].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+  attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 2;
-  CRF_CUDA(cudaLaunchKernelEx(&cfg, kern, tmA, tmB, tmO0, tmO1, tmAux, a.M, a.N, a.K, a.b_major, ep, streamk, snap,
-                                sk_ws, sk_flags));
+  CRF_CUDA(cudaLaunchKernelEx(&cfg, kern, tmA, tmB, tmO0, tmO1, tmAux, a.M, a.N, a.K, a.b_major, ep));
   note_launch();
   return 0;
 }
 
 }  // namespace
 
-// flags (4 KB) + one 256 x 256 fp32 partial tile per SM pair
-size_t gemm_pair_streamk_bytes(int device) {
-  return 4096 + static_cast<size_t>(num_sms(device) / 2) * PM * PN * sizeof(float);
-}
-
 // fprop / dgrad (A K-major) with N a multiple of 256 and enough work for CTA pairs.  Returns -1 if not eligible.
 int launch_gemm_pair(const crf_gemm_args& a, cudaStream_t st) {
   // verified (tests/test_gpu_stages.py, block parity) and measured on B200: 15-30 % faster than the single-CTA kernel on
-  // every C >= 512 projection (profiles/r02_gemm_pair.md); CRF_GEMM_PAIR=0 falls back to the single-CTA kernel
-  static const int mode = [] { const char* e = getenv("CRF_GEMM_PAIR"); return e ? atoi(e) : 1; }();
-  if (mode == 0) return -1;
+  // every C >= 512 projection (profiles/r02_gemm_pair.md)
   if (a.a_major != 0 || a.N % PN != 0 || a.epilogue == CRF_EPI_SPLITK_F32 || a.split3) return -1;
   if (a.K < 512 || a.N < 512) return -1;
   CUtensorMap tmA, tmB, tmO0, tmO1, tmAux;

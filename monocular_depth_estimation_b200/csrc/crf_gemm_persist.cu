@@ -12,8 +12,6 @@
 // and barrier init / TMEM allocation / descriptor prefetch are paid once per SM instead of once per tile.
 // Barriers: full/empty[stages] (TMA <-> MMA), tmem_full[4] (MMA -> epilogue, tcgen05.commit), tmem_empty[4]
 // (epilogue -> MMA, 128 arrivals), aux[4] (TMA aux-slab loads of each group).
-#include <stdlib.h>
-
 #include "crf_gemm_epi.cuh"
 
 namespace crf {
@@ -243,12 +241,11 @@ int launch_p(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& 
   const int tiles = ((a.M + BM - 1) / BM) * (a.N / BN);
   const int sms = num_sms(a.device);
   // K splits for the fp32-output epilogues when the tile count quantises badly on the SM count: pick the split count
-  // (<= 4, >= 512 K elements per unit) that minimises rounds / splits.  CRF_GEMM_SPLITK=0 turns it off.
+  // (<= 4, >= 512 K elements per unit) that minimises rounds / splits.
   int splits = 1;
   if (EpiTraits<EPI>::kOutF32 && tiles >= sms / 2) {
-    static const bool on = !(getenv("CRF_GEMM_SPLITK") && atoi(getenv("CRF_GEMM_SPLITK")) == 0);
     double best = static_cast<double>((tiles + sms - 1) / sms);
-    for (int s = 2; on && s <= 4 && a.K / s >= 512; ++s) {
+    for (int s = 2; s <= 4 && a.K / s >= 512; ++s) {
       const double cost = static_cast<double>((tiles * s + sms - 1) / sms) / s + 0.04 * (s - 1);  // + per-unit overhead
       if (cost < best - 1e-9) { best = cost; splits = s; }
     }

@@ -1,4 +1,3 @@
-#include <stdlib.h>
 // Host-side plumbing of libcrf_sm100.so: thread-local error string, TMA descriptor creation.
 #include "crf_host.h"
 
@@ -148,11 +147,6 @@ size_t timing_report(char* buf, size_t cap) {
     buf[n] = 0;
   }
   return out.size() + 1;
-}
-
-bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("CRF_PDL"); return e == nullptr || e[0] != '0'; }();
-  return on;
 }
 
 int num_sms(int device) {

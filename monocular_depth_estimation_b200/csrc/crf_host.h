@@ -70,8 +70,7 @@ long long launch_count();
 
 // Kernel launch with the programmatic-stream-serialization attribute (PDL): the kernel may be scheduled while the
 // previous kernel of the stream is still draining; every kernel launched through here begins with pdl_prologue()
-// (crf_ptx.cuh), which waits for the previous grid before anything else runs.  CRF_PDL=0 launches without the attribute.
-bool pdl_enabled();
+// (crf_ptx.cuh), which waits for the previous grid before anything else runs.
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg{};
@@ -81,7 +80,7 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
@@ -91,7 +90,6 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
 int launch_gemm(const crf_gemm_args& a, cudaStream_t st);
 int launch_gemm_persistent(const crf_gemm_args& a, cudaStream_t st);  // -1: shape not eligible
 int launch_gemm_pair(const crf_gemm_args& a, cudaStream_t st);        // cta_group::2 tiles (crf_gemm_pair.cu); -1: not eligible
-size_t gemm_pair_streamk_bytes(int device);   // workspace (crf_gemm_args.workspace) that lets the pair kernel run stream-K
 // crf_precise.cu: the fp32 precision mode (crf_block_desc.precision == CRF_PREC_FP32)
 size_t precise_saved_bytes(const crf_block_desc& d);
 size_t precise_bwd_bytes(const crf_block_desc& d);

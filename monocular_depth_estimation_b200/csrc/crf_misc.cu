@@ -2,8 +2,6 @@
 // change folded in), LayerNorm backward (with the residual add and the gamma/beta reductions folded in), bias
 // gradient column sums, dtype casts, and the stand-alone window gather / scatter / mask used by the bit-exact
 // index tests.  All of these are HBM-bound: coalesced, vectorised accesses, warp-shuffle reductions.
-#include <stdlib.h>
-
 #include "crf_host.h"
 #include "crf_ptx.cuh"
 #include "crf_window.cuh"
@@ -148,117 +146,6 @@ ln_fwd_rows_kernel(const TIn* __restrict__ x, int64_t sb, int64_t st, int T_img,
       store2(xn + t * C + c, a0, a1);
     }
   }
-}
-
-// Same row kernel with R rows per warp iteration: all R rows' loads are issued before the first reduction, so a warp
-// keeps R x C x sizeof(TIn) bytes in flight instead of one row's (the one-row form is latency-bound for narrow rows:
-// 512 B per warp at C = 128 fp32, 0.53 of the HBM peak measured).  Per-row arithmetic and its order are exactly those
-// of ln_fwd_rows_kernel.  CANDIDATE: correct on a B200 (profiles/r01_hwcheck.txt), speed unmeasured: selected only with
-// CRF_LN_ROWS=2|4 (launch_ln_fwd_t / launch_layernorm_fwd); the default path is ln_fwd_rows_kernel.
-template <typename TIn, int NCH, bool DO_LN, typename TOut, int R>
-__global__ void __launch_bounds__(256)
-ln_fwd_multirow_kernel(const TIn* __restrict__ x, int64_t sb, int64_t st, int T_img, int64_t T,
-                       const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
-                       TOut* __restrict__ xn, float* __restrict__ stats, float* __restrict__ x_copy) {
-  pdl_prologue();
-  constexpr int C = 64 * NCH;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t warps_total = static_cast<int64_t>(gridDim.x) * 8;
-  float2 gam[NCH], bet[NCH];
-  if (DO_LN) {
-#pragma unroll
-    for (int k = 0; k < NCH; ++k) {
-      gam[k] = __ldg(reinterpret_cast<const float2*>(gamma + 64 * k + 2 * lane));
-      bet[k] = __ldg(reinterpret_cast<const float2*>(beta + 64 * k + 2 * lane));
-    }
-  }
-  for (int64_t t0 = (static_cast<int64_t>(blockIdx.x) * 8 + warp) * R; t0 < T; t0 += warps_total * R) {
-    float2 v[R][NCH];
-    float s[R];
-#pragma unroll
-    for (int j = 0; j < R; ++j) {
-      const int64_t t = t0 + j < T ? t0 + j : T - 1;  // tail rows re-read the last row (never stored)
-      const int64_t b = t / T_img;
-      const TIn* row = x + b * sb + (t - b * T_img) * st;
-      s[j] = 0.f;
-#pragma unroll
-      for (int k = 0; k < NCH; ++k) {
-        v[j][k] = load2(row + 64 * k + 2 * lane);
-        s[j] += v[j][k].x + v[j][k].y;
-      }
-    }
-    float mean[R], rstd[R];
-#pragma unroll
-    for (int j = 0; j < R; ++j) {
-      mean[j] = 0.f;
-      rstd[j] = 1.f;
-    }
-    if (DO_LN) {
-#pragma unroll
-      for (int j = 0; j < R; ++j) mean[j] = warp_sum(s[j]) * (1.0f / C);
-      float q[R];
-#pragma unroll
-      for (int j = 0; j < R; ++j) {
-        q[j] = 0.f;
-#pragma unroll
-        for (int k = 0; k < NCH; ++k) {
-          const float d0 = v[j][k].x - mean[j], d1 = v[j][k].y - mean[j];
-          q[j] += d0 * d0 + d1 * d1;
-        }
-      }
-#pragma unroll
-      for (int j = 0; j < R; ++j) rstd[j] = rsqrtf(warp_sum(q[j]) * (1.0f / C) + eps);
-    }
-#pragma unroll
-    for (int j = 0; j < R; ++j) {
-      const int64_t t = t0 + j;
-      if (t >= T) break;
-      if (DO_LN && lane == 0 && stats != nullptr) {
-        stats[2 * t] = mean[j];
-        stats[2 * t + 1] = rstd[j];
-      }
-#pragma unroll
-      for (int k = 0; k < NCH; ++k) {
-        const int c = 64 * k + 2 * lane;
-        if (x_copy != nullptr) *reinterpret_cast<float2*>(x_copy + t * C + c) = v[j][k];
-        float a0 = v[j][k].x, a1 = v[j][k].y;
-        if (DO_LN) {
-          a0 = (a0 - mean[j]) * rstd[j] * gam[k].x + bet[k].x;
-          a1 = (a1 - mean[j]) * rstd[j] * gam[k].y + bet[k].y;
-        }
-        store2(xn + t * C + c, a0, a1);
-      }
-    }
-  }
-}
-
-// CRF_LN_ROWS=2|4 selects the multi-row candidate for C <= 256 (read once per process); anything else: the verified kernel.
-int ln_rows_per_warp() {
-  static const int r = [] {
-    const char* e = getenv("CRF_LN_ROWS");
-    const int v = e != nullptr ? atoi(e) : 1;
-    return (v == 2 || v == 4) ? v : 1;
-  }();
-  return r;
-}
-
-template <typename TIn, typename TOut, bool DO_LN>
-bool launch_ln_multirow(int rows, int nch, int blocks8, int sms, cudaStream_t st, const TIn* x, int64_t sb, int64_t st_,
-                        int T_img, int64_t T, const float* gamma, const float* beta, float eps, TOut* xn, float* stats,
-                        float* x_copy) {
-  if (rows == 1 || nch > 4) return false;
-  int blocks = static_cast<int>((T + 8 * rows - 1) / (8 * rows));
-  if (blocks > sms * 16) blocks = sms * 16;
-  (void)blocks8;
-#define CRF_LNM(NCH, R)                                                                                               \
-  if (nch == NCH && rows == R) {                                                                                      \
-    ln_fwd_multirow_kernel<TIn, NCH, DO_LN, TOut, R><<<blocks, 256, 0, st>>>(x, sb, st_, T_img, T, gamma, beta, eps, xn, \
-                                                                             stats, x_copy);                          \
-    return true;                                                                                                      \
-  }
-  CRF_LNM(1, 2) CRF_LNM(2, 2) CRF_LNM(3, 2) CRF_LNM(4, 2) CRF_LNM(1, 4) CRF_LNM(2, 4) CRF_LNM(3, 4) CRF_LNM(4, 4)
-#undef CRF_LNM
-  return false;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -536,19 +423,6 @@ int launch_ln_fwd_t(const void* x, int64_t sb, int64_t st_, int64_t sc, int B, i
     if (blocks > cap) blocks = cap;
     const TIn* xp = reinterpret_cast<const TIn*>(x);
     __nv_bfloat16* xnp = reinterpret_cast<__nv_bfloat16*>(xn);
-    if (ln_rows_per_warp() > 1) {  // opt-in candidate kernel (CRF_LN_ROWS), bit-identical results
-      const bool done = gamma != nullptr
-                            ? launch_ln_multirow<TIn, __nv_bfloat16, true>(ln_rows_per_warp(), C / 64, blocks, num_sms(dev), st, xp,
-                                                                           sb, st_, T_img, T, gamma, beta, eps, xnp, stats, x_copy)
-                            : launch_ln_multirow<TIn, __nv_bfloat16, false>(ln_rows_per_warp(), C / 64, blocks, num_sms(dev), st, xp,
-                                                                            sb, st_, T_img, T, nullptr, nullptr, eps, xnp, nullptr,
-                                                                            x_copy);
-      if (done) {
-        CRF_CUDA(cudaGetLastError());
-        note_launch();
-        return 0;
-      }
-    }
 #define CRF_LNF(NCH)                                                                                                  \
   case NCH:                                                                                                           \
     if (gamma != nullptr)                                                                                             \
@@ -779,19 +653,6 @@ int launch_layernorm_fwd(const float* x, const float* gamma, const float* beta, 
   const int cap = num_sms(dev) * 16;
   if (blocks > cap) blocks = cap;
   KernelTimer tm(st, 0.0, static_cast<double>(T) * C * (4 + (y_dtype == CRF_DT_F32 ? 4 : 2)), "layernorm_fwd_T%d_C%d", T, C);
-  if (ln_rows_per_warp() > 1) {  // opt-in candidate kernel (CRF_LN_ROWS), bit-identical results
-    const bool done = y_dtype == CRF_DT_F32
-                          ? launch_ln_multirow<float, float, true>(ln_rows_per_warp(), C / 64, blocks, num_sms(dev), st, x, 0, C, T,
-                                                                   T, gamma, beta, eps, reinterpret_cast<float*>(y), stats, nullptr)
-                          : launch_ln_multirow<float, __nv_bfloat16, true>(ln_rows_per_warp(), C / 64, blocks, num_sms(dev), st, x,
-                                                                           0, C, T, T, gamma, beta, eps,
-                                                                           reinterpret_cast<__nv_bfloat16*>(y), stats, nullptr);
-    if (done) {
-      CRF_CUDA(cudaGetLastError());
-      note_launch();
-      return 0;
-    }
-  }
 #define CRF_LNS(NCH)                                                                                                   \
   case NCH:                                                                                                            \
     if (y_dtype == CRF_DT_F32)                                                                                         \

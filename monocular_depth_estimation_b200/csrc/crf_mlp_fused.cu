@@ -495,13 +495,9 @@ int launch_mlp_c(const crf_mlp_args& m, cudaStream_t st) {
   if (make_tmap_bf16(&tmW2, m.w2_bf16, C, 4 * C, 128)) return 1;
   // Rows per tile: the MMA tile is always 128 rows; only `tm` of them are normalised, multiplied for real and stored, with
   // tm chosen so that the tiles fill whole rounds of the persistent grid (T = 38400: 300 tiles of 128 rows = 2.03 rounds
-  // on 148 SMs, i.e. 3 rounds; 437 tiles of 88 rows = 2.95 rounds of a shorter tile).  CRF_MLP_TM128=1: always 128.
+  // on 148 SMs, i.e. 3 rounds; 437 tiles of 88 rows = 2.95 rounds of a shorter tile).
   const int sms = num_sms(m.device);
-  int tm = balanced_tile_rows(m.T, sms);
-  {
-    static const bool fixed = getenv("CRF_MLP_TM128") != nullptr;
-    if (fixed) tm = TM;
-  }
+  const int tm = balanced_tile_rows(m.T, sms);
   if (make_tmap_f32(&tmY, m.y, m.T, C, tm)) return 1;
   if (m.training) {
     if (make_tmap_bf16(&tmXn, m.xn2, m.T, C, tm)) return 1;

@@ -1,5 +1,5 @@
 // Work-decomposition arithmetic shared by host launchers and kernels (and compiled on the host by
-// tests/test_sched_host.py): rows per tile of the persistent row-tiled kernels, stream-K ranges of the CTA-pair GEMM.
+// tests/test_sched_host.py): rows per tile of the persistent row-tiled kernels.
 #pragma once
 
 #ifndef __CUDACC__
@@ -23,62 +23,6 @@ __host__ __device__ inline int balanced_tile_rows(int T, int sms) {
   const int n = (rows_per_cta + 127) / 128;
   int tm = (((rows_per_cta + n - 1) / n) + 7) & ~7;
   return tm > 128 ? 128 : tm;
-}
-
-// ---- stream-K (crf_gemm_pair.cu) ----
-// The tiles x K-chunks sequence (tile-major, `total` = tiles * nk units) is cut into npairs contiguous ranges; the
-// boundary of pair p is snapped to a tile boundary when it would leave a piece of fewer than `snap` K chunks.
-__host__ __device__ inline int sk_bound(int p, int npairs, int total, int nk, int snap) {
-  int b = static_cast<int>(static_cast<long long>(p) * total / npairs);
-  const int rem = b % nk;
-  if (rem < snap) b -= rem;
-  else if (nk - rem < snap) b += nk - rem;
-  return b;
-}
-struct Piece {
-  int t, kc0, kc1;   // tile, K-chunk range [kc0, kc1)
-};
-struct PieceIter {
-  int nk, tiles, pair, npairs, streamk, w, w1, i;
-  __host__ __device__ PieceIter(int nk_, int tiles_, int pair_, int npairs_, int streamk_, int snap)
-      : nk(nk_), tiles(tiles_), pair(pair_), npairs(npairs_), streamk(streamk_), w(0), w1(0), i(0) {
-    if (streamk) {
-      w = sk_bound(pair, npairs, tiles * nk, nk, snap);
-      w1 = sk_bound(pair + 1, npairs, tiles * nk, nk, snap);
-    }
-  }
-  __host__ __device__ bool next(Piece& p) {
-    if (!streamk) {   // classic: whole tiles pair, pair + npairs, ...
-      const int t = pair + i * npairs;
-      if (t >= tiles) return false;
-      ++i;
-      p.t = t; p.kc0 = 0; p.kc1 = nk;
-      return true;
-    }
-    if (w >= w1) return false;
-    p.t = w / nk;
-    p.kc0 = w - p.t * nk;
-    const int left = w1 - w;
-    p.kc1 = p.kc0 + left < nk ? p.kc0 + left : nk;
-    w += p.kc1 - p.kc0;
-    return true;
-  }
-};
-constexpr int kMaxContrib = 8;
-// Pairs whose FIRST piece finishes the tile that pair `pair` owns up to chunk kc1 (an owner piece): fills q[] with their
-// indices, returns the count, or -1 if the tile is not covered by at most kMaxContrib of them.
-__host__ __device__ inline int sk_contributors(int pair, int npairs, int tiles, int nk, int snap, int t, int kc1, int* q) {
-  const int total = tiles * nk, tile_end = (t + 1) * nk;
-  int pos = t * nk + kc1, n = 0;
-  for (int c = pair + 1; pos < tile_end && c < npairs; ++c) {
-    const int c0 = sk_bound(c, npairs, total, nk, snap), c1 = sk_bound(c + 1, npairs, total, nk, snap);
-    if (c1 > c0) {
-      if (n == kMaxContrib) return -1;
-      q[n++] = c;
-      pos = c1 < tile_end ? c1 : tile_end;
-    }
-  }
-  return pos >= tile_end ? n : -1;
 }
 
 }  // namespace crf

@@ -13,12 +13,8 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-import os
-
-from .functional import pixel_shuffle2
 from .newcrf_layers import NewCRF
 
-_FUSE_SHUFFLE = os.environ.get("CRF_FUSE_SHUFFLE", "1") != "0"
 CRF_DIMS = (128, 256, 512, 1024)      # embed dim per scale 1/4 .. 1/32
 V_DIMS = (64, 128, 256, 512)          # depth-feature channels entering each stage
 NUM_HEADS = (4, 8, 16, 32)
@@ -40,11 +36,8 @@ class Decoder(nn.Module):
         e = self.conv0(feats[ENC_TAPS[4]])
         for s in (3, 2, 1, 0):
             # nn.PixelShuffle(2) between the stages (model_mobileV3_large_newCRFs.py:116-120) is folded into the store of
-            # the producing stage's closing LayerNorm (no separate permutation pass; CRF_FUSE_SHUFFLE=0 restores it)
-            fuse = s != 0 and _FUSE_SHUFFLE
-            e = getattr(self, f"crf{s}")(feats[ENC_TAPS[s]], e, pixel_shuffle=fuse)
-            if s != 0 and not fuse:
-                e = pixel_shuffle2(e)
+            # the producing stage's closing LayerNorm (no separate permutation pass)
+            e = getattr(self, f"crf{s}")(feats[ENC_TAPS[s]], e, pixel_shuffle=(s != 0))
         d = self.sigmoid(self.conv1(e))
         return F.interpolate(d, scale_factor=4, mode="bilinear", align_corners=False)
 

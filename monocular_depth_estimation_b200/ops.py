@@ -72,7 +72,7 @@ def make_desc(B, H, W, Cdim, num_heads, shift, *, window=7, training=1, device=0
 
 
 def gemm(A, B, M, N, K, *, a_major=0, b_major=0, epilogue=L.EPI_STORE_F32, out0, out1=None, bias=None, aux1=None,
-         ld_out=None, scale=1.0, scale_cols=0, split_k=0, colsum=None, streamk=False):
+         ld_out=None, scale=1.0, scale_cols=0, split_k=0, colsum=None):
     a = L.GemmArgs()
     a.A, a.B = A.data_ptr(), B.data_ptr()
     a.a_major, a.b_major = a_major, b_major
@@ -92,10 +92,6 @@ def gemm(A, B, M, N, K, *, a_major=0, b_major=0, epilogue=L.EPI_STORE_F32, out0,
         if need:
             ws = torch.empty(need, dtype=torch.uint8, device=A.device)
             a.workspace, a.workspace_bytes = ws.data_ptr(), need
-    elif streamk:   # scratch that lets the CTA-pair kernel cut the K loop of its tiles across SM pairs
-        need = L.lib().crf_gemm_streamk_bytes(a.device)
-        ws = torch.empty(need, dtype=torch.uint8, device=A.device)
-        a.workspace, a.workspace_bytes = ws.data_ptr(), need
     L.check(L.lib().crf_gemm(C.byref(a), _stream(A)), "crf_gemm")
     return out0
 

@@ -60,14 +60,12 @@ def wrap_ddp(model, device, world, grad_dtype=None, bucket_cap_mb=64):
     """The DDP wrapper `train.py` lacks: gradients are averaged with an NCCL all-reduce, bucketed and launched while
     backward is still running (crf3's 29 M parameters become ready first and are reduced under the rest).
 
-    grad_dtype=torch.bfloat16 (or CRF_DDP_GRAD_BF16=1) exchanges the buckets in bf16 -- 90 MB instead of 180 MB per
+    grad_dtype=torch.bfloat16 exchanges the buckets in bf16 -- 90 MB instead of 180 MB per
     step (SURVEY.md 8e) -- through DDP's stock bf16_compress_hook: each rank's gradient is divided by the world size,
     rounded to bf16, summed by the all-reduce in bf16 and widened back to fp32.  Off by default: the averaged gradient
     then carries a bf16 rounding (rel ~ 2^-9) the fp32 exchange does not have."""
     if world <= 1:
         return model
-    if grad_dtype is None and os.environ.get("CRF_DDP_GRAD_BF16", "0") == "1":
-        grad_dtype = torch.bfloat16
     if grad_dtype not in (None, torch.float32, torch.bfloat16):
         raise ValueError(f"wrap_ddp: grad_dtype must be None, torch.float32 or torch.bfloat16 (got {grad_dtype})")
     from torch.nn.parallel import DistributedDataParallel as DDP
@@ -81,7 +79,7 @@ def wrap_ddp(model, device, world, grad_dtype=None, bucket_cap_mb=64):
         # broadcast_buffers=False: BatchNorm running statistics stay rank-local (46 BN layers would otherwise add a
         # broadcast of ~140 small buffers to every forward); gradients are what is averaged.
         net = DDP(model, device_ids=[device.index], bucket_cap_mb=bucket_cap_mb, broadcast_buffers=False,
-                  gradient_as_bucket_view=os.environ.get("CRF_DDP_BUCKET_VIEW", "1") != "0")
+                  gradient_as_bucket_view=True)
     else:
         net = DDP(model)
     if grad_dtype == torch.bfloat16:

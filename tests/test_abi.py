@@ -32,7 +32,7 @@ def test_version_and_error_reporting_without_gpu():
     if not os.path.exists(_lib.LIB_PATH):
         pytest.skip("extension not built")
     lib = _lib.lib()
-    assert lib.crf_abi_version() == 3
+    assert lib.crf_abi_version() == 4
     d = _lib.BlockDesc()
     d.B, d.H, d.W, d.C, d.num_heads, d.window, d.shift = 1, 7, 7, 96, 3, 7, 0   # C not a multiple of 64
     s = ctypes.c_size_t()

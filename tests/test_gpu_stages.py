@@ -170,10 +170,9 @@ def test_gemm_bias_residual_with_k_splits(M, N, K):
                                    (9600, 512, 512), (9600, 2048, 512), (9600, 512, 2048), (9600, 1024, 512),
                                    (1000, 512, 1024), (300, 1024, 2048)])
 @pytest.mark.parametrize("kind", ["fprop", "dgrad"])
-def test_gemm_pair_stream_k(M, N, K, kind):
-    """The CTA-pair GEMM with the stream-K work split (csrc/crf_gemm_pair.cu): the K loop of the 256 x 256 tiles is cut
-    across SM pairs, partial accumulators meet in the workspace.  Every epilogue the C >= 512 projections use, against
-    fp32 PyTorch and against the same kernel without the workspace (whole tiles)."""
+def test_gemm_pair_epilogues(M, N, K, kind):
+    """The CTA-pair GEMM (csrc/crf_gemm_pair.cu, 256 x 256 tiles on the two SMs of a TPC) with every epilogue the
+    C >= 512 projections use, against fp32 PyTorch."""
     ops, L = _ops(), _L()
     bm = 0 if kind == "fprop" else 1
     A = _rand_bf16(M, K, seed=21)
@@ -181,39 +180,32 @@ def test_gemm_pair_stream_k(M, N, K, kind):
     acc = A.float() @ (W.float().t() if bm == 0 else W.float())
     bias = torch.randn(N, device=DEV)
     res = torch.randn(M, N, device=DEV)
-    outs = {}
-    for sk in (False, True):
-        o32 = torch.full((M, N), float("nan"), device=DEV)
-        ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_STORE_F32, out0=o32, streamk=sk)
-        _check(o32, acc, 1e-5, f"streamk={sk} store_f32")
-        o16 = torch.zeros(M, N, dtype=torch.bfloat16, device=DEV)
-        ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_STORE_BF16, out0=o16, bias=bias, scale=0.25, scale_cols=N // 2,
-                 streamk=sk)
-        ref = acc + bias
-        ref[:, :N // 2] *= 0.25
-        _check(o16.float(), ref, 4e-3, f"streamk={sk} store_bf16")
-        ores = torch.full((M, N), float("nan"), device=DEV)
-        ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_BIAS_RES_F32, out0=ores, bias=bias, aux1=res, streamk=sk)
-        _check(ores, acc + bias + res, 1e-5, f"streamk={sk} bias_res")
-        pre = torch.zeros(M, N, dtype=torch.bfloat16, device=DEV)
-        act = torch.zeros(M, N, dtype=torch.bfloat16, device=DEV)
-        ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_BIAS_GELU, out0=pre, out1=act, bias=bias, streamk=sk)
-        _check(pre.float(), acc + bias, 4e-3, f"streamk={sk} gelu.pre")
-        _check(act.float(), F.gelu(acc + bias), 4e-3, f"streamk={sk} gelu.act")
-        dg = torch.zeros(M, N, dtype=torch.bfloat16, device=DEV)
-        ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_MUL_DGELU, out0=dg, aux1=pre, streamk=sk)
-        p = pre.float().requires_grad_(True)
-        F.gelu(p).sum().backward()
-        _check(dg.float(), acc * p.grad, 4e-3, f"streamk={sk} mul_dgelu")
-        torch.cuda.synchronize()
-        outs[sk] = (o32, o16, ores, pre, act, dg)
-    for a_, b_ in zip(outs[False], outs[True]):   # same products, summed in a different order
-        _check(b_.float(), a_.float(), 1e-5 if a_.dtype == torch.float32 else 4e-3, "stream-K vs whole tiles")
-    # repeatable: the split is a pure function of the shape
+    o32 = torch.full((M, N), float("nan"), device=DEV)
+    ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_STORE_F32, out0=o32)
+    _check(o32, acc, 1e-5, "store_f32")
+    o16 = torch.zeros(M, N, dtype=torch.bfloat16, device=DEV)
+    ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_STORE_BF16, out0=o16, bias=bias, scale=0.25, scale_cols=N // 2)
+    ref = acc + bias
+    ref[:, :N // 2] *= 0.25
+    _check(o16.float(), ref, 4e-3, "store_bf16")
+    ores = torch.full((M, N), float("nan"), device=DEV)
+    ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_BIAS_RES_F32, out0=ores, bias=bias, aux1=res)
+    _check(ores, acc + bias + res, 1e-5, "bias_res")
+    pre = torch.zeros(M, N, dtype=torch.bfloat16, device=DEV)
+    act = torch.zeros(M, N, dtype=torch.bfloat16, device=DEV)
+    ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_BIAS_GELU, out0=pre, out1=act, bias=bias)
+    _check(pre.float(), acc + bias, 4e-3, "gelu.pre")
+    _check(act.float(), F.gelu(acc + bias), 4e-3, "gelu.act")
+    dg = torch.zeros(M, N, dtype=torch.bfloat16, device=DEV)
+    ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_MUL_DGELU, out0=dg, aux1=pre)
+    p = pre.float().requires_grad_(True)
+    F.gelu(p).sum().backward()
+    _check(dg.float(), acc * p.grad, 4e-3, "mul_dgelu")
+    # repeatable: two runs of the same call give the same bits
     o2 = torch.full((M, N), float("nan"), device=DEV)
-    ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_STORE_F32, out0=o2, streamk=True)
+    ops.gemm(A, W, M, N, K, b_major=bm, epilogue=L.EPI_STORE_F32, out0=o2)
     torch.cuda.synchronize()
-    assert torch.equal(o2, outs[True][0])
+    assert torch.equal(o2, o32)
 
 
 def test_gemm_epilogues():

@@ -1,18 +1,11 @@
 """Work-decomposition arithmetic of the persistent kernels, compiled on the host (no GPU) from the header the kernels
-and launchers include (csrc/crf_sched.h):
-
-1. `balanced_tile_rows` (fused MLP forward, fused d.LN' kernel): rows per tile are a multiple of 8, at most 128, cover the
-   input, and never need more rounds of the grid than 128-row tiles do.
-2. stream-K of the CTA-pair GEMM (`sk_bound`, `PieceIter`, `sk_contributors`): the pieces of all pairs cover every
-   (tile, K chunk) unit exactly once, a pair has at most one piece that does not start a tile and it is its FIRST one (so
-   nobody ever waits on a pair that waits), and the contributors an owner piece enumerates are exactly the pairs whose
-   first piece holds the rest of that tile.
+and launchers include (csrc/crf_sched.h): `balanced_tile_rows` (fused MLP forward, fused d.LN' kernel) gives rows per
+tile that are a multiple of 8, at most 128, cover the input, and never need more rounds of the grid than 128-row tiles do.
 """
 import ctypes
 import os
 import subprocess
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -21,22 +14,6 @@ CSRC = os.path.join(ROOT, "monocular_depth_estimation_b200", "csrc")
 SHIM = r"""
 #include "crf_sched.h"
 extern "C" int tile_rows(int T, int sms) { return crf::balanced_tile_rows(T, sms); }
-// pieces of every pair: out[4 * i] = pair, tile, kc0, kc1; returns the count
-extern "C" int pieces(int tiles, int nk, int npairs, int streamk, int snap, int* out, int cap) {
-  int n = 0;
-  for (int p = 0; p < npairs; ++p) {
-    crf::PieceIter it(nk, tiles, p, npairs, streamk, snap);
-    crf::Piece pc;
-    while (it.next(pc)) {
-      if (n < cap) { out[4 * n] = p; out[4 * n + 1] = pc.t; out[4 * n + 2] = pc.kc0; out[4 * n + 3] = pc.kc1; }
-      ++n;
-    }
-  }
-  return n;
-}
-extern "C" int contributors(int pair, int npairs, int tiles, int nk, int snap, int t, int kc1, int* q) {
-  return crf::sk_contributors(pair, npairs, tiles, nk, snap, t, kc1, q);
-}
 """
 
 
@@ -47,10 +24,7 @@ def shim(tmp_path_factory):
     src.write_text(SHIM)
     subprocess.run(["g++", "-O1", "-shared", "-fPIC", "-x", "c++", "-I", CSRC, str(src), "-o", str(so)], check=True)
     lib = ctypes.CDLL(str(so))
-    ip = ctypes.POINTER(ctypes.c_int)
     lib.tile_rows.argtypes = [ctypes.c_int, ctypes.c_int]
-    lib.pieces.argtypes = [ctypes.c_int] * 5 + [ip, ctypes.c_int]
-    lib.contributors.argtypes = [ctypes.c_int] * 7 + [ip]
     return lib
 
 
@@ -66,46 +40,3 @@ def test_balanced_tile_rows(shim):
         assert rounds * tm <= rounds128 * 128, (T, tm)           # and never more row-time
     assert shim.tile_rows(38400, sms) == 88 and shim.tile_rows(153600, sms) == 120    # the two decoder scales that use it
     assert shim.tile_rows(128, sms) == 128 and shim.tile_rows(1000, sms) == 128
-
-
-# (M, N, K) of the C >= 512 projections (crf_gemm_pair.cu: 256 x 256 tiles, 64-wide K chunks, 74 pairs on a B200)
-SHAPES = [(2400, 4096, 1024), (2400, 1024, 4096), (2400, 1024, 1024), (2400, 2048, 1024), (9600, 512, 512),
-          (9600, 2048, 512), (9600, 512, 2048), (9600, 1024, 512), (1000, 512, 1024), (300, 1024, 2048)]
-
-
-@pytest.mark.parametrize("M,N,K", SHAPES)
-@pytest.mark.parametrize("npairs", [74, 66, 7])
-def test_stream_k_partition(shim, M, N, K, npairs):
-    tiles, nk = -(-M // 256) * (N // 256), -(-K // 64)
-    snap = max(1, min(4, nk // 8))
-    buf = np.zeros(4 * 4096, dtype=np.int32)
-    ip = ctypes.POINTER(ctypes.c_int)
-    for streamk in (0, 1):
-        if not streamk and npairs > tiles:
-            continue
-        n = shim.pieces(tiles, nk, npairs, streamk, snap, buf.ctypes.data_as(ip), 4096)
-        assert 0 < n <= 4096
-        pcs = buf[:4 * n].reshape(n, 4)
-        cover = np.zeros((tiles, nk), dtype=np.int32)
-        for p, t, k0, k1 in pcs:
-            assert 0 <= t < tiles and 0 <= k0 < k1 <= nk
-            cover[t, k0:k1] += 1
-        assert (cover == 1).all(), "every (tile, K chunk) unit exactly once"
-        if not streamk:
-            assert ((pcs[:, 2] == 0) & (pcs[:, 3] == nk)).all()
-            continue
-        q = np.zeros(8, dtype=np.int32)
-        for p in range(npairs):
-            mine = pcs[pcs[:, 0] == p]
-            # only the first piece of a pair may start inside a tile; pieces are in sequence order
-            assert (mine[1:, 2] == 0).all(), (p, mine)
-            for idx, (_, t, k0, k1) in enumerate(mine):
-                if k0 == 0 and k1 < nk:                      # owner piece: its contributors hold [k1, nk) of the tile
-                    assert idx == len(mine) - 1, "an owner piece is the last piece of its pair"
-                    c = shim.contributors(p, npairs, tiles, nk, snap, int(t), int(k1), q.ctypes.data_as(ip))
-                    assert c >= 1
-                    rest = pcs[(pcs[:, 1] == t) & (pcs[:, 2] > 0)]
-                    assert sorted(rest[:, 0].tolist()) == sorted(q[:c].tolist())
-                    for cp in q[:c]:                          # ... and each of them has that piece FIRST
-                        first = pcs[pcs[:, 0] == cp][0]
-                        assert first[1] == t and first[2] > 0

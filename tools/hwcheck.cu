@@ -4,12 +4,12 @@
 // on the same bf16-rounded inputs:
 //   1. window-attention core forward / backward: head_dim 32 (the verified kernels: validates THIS harness), then
 //      head_dim 64 and 128 (csrc/crf_attn_wide.cu)
-//   2. LayerNorm forward with 4 rows in flight per warp (CRF_LN_ROWS=4)
+//   2. the stand-alone LayerNorm forward (crf_layernorm_fwd)
 //   3. the multi-tensor Adam step (crf_adam_step)
 // Every result line goes to stdout and to gpurun_out/hwcheck.txt as soon as it is known.
 //   make -C monocular_depth_estimation_b200/csrc hwcheck
 //   tools/hwcheck            (on a B200)          tools/hwcheck --dry DIR   (no GPU: dumps inputs + references to DIR)
-//   tools/hwcheck --bench    (on a B200: CUDA-event timings of the opt-in kernels at config-2 sizes, a few seconds)
+//   tools/hwcheck --bench    (on a B200: CUDA-event timings of these kernels at config-2 sizes, a few seconds)
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdarg.h>
@@ -364,7 +364,7 @@ static int run_attn_case(const AttnCase& c, const char* tag, const std::string& 
 }
 
 // =====================================================================================================
-// LayerNorm forward (multi-row candidate when CRF_LN_ROWS is set)
+// LayerNorm forward
 // =====================================================================================================
 static int run_ln_case(int T, int C) {
   Rng rng(77 + C);
@@ -399,8 +399,8 @@ static int run_ln_case(int T, int C) {
     for (int c = 0; c < C; ++c) ref[static_cast<size_t>(t) * C + c] = (x[static_cast<size_t>(t) * C + c] - m) * rstd * gamma[c] + beta[c];
   }
   const double ey = rel_l2(got, ref);
-  say("layernorm_fwd T%d C%d (CRF_LN_ROWS=%s): rel_l2(y) %.2e  stats err %.2e (tol 1e-5) -> %s", T, C,
-      getenv("CRF_LN_ROWS") ? getenv("CRF_LN_ROWS") : "unset", ey, se, (ey < 1e-5 && se < 1e-5) ? "PASS" : "FAIL");
+  say("layernorm_fwd T%d C%d: rel_l2(y) %.2e  stats err %.2e (tol 1e-5) -> %s", T, C, ey, se,
+      (ey < 1e-5 && se < 1e-5) ? "PASS" : "FAIL");
   cudaFree(dx); cudaFree(dg); cudaFree(db); cudaFree(dy); cudaFree(ds);
   return 0;
 }
@@ -467,8 +467,7 @@ static int run_adam() {
 
 static int init_device_quiet();
 // =====================================================================================================
-// --bench: CUDA-event timings of the opt-in kernels at config-2 sizes (seconds of GPU time; one child process per
-// setting because the switches are read once per process)
+// --bench: CUDA-event timings at config-2 sizes (seconds of GPU time; one child process per job)
 // =====================================================================================================
 static float time_ms(cudaEvent_t e0, cudaEvent_t e1) {
   float ms = 0;
@@ -498,8 +497,8 @@ static int bench_ln(int T, int C) {
     cudaEventRecord(e1);
     const float ms = time_ms(e0, e1) / it;
     const double bytes = static_cast<double>(T) * C * (4 + (dt == 0 ? 2 : 4));
-    say("bench layernorm_fwd T%d C%d out=%s CRF_LN_ROWS=%s: %.2f us, %.0f GB/s", T, C, dt == 0 ? "bf16" : "f32",
-        getenv("CRF_LN_ROWS") ? getenv("CRF_LN_ROWS") : "1", ms * 1e3, bytes / ms / 1e6);
+    say("bench layernorm_fwd T%d C%d out=%s: %.2f us, %.0f GB/s", T, C, dt == 0 ? "bf16" : "f32", ms * 1e3,
+        bytes / ms / 1e6);
   }
   return 0;
 }
@@ -631,7 +630,6 @@ static int run_group(int grp) {
 
 int main(int argc, char** argv) {
   g_t0 = now_s();
-  setenv("CRF_LN_ROWS", "4", 1);
   if (argc >= 3 && strcmp(argv[1], "--dry") == 0) {
     for (int i = 0; i < 5; ++i) run_attn_case(kCases[i], kTags[i], argv[2]);
     return 0;
@@ -640,19 +638,18 @@ int main(int argc, char** argv) {
   g_log = fopen("gpurun_out/hwcheck.txt", "a");
   if (argc >= 3 && strcmp(argv[1], "--group") == 0) return run_group(atoi(argv[2]));
   if (argc >= 2 && strcmp(argv[1], "--bench") == 0) {
-    // config-2 sizes; every setting in its own child (env switches are read once per process), one after the other
-    struct Job { int kind; const char* rows; AttnCase c; };
+    // config-2 sizes; every job in its own child, one after the other
+    struct Job { int kind; AttnCase c; };
     const Job jobs[] = {
-        {0, "1", {}}, {0, "4", {}}, {0, "2", {}},                       // LayerNorm forward, 1/4 scale, rows per warp
-        {1, "1", {}},                                                   // Adam over 45 M parameters
-        {2, "1", {8, 120, 160, 128, 4, 3}},                             // attention, head_dim 32 (tuned kernels)
-        {2, "1", {8, 120, 160, 128, 2, 3}}, {2, "1", {8, 120, 160, 128, 1, 3}},   // head_dim 64, 128 at the 1/4 scale
-        {2, "1", {8, 30, 40, 512, 8, 3}}, {2, "1", {8, 30, 40, 512, 4, 3}},       // head_dim 64, 128 at the 1/16 scale
+        {0, {}},                                              // LayerNorm forward, 1/4 and 1/8 scale
+        {1, {}},                                              // Adam over 45 M parameters
+        {2, {8, 120, 160, 128, 4, 3}},                        // attention, head_dim 32 (tuned kernels)
+        {2, {8, 120, 160, 128, 2, 3}}, {2, {8, 120, 160, 128, 1, 3}},   // head_dim 64, 128 at the 1/4 scale
+        {2, {8, 30, 40, 512, 8, 3}}, {2, {8, 30, 40, 512, 4, 3}},       // head_dim 64, 128 at the 1/16 scale
     };
     for (const Job& j : jobs) {
       const pid_t pid = fork();
       if (pid == 0) {
-        setenv("CRF_LN_ROWS", j.rows, 1);
         int rc = 0;
         if (j.kind == 0) rc = bench_ln(153600, 128) | bench_ln(38400, 256);
         else if (j.kind == 1) rc = bench_adam(45000000LL, 300);
@@ -674,7 +671,7 @@ int main(int argc, char** argv) {
   for (int grp = 0; grp < 4; ++grp) {
     int st = 0;
     waitpid(pids[grp], &st, 0);
-    say("group %d (%s): exit %d%s", grp, grp == 0 ? "hd32 + hd64" : grp == 1 ? "hd128" : grp == 2 ? "layernorm rows=4" : "adam",
+    say("group %d (%s): exit %d%s", grp, grp == 0 ? "hd32 + hd64" : grp == 1 ? "hd128" : grp == 2 ? "layernorm" : "adam",
         WIFEXITED(st) ? WEXITSTATUS(st) : -1, WIFSIGNALED(st) ? " (killed by a signal)" : "");
   }
   say("hwcheck finished (PASS / FAIL per line above)");

@@ -36,7 +36,6 @@ def main():
     ap.add_argument("--batch", type=int, default=8)
     ap.add_argument("--shift", type=int, default=3)
     ap.add_argument("--iters", type=int, default=5)
-    ap.add_argument("--streamk", action="store_true", help="gemms: hand the stream-K scratch to the CTA-pair kernel")
     ap.add_argument("--only", default="", help="gemms: run only the shape with this label (e.g. \"d_fc2*gelu'\")")
     a = ap.parse_args()
     H, W, C, nH = STAGES[a.stage]
@@ -153,7 +152,7 @@ def main():
                    torch.randn(M, N, device=dev).to(torch.bfloat16) if epi == L.EPI_MUL_DGELU else None)
             bias = torch.randn(N, device=dev) if not bmaj else None
             ms = timed(lambda: ops.gemm(A, Wt, M, N, K, b_major=bmaj, epilogue=epi, out0=out0, out1=out1, bias=bias,
-                                        aux1=aux, streamk=a.streamk), a.iters)
+                                        aux1=aux), a.iters)
             print(f"{name:12s} M{M} N{N} K{K}: {ms*1e3:8.1f} us  {2.0*M*N*K/ms/1e9:7.1f} TFLOP/s")
     else:
         M, N, K = T, 4 * C, C
