@@ -418,17 +418,10 @@ int crf_layer_fwd(const crf_block_desc* d, const crf_layer_args* a, const void* 
     if (block_fwd_impl(&bd, a->params + i, xin, vin, yo, S + L.blk[i], stream)) return 1;
     xin = yo;
   }
-  if (with_norm) {
-    if (a->out_shuffle) {
-      if (launch_layernorm_ps_fwd(static_cast<const float*>(xin), a->norm_w, a->norm_b, a->params[0].ln_eps, y,
-                                  a->out_dtype, reinterpret_cast<float*>(S + L.norm_stats), d->B, d->H, d->W, d->C,
-                                  static_cast<cudaStream_t>(stream)))
-        return 1;
-    } else if (launch_layernorm_fwd(static_cast<const float*>(xin), a->norm_w, a->norm_b, a->params[0].ln_eps, y,
-                                    a->out_dtype, reinterpret_cast<float*>(S + L.norm_stats), T, d->C,
-                                    static_cast<cudaStream_t>(stream)))
-      return 1;
-  }
+  if (with_norm && launch_layernorm_fwd(static_cast<const float*>(xin), a->norm_w, a->norm_b, a->params[0].ln_eps, y,
+                                        a->out_dtype, reinterpret_cast<float*>(S + L.norm_stats), T, d->C,
+                                        static_cast<cudaStream_t>(stream), a->out_shuffle ? d->W : 0))
+    return 1;
   return 0;
 }
 
@@ -458,24 +451,18 @@ int crf_layer_bwd(const crf_block_desc* d, const crf_layer_args* a, const void* 
   if (with_norm) {
     const float* ylast = reinterpret_cast<const float*>(S + L.yout[a->depth - 1]);
     float* gn = reinterpret_cast<float*>(Wk + W.g_f32);
+    const float* stats = reinterpret_cast<const float*>(S + L.norm_stats);
     // LayerNorm backward writes dx in fp32 and its bf16 twin in one pass (the MLP GEMMs read the twin)
-    if (a->out_shuffle) {
-      if (launch_layernorm_ps_bwd(dy, a->out_dtype, ylast, reinterpret_cast<const float*>(S + L.norm_stats), a->norm_w, gn,
-                                  Wk + W.g_bf16, dnorm_w, dnorm_b, d->B, d->H, d->W, d->C, st))
+    if (a->out_dtype == CRF_DT_F32 && !a->out_shuffle) {
+      if (launch_ln_bwd(static_cast<const float*>(dy), ylast, stats, a->norm_w, nullptr, gn, Wk + W.g_bf16, dnorm_w,
+                        dnorm_b, static_cast<int>(T), d->C, st))
         return 1;
-      g16 = Wk + W.g_bf16;
-    } else if (a->out_dtype == CRF_DT_F32) {
-      if (launch_ln_bwd(static_cast<const float*>(dy), ylast, reinterpret_cast<const float*>(S + L.norm_stats), a->norm_w,
-                        nullptr, gn, Wk + W.g_bf16, dnorm_w, dnorm_b, static_cast<int>(T), d->C, st))
-        return 1;
-      g16 = Wk + W.g_bf16;
-    } else {
-      if (launch_layernorm_bwd(dy, CRF_DT_BF16, ylast, reinterpret_cast<const float*>(S + L.norm_stats), a->norm_w, gn,
-                               Wk + W.g_bf16, dnorm_w, dnorm_b, static_cast<int>(T), d->C, st))
-        return 1;
-      g16 = Wk + W.g_bf16;
+    } else if (launch_layernorm_bwd(dy, a->out_dtype, ylast, stats, a->norm_w, gn, Wk + W.g_bf16, dnorm_w, dnorm_b,
+                                    static_cast<int>(T), d->C, st, a->out_shuffle ? d->W : 0)) {
+      return 1;
     }
     g32 = gn;
+    g16 = Wk + W.g_bf16;
   }
   for (int i = a->depth - 1; i >= 0; --i) {
     const crf_block_desc bd = block_desc_of(*d, i);
@@ -525,7 +512,8 @@ int crf_layernorm_ps_fwd(const float* x, const float* gamma, const float* beta, 
   CRF_CHECK(x && gamma && beta && y && stats && B > 0 && H > 0 && W > 0, "crf_layernorm_ps_fwd: bad arguments");
   DeviceGuard guard(device);
   CRF_CHECK(guard.ok, "cannot select device %d", device);
-  return launch_layernorm_ps_fwd(x, gamma, beta, eps, y, y_dtype, stats, B, H, W, C, static_cast<cudaStream_t>(stream));
+  return launch_layernorm_fwd(x, gamma, beta, eps, y, y_dtype, stats, B * H * W, C, static_cast<cudaStream_t>(stream),
+                              W);
 }
 int crf_layernorm_ps_bwd(const void* g, int g_dtype, const float* x, const float* stats, const float* gamma, float* dx,
                          float* dgamma, float* dbeta, int B, int H, int W, int C, int device, void* stream) {
@@ -533,8 +521,8 @@ int crf_layernorm_ps_bwd(const void* g, int g_dtype, const float* x, const float
             "crf_layernorm_ps_bwd: bad arguments");
   DeviceGuard guard(device);
   CRF_CHECK(guard.ok, "cannot select device %d", device);
-  return launch_layernorm_ps_bwd(g, g_dtype, x, stats, gamma, dx, nullptr, dgamma, dbeta, B, H, W, C,
-                                 static_cast<cudaStream_t>(stream));
+  return launch_layernorm_bwd(g, g_dtype, x, stats, gamma, dx, nullptr, dgamma, dbeta, B * H * W, C,
+                              static_cast<cudaStream_t>(stream), W);
 }
 
 int crf_dgrad_ln_bwd(const void* dy_bf16, const void* w_bf16, int K, const float* x, const float* stats,

@@ -112,14 +112,13 @@ bool dgrad_lnbwd_supported(int C, int K);
 int launch_dgrad_lnbwd(const void* dY, const void* W, int K, const float* x, const float* stats, const float* gamma,
                        const float* dres, float* dx, void* dx_bf16, float* dgamma, float* dbeta, int T, int C, int device,
                        cudaStream_t st);
+// The closing LayerNorm of a decoder stage over (T, C) fp32 rows, T = B H W tokens.  shuffle_w = W > 0: the
+// PixelShuffle(2) that follows is folded into the output store / the gradient load, y and g being (B, 2H, 2W, C/4)
+// NHWC maps.
 int launch_layernorm_fwd(const float* x, const float* gamma, const float* beta, float eps, void* y, int y_dtype,
-                         float* stats, int T, int C, cudaStream_t st);
+                         float* stats, int T, int C, cudaStream_t st, int shuffle_w = 0);
 int launch_layernorm_bwd(const void* g, int g_dtype, const float* x, const float* stats, const float* gamma, float* dx,
-                         void* dx_bf16, float* dgamma, float* dbeta, int T, int C, cudaStream_t st);
-int launch_layernorm_ps_fwd(const float* x, const float* gamma, const float* beta, float eps, void* y, int y_dtype,
-                            float* stats, int B, int H, int W, int C, cudaStream_t st);
-int launch_layernorm_ps_bwd(const void* g, int g_dtype, const float* x, const float* stats, const float* gamma, float* dx,
-                            void* dx_bf16, float* dgamma, float* dbeta, int B, int H, int W, int C, cudaStream_t st);
+                         void* dx_bf16, float* dgamma, float* dbeta, int T, int C, cudaStream_t st, int shuffle_w = 0);
 int launch_depth_loss_fwd(const void* pred, int pred_dtype, const float* tgt, int n_img, int H, int W, float* sums,
                           float* G, cudaStream_t st);
 int launch_depth_loss_bwd(const void* pred, int pred_dtype, const float* tgt, const float* G, const float* gout,

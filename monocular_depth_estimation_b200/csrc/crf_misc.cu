@@ -2,6 +2,11 @@
 // change folded in), LayerNorm backward (with the residual add and the gamma/beta reductions folded in), bias
 // gradient column sums, dtype casts, and the stand-alone window gather / scatter / mask used by the bit-exact
 // index tests.  All of these are HBM-bound: coalesced, vectorised accesses, warp-shuffle reductions.
+// The two LayerNorm row kernels (ln_fwd_rows_kernel, ln_bwd_kernel) take the layout of their output / incoming
+// gradient as a template type: token-major rows, or the PixelShuffle(2) map that follows a decoder stage's closing
+// norm.  The shuffled forms are instances of the same kernels, with the same arithmetic in the same order.
+#include <algorithm>
+
 #include "crf_host.h"
 #include "crf_ptx.cuh"
 #include "crf_window.cuh"
@@ -85,7 +90,8 @@ ln_fwd_kernel(const TIn* __restrict__ x, int64_t sb, int64_t st, int64_t sc, int
 // ------------------------------------------------------------------------------------------------
 // LayerNorm forward, row-contiguous fast path (channel stride 1: token-major or channels-last input).
 // One warp per token row, the row lives in registers (each lane owns channels {2*lane + 64k, +1}): x is read
-// exactly once, two-pass mean / variance like torch's kernel.
+// exactly once, two-pass mean / variance like torch's kernel.  Rows is the layout of the output xn (TokenRows /
+// ShuffledRows below).
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float2 load2(const float* p) { return __ldg(reinterpret_cast<const float2*>(p)); }
 __device__ __forceinline__ float2 load2(const __nv_bfloat16* p) {
@@ -98,17 +104,59 @@ __device__ __forceinline__ void store2(__nv_bfloat16* p, float a, float b) {
 }
 __device__ __forceinline__ void store2(float* p, float a, float b) { *reinterpret_cast<float2*>(p) = make_float2(a, b); }
 
-template <typename TIn, int NCH, bool DO_LN, typename TOut = __nv_bfloat16>
+// Row layouts of the two row kernels: where the channel pair (c, c + 1), c even, of token t of a (T, C) tensor p is
+// stored (forward output) or loaded from (backward gradient).  Token-major rows: one packed access at p + t * C + c.
+struct TokenRows {
+  template <int C, typename T>
+  __device__ __forceinline__ void store(T* p, int64_t t, int c, float a, float b) const { store2(p + t * C + c, a, b); }
+  template <int C, typename T>
+  __device__ __forceinline__ float2 load(const T* p, int64_t t, int c) const { return load2(p + t * C + c); }
+};
+
+// The same rows through the PixelShuffle(2) that follows a decoder stage (model_mobileV3_large_newCRFs.py:116-120):
+// token (b, h, w) of an H x W grid, channel c = 4 k' + 2 i + j  <->  element (b, 2h + i, 2w + j, k') of the
+// (B, 2H, 2W, C/4) NHWC map.  A pair (c, c + 1) is j = 0 / 1 of one output row: two scalar accesses C/4 apart.
+// Output row 2h + i of image b is row 2 (b H + h) + i of the batch, so only W enters the map.
+struct ShuffledRows {
+  int W;
+  template <int C>
+  __device__ __forceinline__ int64_t offset(int64_t t, int c) const {
+    const int ti = static_cast<int>(t);  // T = B H W is an int in the launchers
+    const int w = ti % W, bh = ti / W;
+    // c = 64 k + lo with k the unrolled loop index: written this way the compiler sees that only lo moves the
+    // address off a per-lane base, so all of a row's accesses share one base register
+    const int lo = c & 63;
+    const int64_t pix = (static_cast<int64_t>(bh) * 2 + ((lo >> 1) & 1)) * 2 * W + 2 * w;
+    return pix * (C / 4) + (lo >> 2) + 16 * (c >> 6);
+  }
+  template <int C, typename T>
+  __device__ __forceinline__ void store(T* p, int64_t t, int c, float a, float b) const {
+    T* o = p + offset<C>(t, c);
+    o[0] = T(a);
+    o[C / 4] = T(b);
+  }
+  template <int C, typename T>
+  __device__ __forceinline__ float2 load(const T* p, int64_t t, int c) const {
+    const T* o = p + offset<C>(t, c);
+    return make_float2(static_cast<float>(__ldg(o)), static_cast<float>(__ldg(o + C / 4)));
+  }
+};
+
+template <typename TIn, int NCH, bool DO_LN, typename TOut, typename Rows>
 __global__ void __launch_bounds__(256)
 ln_fwd_rows_kernel(const TIn* __restrict__ x, int64_t sb, int64_t st, int T_img, int64_t T,
                    const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
-                   TOut* __restrict__ xn, float* __restrict__ stats, float* __restrict__ x_copy) {
+                   TOut* __restrict__ xn, float* __restrict__ stats, float* __restrict__ x_copy, const Rows rows) {
   pdl_prologue();
   constexpr int C = 64 * NCH;
+  // Input strided per image (sb, T_img) and the fp32 copy of x are LN1's, which is token-major.  The shuffled
+  // (closing-norm) instances read one contiguous (T, C) block (sb = 0, T_img = T) and never copy x: without the 64-bit
+  // division and the copy branch they have no stack frame and no spills (launch_ln_fwd_rows checks both conditions).
+  constexpr bool kLn1 = std::is_same<Rows, TokenRows>::value;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t warps_total = static_cast<int64_t>(gridDim.x) * 8;
   for (int64_t t = static_cast<int64_t>(blockIdx.x) * 8 + warp; t < T; t += warps_total) {
-    const int64_t b = t / T_img;
+    const int64_t b = kLn1 ? t / T_img : 0;
     const TIn* row = x + b * sb + (t - b * T_img) * st;
     float2 v[NCH];
     float s = 0.f;
@@ -135,7 +183,7 @@ ln_fwd_rows_kernel(const TIn* __restrict__ x, int64_t sb, int64_t st, int T_img,
 #pragma unroll
     for (int k = 0; k < NCH; ++k) {
       const int c = 64 * k + 2 * lane;
-      if (x_copy != nullptr) *reinterpret_cast<float2*>(x_copy + t * C + c) = v[k];
+      if (kLn1 && x_copy != nullptr) *reinterpret_cast<float2*>(x_copy + t * C + c) = v[k];
       float a0 = v[k].x, a1 = v[k].y;
       if (DO_LN) {
         const float2 g = __ldg(reinterpret_cast<const float2*>(gamma + c));
@@ -143,7 +191,7 @@ ln_fwd_rows_kernel(const TIn* __restrict__ x, int64_t sb, int64_t st, int T_img,
         a0 = (a0 - mean) * rstd * g.x + be.x;
         a1 = (a1 - mean) * rstd * g.y + be.y;
       }
-      store2(xn + t * C + c, a0, a1);
+      rows.template store<C>(xn, t, c, a0, a1);
     }
   }
 }
@@ -152,12 +200,14 @@ ln_fwd_rows_kernel(const TIn* __restrict__ x, int64_t sb, int64_t st, int T_img,
 // LayerNorm backward.  One warp per token row (grid-stride); each lane owns channels {2*lane + 64k, +1}.
 //   dx = rstd * (g*gamma - mean_c(g*gamma) - xhat * mean_c(g*gamma*xhat)) + dres
 //   dgamma += sum_t g * xhat,  dbeta += sum_t g
+// Rows is the layout of g (TokenRows / ShuffledRows); x, dres and dx are token-major.
 // ------------------------------------------------------------------------------------------------
-template <int NCH, typename TG = float>  // C = 64 * NCH
+template <int NCH, typename TG, typename Rows>  // C = 64 * NCH
 __global__ void __launch_bounds__(256)
 ln_bwd_kernel(const TG* __restrict__ g, const float* __restrict__ x, const float* __restrict__ stats,
               const float* __restrict__ gamma, const float* __restrict__ dres, float* __restrict__ dx,
-              __nv_bfloat16* __restrict__ dx_bf16, float* __restrict__ dgamma, float* __restrict__ dbeta, int T) {
+              __nv_bfloat16* __restrict__ dx_bf16, float* __restrict__ dgamma, float* __restrict__ dbeta, int T,
+              const Rows rows) {
   pdl_prologue();
   constexpr int C = 64 * NCH;
   __shared__ __align__(16) float red[8][64];
@@ -172,14 +222,12 @@ ln_bwd_kernel(const TG* __restrict__ g, const float* __restrict__ x, const float
   const int warps_total = gridDim.x * 8;
   for (int t = blockIdx.x * 8 + warp; t < T; t += warps_total) {
     const float mean = __ldg(stats + 2 * t), rstd = __ldg(stats + 2 * t + 1);
-    const TG* gr = g + static_cast<int64_t>(t) * C;
-    const float* xr = x + static_cast<int64_t>(t) * C;
     float2 gv[NCH], xh[NCH];
     float s1 = 0.f, s2 = 0.f;
 #pragma unroll
     for (int k = 0; k < NCH; ++k) {
-      gv[k] = load2(gr + 64 * k + 2 * lane);
-      const float2 xv = __ldg(reinterpret_cast<const float2*>(xr + 64 * k + 2 * lane));
+      gv[k] = rows.template load<C>(g, t, 64 * k + 2 * lane);
+      const float2 xv = __ldg(reinterpret_cast<const float2*>(x + static_cast<int64_t>(t) * C + 64 * k + 2 * lane));
       xh[k] = make_float2((xv.x - mean) * rstd, (xv.y - mean) * rstd);
       dga[k].x += gv[k].x * xh[k].x; dga[k].y += gv[k].y * xh[k].y;
       dbe[k].x += gv[k].x;           dbe[k].y += gv[k].y;
@@ -405,6 +453,91 @@ pixel_shuffle_nhwc_kernel(const T* __restrict__ src, T* __restrict__ dst, int B,
   }
 }
 
+// Calls f(std::integral_constant<int, C / 64>()) for a width the row kernels are instantiated for (C = 64 .. 1024 in
+// steps of 64) and returns its result; returns -1 for any other C.
+template <typename F>
+int with_nch(int C, F&& f) {
+  if (C % 64 != 0) return -1;
+  switch (C / 64) {
+    case 1: return f(std::integral_constant<int, 1>());
+    case 2: return f(std::integral_constant<int, 2>());
+    case 3: return f(std::integral_constant<int, 3>());
+    case 4: return f(std::integral_constant<int, 4>());
+    case 5: return f(std::integral_constant<int, 5>());
+    case 6: return f(std::integral_constant<int, 6>());
+    case 7: return f(std::integral_constant<int, 7>());
+    case 8: return f(std::integral_constant<int, 8>());
+    case 9: return f(std::integral_constant<int, 9>());
+    case 10: return f(std::integral_constant<int, 10>());
+    case 11: return f(std::integral_constant<int, 11>());
+    case 12: return f(std::integral_constant<int, 12>());
+    case 13: return f(std::integral_constant<int, 13>());
+    case 14: return f(std::integral_constant<int, 14>());
+    case 15: return f(std::integral_constant<int, 15>());
+    case 16: return f(std::integral_constant<int, 16>());
+    default: return -1;
+  }
+}
+
+// Calls f with the row layout: the PixelShuffle(2) map of a token grid W wide when W > 0, token-major otherwise
+template <typename F>
+int with_rows(int W, F&& f) {
+  return W > 0 ? f(ShuffledRows{W}) : f(TokenRows{});
+}
+
+// Grid of the warp-per-row kernels: one CTA per 8 rows, at most ctas_per_sm CTAs per SM (the kernels grid-stride)
+int row_grid(int64_t rows, int ctas_per_sm) {
+  int dev = 0;
+  cudaGetDevice(&dev);
+  return static_cast<int>(std::min<int64_t>((rows + 7) / 8, static_cast<int64_t>(num_sms(dev)) * ctas_per_sm));
+}
+
+template <typename TIn, bool DO_LN, typename TOut, typename Rows>
+int launch_ln_fwd_rows(const TIn* x, int64_t sb, int64_t st_, int T_img, int64_t T, int C, const float* gamma,
+                       const float* beta, float eps, TOut* xn, float* stats, float* x_copy, Rows rows,
+                       int ctas_per_sm, cudaStream_t st) {
+  // the shuffled instances read one contiguous (T, C) block and write no copy of x (see the kernel)
+  CRF_CHECK((std::is_same<Rows, TokenRows>::value || (x_copy == nullptr && sb == 0 && T_img == T)),
+            "LayerNorm forward: the PixelShuffle(2) layout takes contiguous rows and no copy of x");
+  const int blocks = row_grid(T, ctas_per_sm);
+  const int rc = with_nch(C, [&](auto nch) {
+    launch_pdl((ln_fwd_rows_kernel<TIn, decltype(nch)::value, DO_LN, TOut, Rows>), blocks, 256, 0, st, x, sb, st_,
+               T_img, T, gamma, beta, eps, xn, stats, x_copy, rows);
+    return 0;
+  });
+  if (rc < 0) return set_error("LayerNorm forward: no row kernel for C=%d", C);
+  CRF_CUDA(cudaGetLastError());
+  note_launch();
+  return 0;
+}
+
+// ctas_per_sm = 0: one resident wave, occupancy x SMs with at most 8 CTAs per SM
+template <typename TG, typename Rows>
+int launch_ln_bwd_rows(const TG* g, Rows rows, const float* x, const float* stats, const float* gamma,
+                       const float* dres, float* dx, void* dx_bf16, float* dgamma, float* dbeta, int T, int C,
+                       int ctas_per_sm, cudaStream_t st) {
+  __nv_bfloat16* dxb = reinterpret_cast<__nv_bfloat16*>(dx_bf16);
+  const int rc = with_nch(C, [&](auto nch) {
+    const auto kern = ln_bwd_kernel<decltype(nch)::value, TG, Rows>;
+    int cap = ctas_per_sm;
+    if (cap == 0) {
+      static int occ = 0;
+      if (occ == 0) {
+        int o = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, kern, 256, 0) != cudaSuccess || o < 1) o = 1;
+        occ = o > 8 ? 8 : o;
+      }
+      cap = occ;
+    }
+    launch_pdl(kern, row_grid(T, cap), 256, 0, st, g, x, stats, gamma, dres, dx, dxb, dgamma, dbeta, T, rows);
+    return 0;
+  });
+  if (rc < 0) return set_error("LayerNorm backward: no row kernel for C=%d", C);
+  CRF_CUDA(cudaGetLastError());
+  note_launch();
+  return 0;
+}
+
 template <typename TIn>
 int launch_ln_fwd_t(const void* x, int64_t sb, int64_t st_, int64_t sc, int B, int T_img, int C, const float* gamma,
                     const float* beta, float eps, void* xn, float* stats, float* x_copy, cudaStream_t st) {
@@ -415,30 +548,14 @@ int launch_ln_fwd_t(const void* x, int64_t sb, int64_t st_, int64_t sc, int B, i
                  gamma != nullptr ? "ln_fwd" : "convert_bf16", B * T_img, C);
   const bool aligned = (reinterpret_cast<uintptr_t>(x) % 8 == 0) && (sb % 2 == 0) && (st_ % 2 == 0);
   if (sc == 1 && aligned) {  // rows are contiguous: warp-per-row, row held in registers, x read once
-    int dev = 0;
-    cudaGetDevice(&dev);
-    const int64_t T = static_cast<int64_t>(B) * T_img;
-    int blocks = static_cast<int>((T + 7) / 8);
-    const int cap = num_sms(dev) * 16;
-    if (blocks > cap) blocks = cap;
     const TIn* xp = reinterpret_cast<const TIn*>(x);
+    const int64_t T = static_cast<int64_t>(B) * T_img;
     __nv_bfloat16* xnp = reinterpret_cast<__nv_bfloat16*>(xn);
-#define CRF_LNF(NCH)                                                                                                  \
-  case NCH:                                                                                                           \
-    if (gamma != nullptr)                                                                                             \
-      launch_pdl((ln_fwd_rows_kernel<TIn, NCH, true>), blocks, 256, 0, st, xp, sb, st_, T_img, T, gamma, beta, eps, xnp, stats, x_copy); \
-    else                                                                                                              \
-      launch_pdl((ln_fwd_rows_kernel<TIn, NCH, false>), blocks, 256, 0, st, xp, sb, st_, T_img, T, nullptr, nullptr, eps, xnp, nullptr, x_copy); \
-    break;
-    switch (C / 64) {
-      CRF_LNF(1) CRF_LNF(2) CRF_LNF(3) CRF_LNF(4) CRF_LNF(5) CRF_LNF(6) CRF_LNF(7) CRF_LNF(8) CRF_LNF(9) CRF_LNF(10)
-      CRF_LNF(11) CRF_LNF(12) CRF_LNF(13) CRF_LNF(14) CRF_LNF(15) CRF_LNF(16)
-      default: return set_error("ln_fwd: unsupported C=%d for the row kernel", C);
-    }
-#undef CRF_LNF
-    CRF_CUDA(cudaGetLastError());
-    note_launch();
-    return 0;
+    if (gamma != nullptr)
+      return launch_ln_fwd_rows<TIn, true>(xp, sb, st_, T_img, T, C, gamma, beta, eps, xnp, stats, x_copy, TokenRows{},
+                                           16, st);
+    return launch_ln_fwd_rows<TIn, false>(xp, sb, st_, T_img, T, C, nullptr, nullptr, eps, xnp, nullptr, x_copy,
+                                          TokenRows{}, 16, st);
   }
   if (gamma != nullptr) {
     auto k = ln_fwd_kernel<TIn, true>;
@@ -484,289 +601,55 @@ int launch_convert_tokens(const void* src, int dtype, int64_t sb, int64_t st_, i
 int launch_ln_bwd(const float* g, const float* x, const float* stats, const float* gamma, const float* dres,
                   float* dx, void* dx_bf16, float* dgamma, float* dbeta, int T, int C, cudaStream_t st) {
   CRF_CHECK(C % 64 == 0, "ln_bwd: C=%d must be a multiple of 64", C);
-  int dev = 0;
-  cudaGetDevice(&dev);
-  // one warp per row, grid-stride; ONE resident wave of CTAs (occupancy x SMs): the wide rows (C >= 512: 100-170
-  // registers per thread, 1-2 CTAs per SM) otherwise ran 300 CTAs as 2.03 waves = 3 rounds of latency-bound work, and
-  // every CTA ends with 2 C column reductions into dgamma / dbeta
-  const int sms = num_sms(dev);
-  __nv_bfloat16* dxb = reinterpret_cast<__nv_bfloat16*>(dx_bf16);
   KernelTimer tm(st, 0.0, static_cast<double>(T) * C * (12 + (dres != nullptr ? 4 : 0) + (dx_bf16 != nullptr ? 2 : 0)),
                  "ln_bwd_T%d_C%d", T, C);
-#define CRF_LNB(NCH)                                                                                         \
-  case NCH: {                                                                                                \
-    static int occ = 0;                                                                                      \
-    if (occ == 0) {                                                                                          \
-      int o = 0;                                                                                             \
-      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, ln_bwd_kernel<NCH, float>, 256, 0) != cudaSuccess || o < 1) o = 1; \
-      occ = o > 8 ? 8 : o;                                                                                   \
-    }                                                                                                        \
-    int blocks = (T + 7) / 8;                                                                                \
-    if (blocks > sms * occ) blocks = sms * occ;                                                              \
-    launch_pdl((ln_bwd_kernel<NCH>), blocks, 256, 0, st, g, x, stats, gamma, dres, dx, dxb, dgamma, dbeta, T);         \
-    break;                                                                                                   \
-  }
-  switch (C / 64) {
-    CRF_LNB(1) CRF_LNB(2) CRF_LNB(3) CRF_LNB(4) CRF_LNB(5) CRF_LNB(6) CRF_LNB(7) CRF_LNB(8) CRF_LNB(9) CRF_LNB(10)
-    CRF_LNB(11) CRF_LNB(12) CRF_LNB(13) CRF_LNB(14) CRF_LNB(15) CRF_LNB(16)
-    default: return set_error("ln_bwd: unsupported C=%d", C);
-  }
-#undef CRF_LNB
-  CRF_CUDA(cudaGetLastError());
-  note_launch();
-  return 0;
-}
-
-// ------------------------------------------------------------------------------------------------
-// The closing LayerNorm of a decoder stage with the PixelShuffle(2) that follows it folded into its store / load
-// (model_mobileV3_large_newCRFs.py:116-120: `PixelShuffle(2)` between the stages, fed by newcrf_layers.py:430-432).
-// Token (b, h, w), channel c = 4 k' + 2 i + j  <->  NHWC element (b, 2h + i, 2w + j, k') of the (B, 2H, 2W, C/4) map.
-// Same arithmetic, in the same order, as ln_fwd_rows_kernel / ln_bwd_kernel (one warp per row, lane owns channels
-// {2 lane + 64 k, +1}): a lane's two channels are the j = 0 / 1 neighbours of one output row i = lane & 1.
-// ------------------------------------------------------------------------------------------------
-template <typename T>
-__device__ __forceinline__ void store1(T* p, float v);
-template <>
-__device__ __forceinline__ void store1<float>(float* p, float v) { *p = v; }
-template <>
-__device__ __forceinline__ void store1<__nv_bfloat16>(__nv_bfloat16* p, float v) { *p = __float2bfloat16(v); }
-__device__ __forceinline__ float load1(const float* p) { return __ldg(p); }
-__device__ __forceinline__ float load1(const __nv_bfloat16* p) { return __bfloat162float(*p); }
-
-template <int NCH, typename TOut>
-__global__ void __launch_bounds__(256)
-layernorm_ps_fwd_kernel(const float* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
-                        float eps, TOut* __restrict__ y, float* __restrict__ stats, int T, int H, int W) {
-  pdl_prologue();
-  constexpr int C = 64 * NCH, C4 = C / 4;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int warps_total = gridDim.x * 8;
-  for (int t = blockIdx.x * 8 + warp; t < T; t += warps_total) {
-    const float* row = x + static_cast<int64_t>(t) * C;
-    float2 v[NCH];
-    float s = 0.f;
-#pragma unroll
-    for (int k = 0; k < NCH; ++k) {
-      v[k] = load2(row + 64 * k + 2 * lane);
-      s += v[k].x + v[k].y;
-    }
-    const float mean = warp_sum(s) * (1.0f / C);
-    float q = 0.f;
-#pragma unroll
-    for (int k = 0; k < NCH; ++k) {
-      const float d0 = v[k].x - mean, d1 = v[k].y - mean;
-      q += d0 * d0 + d1 * d1;
-    }
-    const float rstd = rsqrtf(warp_sum(q) * (1.0f / C) + eps);
-    if (lane == 0) {
-      stats[2 * t] = mean;
-      stats[2 * t + 1] = rstd;
-    }
-    const int w = t % W, bh = t / W, h = bh % H, b = bh / H;
-    const int64_t pix = (static_cast<int64_t>(b) * 2 * H + 2 * h + (lane & 1)) * 2 * W + 2 * w;   // (i = lane & 1, j = 0)
-#pragma unroll
-    for (int k = 0; k < NCH; ++k) {
-      const int c = 64 * k + 2 * lane;
-      const float2 g = __ldg(reinterpret_cast<const float2*>(gamma + c));
-      const float2 be = __ldg(reinterpret_cast<const float2*>(beta + c));
-      const int kp = 16 * k + (lane >> 1);
-      store1(y + pix * C4 + kp, (v[k].x - mean) * rstd * g.x + be.x);
-      store1(y + (pix + 1) * C4 + kp, (v[k].y - mean) * rstd * g.y + be.y);
-    }
-  }
-}
-
-template <int NCH, typename TG>
-__global__ void __launch_bounds__(256)
-layernorm_ps_bwd_kernel(const TG* __restrict__ g, const float* __restrict__ x, const float* __restrict__ stats,
-                        const float* __restrict__ gamma, float* __restrict__ dx, __nv_bfloat16* __restrict__ dx_bf16,
-                        float* __restrict__ dgamma, float* __restrict__ dbeta, int T, int H, int W) {
-  pdl_prologue();
-  constexpr int C = 64 * NCH, C4 = C / 4;
-  __shared__ float red[8][64];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  float2 gam[NCH], dga[NCH], dbe[NCH];
-#pragma unroll
-  for (int k = 0; k < NCH; ++k) {
-    gam[k] = __ldg(reinterpret_cast<const float2*>(gamma + 64 * k + 2 * lane));
-    dga[k] = make_float2(0.f, 0.f);
-    dbe[k] = make_float2(0.f, 0.f);
-  }
-  const int warps_total = gridDim.x * 8;
-  for (int t = blockIdx.x * 8 + warp; t < T; t += warps_total) {
-    const float mean = __ldg(stats + 2 * t), rstd = __ldg(stats + 2 * t + 1);
-    const float* xr = x + static_cast<int64_t>(t) * C;
-    const int w = t % W, bh = t / W, h = bh % H, b = bh / H;
-    const int64_t pix = (static_cast<int64_t>(b) * 2 * H + 2 * h + (lane & 1)) * 2 * W + 2 * w;
-    float2 gv[NCH], xh[NCH];
-    float s1 = 0.f, s2 = 0.f;
-#pragma unroll
-    for (int k = 0; k < NCH; ++k) {
-      const int kp = 16 * k + (lane >> 1);
-      gv[k] = make_float2(load1(g + pix * C4 + kp), load1(g + (pix + 1) * C4 + kp));
-      const float2 xv = __ldg(reinterpret_cast<const float2*>(xr + 64 * k + 2 * lane));
-      xh[k] = make_float2((xv.x - mean) * rstd, (xv.y - mean) * rstd);
-      dga[k].x += gv[k].x * xh[k].x; dga[k].y += gv[k].y * xh[k].y;
-      dbe[k].x += gv[k].x;           dbe[k].y += gv[k].y;
-      gv[k].x *= gam[k].x;           gv[k].y *= gam[k].y;
-      s1 += gv[k].x + gv[k].y;
-      s2 += gv[k].x * xh[k].x + gv[k].y * xh[k].y;
-    }
-    s1 = warp_sum(s1) * (1.0f / C);
-    s2 = warp_sum(s2) * (1.0f / C);
-#pragma unroll
-    for (int k = 0; k < NCH; ++k) {
-      const float o0 = rstd * (gv[k].x - s1 - xh[k].x * s2);
-      const float o1 = rstd * (gv[k].y - s1 - xh[k].y * s2);
-      const int64_t off = static_cast<int64_t>(t) * C + 64 * k + 2 * lane;
-      if (dx != nullptr) *reinterpret_cast<float2*>(dx + off) = make_float2(o0, o1);
-      if (dx_bf16 != nullptr) *reinterpret_cast<uint32_t*>(dx_bf16 + off) = pack_bf16(o0, o1);
-    }
-  }
-#pragma unroll
-  for (int k = 0; k < NCH; ++k) {
-    for (int pass = 0; pass < 2; ++pass) {
-      const float2 v = pass == 0 ? dga[k] : dbe[k];
-      red[warp][2 * lane] = v.x;
-      red[warp][2 * lane + 1] = v.y;
-      __syncthreads();
-      if (threadIdx.x < 64) {
-        float s = 0.f;
-#pragma unroll
-        for (int w8 = 0; w8 < 8; ++w8) s += red[w8][threadIdx.x];
-        atomicAdd((pass == 0 ? dgamma : dbeta) + 64 * k + threadIdx.x, s);
-      }
-      __syncthreads();
-    }
-  }
+  // ONE resident wave of CTAs (occupancy x SMs): the wide rows (C >= 512: 100-170 registers per thread, 1-2 CTAs per
+  // SM) otherwise ran 300 CTAs as 2.03 waves = 3 rounds of latency-bound work, and every CTA ends with 2 C column
+  // reductions into dgamma / dbeta
+  return launch_ln_bwd_rows(g, TokenRows{}, x, stats, gamma, dres, dx, dx_bf16, dgamma, dbeta, T, C, 0, st);
 }
 
 // Stand-alone LayerNorm over contiguous (T, C) fp32 rows (the final norm_crf of a decoder stage,
-// newcrf_layers.py:430-431): y fp32 or bf16, stats (mean, rstd) for the backward.
+// newcrf_layers.py:430-431): y fp32 or bf16, stats (mean, rstd) for the backward.  With shuffle_w > 0 the
+// PixelShuffle(2) that follows the stage is folded into the store: y is the (B, 2H, 2W, C/4) NHWC map of the
+// (B, H, W) token grid, W = shuffle_w.
 int launch_layernorm_fwd(const float* x, const float* gamma, const float* beta, float eps, void* y, int y_dtype,
-                         float* stats, int T, int C, cudaStream_t st) {
-  CRF_CHECK(C % 64 == 0 && C >= 64 && C <= 1024, "layernorm_fwd: C=%d must be a multiple of 64 in [64,1024]", C);
-  CRF_CHECK(y_dtype == CRF_DT_F32 || y_dtype == CRF_DT_BF16, "layernorm_fwd: unsupported output dtype %d", y_dtype);
-  int dev = 0;
-  cudaGetDevice(&dev);
-  int blocks = (T + 7) / 8;
-  const int cap = num_sms(dev) * 16;
-  if (blocks > cap) blocks = cap;
-  KernelTimer tm(st, 0.0, static_cast<double>(T) * C * (4 + (y_dtype == CRF_DT_F32 ? 4 : 2)), "layernorm_fwd_T%d_C%d", T, C);
-#define CRF_LNS(NCH)                                                                                                   \
-  case NCH:                                                                                                            \
-    if (y_dtype == CRF_DT_F32)                                                                                         \
-      launch_pdl((ln_fwd_rows_kernel<float, NCH, true, float>), blocks, 256, 0, st, x, 0, C, T, T, gamma, beta, eps,             \
-                                                                            reinterpret_cast<float*>(y), stats, nullptr); \
-    else                                                                                                               \
-      launch_pdl((ln_fwd_rows_kernel<float, NCH, true, __nv_bfloat16>), blocks, 256, 0, st,                                      \
-          x, 0, C, T, T, gamma, beta, eps, reinterpret_cast<__nv_bfloat16*>(y), stats, nullptr);                       \
-    break;
-  switch (C / 64) {
-    CRF_LNS(1) CRF_LNS(2) CRF_LNS(3) CRF_LNS(4) CRF_LNS(5) CRF_LNS(6) CRF_LNS(7) CRF_LNS(8) CRF_LNS(9) CRF_LNS(10)
-    CRF_LNS(11) CRF_LNS(12) CRF_LNS(13) CRF_LNS(14) CRF_LNS(15) CRF_LNS(16)
-    default: return set_error("layernorm_fwd: unsupported C=%d", C);
-  }
-#undef CRF_LNS
-  CRF_CUDA(cudaGetLastError());
-  note_launch();
-  return 0;
+                         float* stats, int T, int C, cudaStream_t st, int shuffle_w) {
+  const bool ps = shuffle_w > 0;
+  const char* name = ps ? "layernorm_ps_fwd" : "layernorm_fwd";
+  CRF_CHECK(C % 64 == 0 && C >= 64 && C <= 1024, "%s: C=%d must be a multiple of 64 in [64,1024]", name, C);
+  CRF_CHECK(y_dtype == CRF_DT_F32 || y_dtype == CRF_DT_BF16, "%s: unsupported output dtype %d", name, y_dtype);
+  KernelTimer tm(st, 0.0, static_cast<double>(T) * C * (4 + (y_dtype == CRF_DT_F32 ? 4 : 2)), "%s_T%d_C%d", name, T, C);
+  const int ctas_per_sm = ps ? 8 : 16;
+  return with_rows(shuffle_w, [&](auto rows) {
+    if (y_dtype == CRF_DT_F32)
+      return launch_ln_fwd_rows<float, true>(x, 0, C, T, T, C, gamma, beta, eps, static_cast<float*>(y), stats, nullptr,
+                                             rows, ctas_per_sm, st);
+    return launch_ln_fwd_rows<float, true>(x, 0, C, T, T, C, gamma, beta, eps, static_cast<__nv_bfloat16*>(y), stats,
+                                           nullptr, rows, ctas_per_sm, st);
+  });
 }
 
+// Its backward; with shuffle_w > 0, g is the gradient of the shuffled NHWC map.
 int launch_layernorm_bwd(const void* g, int g_dtype, const float* x, const float* stats, const float* gamma, float* dx,
-                         void* dx_bf16, float* dgamma, float* dbeta, int T, int C, cudaStream_t st) {
-  __nv_bfloat16* dxb = reinterpret_cast<__nv_bfloat16*>(dx_bf16);
-  CRF_CHECK(C % 64 == 0 && C >= 64 && C <= 1024, "layernorm_bwd: C=%d must be a multiple of 64 in [64,1024]", C);
-  CRF_CHECK(g_dtype == CRF_DT_F32 || g_dtype == CRF_DT_BF16, "layernorm_bwd: unsupported gradient dtype %d", g_dtype);
-  int dev = 0;
-  cudaGetDevice(&dev);
-  int blocks = (T + 7) / 8;
-  const int cap = num_sms(dev) * 8;
-  if (blocks > cap) blocks = cap;
-  KernelTimer tm(st, 0.0, static_cast<double>(T) * C * (8 + (g_dtype == CRF_DT_F32 ? 4 : 2)), "layernorm_bwd_T%d_C%d", T, C);
-#define CRF_LNSB(NCH)                                                                                                  \
-  case NCH:                                                                                                            \
-    if (g_dtype == CRF_DT_F32)                                                                                         \
-      launch_pdl((ln_bwd_kernel<NCH, float>), blocks, 256, 0, st, reinterpret_cast<const float*>(g), x, stats, gamma, nullptr,   \
-                                                        dx, dxb, dgamma, dbeta, T);                                    \
-    else                                                                                                               \
-      launch_pdl((ln_bwd_kernel<NCH, __nv_bfloat16>), blocks, 256, 0, st, reinterpret_cast<const __nv_bfloat16*>(g), x, stats,    \
-                                                                gamma, nullptr, dx, dxb, dgamma, dbeta, T);            \
-    break;
-  switch (C / 64) {
-    CRF_LNSB(1) CRF_LNSB(2) CRF_LNSB(3) CRF_LNSB(4) CRF_LNSB(5) CRF_LNSB(6) CRF_LNSB(7) CRF_LNSB(8) CRF_LNSB(9)
-    CRF_LNSB(10) CRF_LNSB(11) CRF_LNSB(12) CRF_LNSB(13) CRF_LNSB(14) CRF_LNSB(15) CRF_LNSB(16)
-    default: return set_error("layernorm_bwd: unsupported C=%d", C);
-  }
-#undef CRF_LNSB
-  CRF_CUDA(cudaGetLastError());
-  note_launch();
-  return 0;
-}
-
-// The closing LayerNorm with the following PixelShuffle(2) folded in: y / g are (B, 2H, 2W, C/4) NHWC maps.
-int launch_layernorm_ps_fwd(const float* x, const float* gamma, const float* beta, float eps, void* y, int y_dtype,
-                            float* stats, int B, int H, int W, int C, cudaStream_t st) {
-  CRF_CHECK(C % 64 == 0 && C >= 64 && C <= 1024, "layernorm_ps_fwd: C=%d must be a multiple of 64 in [64,1024]", C);
-  CRF_CHECK(y_dtype == CRF_DT_F32 || y_dtype == CRF_DT_BF16, "layernorm_ps_fwd: unsupported output dtype %d", y_dtype);
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const int T = B * H * W;
-  int blocks = (T + 7) / 8;
-  const int cap = num_sms(dev) * 8;
-  if (blocks > cap) blocks = cap;
-  KernelTimer tm(st, 0.0, static_cast<double>(T) * C * (4 + (y_dtype == CRF_DT_F32 ? 4 : 2)), "layernorm_ps_fwd_T%d_C%d", T, C);
-#define CRF_LPS(NCH)                                                                                                    \
-  case NCH:                                                                                                             \
-    if (y_dtype == CRF_DT_F32)                                                                                          \
-      launch_pdl((layernorm_ps_fwd_kernel<NCH, float>), blocks, 256, 0, st, x, gamma, beta, eps, reinterpret_cast<float*>(y), stats, \
-                                                                   T, H, W);                                            \
-    else                                                                                                                \
-      launch_pdl((layernorm_ps_fwd_kernel<NCH, __nv_bfloat16>), blocks, 256, 0, st, x, gamma, beta, eps,                          \
-                                                                           reinterpret_cast<__nv_bfloat16*>(y), stats, T, H, W); \
-    break;
-  switch (C / 64) {
-    CRF_LPS(1) CRF_LPS(2) CRF_LPS(3) CRF_LPS(4) CRF_LPS(5) CRF_LPS(6) CRF_LPS(7) CRF_LPS(8) CRF_LPS(9) CRF_LPS(10)
-    CRF_LPS(11) CRF_LPS(12) CRF_LPS(13) CRF_LPS(14) CRF_LPS(15) CRF_LPS(16)
-    default: return set_error("layernorm_ps_fwd: unsupported C=%d", C);
-  }
-#undef CRF_LPS
-  CRF_CUDA(cudaGetLastError());
-  note_launch();
-  return 0;
-}
-
-int launch_layernorm_ps_bwd(const void* g, int g_dtype, const float* x, const float* stats, const float* gamma, float* dx,
-                            void* dx_bf16, float* dgamma, float* dbeta, int B, int H, int W, int C, cudaStream_t st) {
-  CRF_CHECK(C % 64 == 0 && C >= 64 && C <= 1024, "layernorm_ps_bwd: C=%d must be a multiple of 64 in [64,1024]", C);
-  CRF_CHECK(g_dtype == CRF_DT_F32 || g_dtype == CRF_DT_BF16, "layernorm_ps_bwd: unsupported gradient dtype %d", g_dtype);
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const int T = B * H * W;
-  int blocks = (T + 7) / 8;
-  const int cap = num_sms(dev) * (C >= 512 ? 1 : 4);
-  if (blocks > cap) blocks = cap;
-  __nv_bfloat16* dxb = reinterpret_cast<__nv_bfloat16*>(dx_bf16);
-  KernelTimer tm(st, 0.0, static_cast<double>(T) * C * ((g_dtype == CRF_DT_F32 ? 4 : 2) + 8 + (dx_bf16 != nullptr ? 2 : 0)),
-                 "layernorm_ps_bwd_T%d_C%d", T, C);
-#define CRF_LPB(NCH)                                                                                                    \
-  case NCH:                                                                                                             \
-    if (g_dtype == CRF_DT_F32)                                                                                          \
-      launch_pdl((layernorm_ps_bwd_kernel<NCH, float>), blocks, 256, 0, st, reinterpret_cast<const float*>(g), x, stats, gamma, dx, \
-                                                                   dxb, dgamma, dbeta, T, H, W);                        \
-    else                                                                                                                \
-      launch_pdl((layernorm_ps_bwd_kernel<NCH, __nv_bfloat16>), blocks, 256, 0, st, reinterpret_cast<const __nv_bfloat16*>(g), x,  \
-                                                                           stats, gamma, dx, dxb, dgamma, dbeta, T, H, W); \
-    break;
-  switch (C / 64) {
-    CRF_LPB(1) CRF_LPB(2) CRF_LPB(3) CRF_LPB(4) CRF_LPB(5) CRF_LPB(6) CRF_LPB(7) CRF_LPB(8) CRF_LPB(9) CRF_LPB(10)
-    CRF_LPB(11) CRF_LPB(12) CRF_LPB(13) CRF_LPB(14) CRF_LPB(15) CRF_LPB(16)
-    default: return set_error("layernorm_ps_bwd: unsupported C=%d", C);
-  }
-#undef CRF_LPB
-  CRF_CUDA(cudaGetLastError());
-  note_launch();
-  return 0;
+                         void* dx_bf16, float* dgamma, float* dbeta, int T, int C, cudaStream_t st, int shuffle_w) {
+  const bool ps = shuffle_w > 0;
+  const char* name = ps ? "layernorm_ps_bwd" : "layernorm_bwd";
+  CRF_CHECK(C % 64 == 0 && C >= 64 && C <= 1024, "%s: C=%d must be a multiple of 64 in [64,1024]", name, C);
+  CRF_CHECK(g_dtype == CRF_DT_F32 || g_dtype == CRF_DT_BF16, "%s: unsupported gradient dtype %d", name, g_dtype);
+  // the two labels keep the byte formulas they have always reported, so timings stay comparable across versions:
+  // only layernorm_ps_bwd counts the bf16 twin of dx
+  KernelTimer tm(st, 0.0,
+                 static_cast<double>(T) * C * ((g_dtype == CRF_DT_F32 ? 4 : 2) + 8 + (ps && dx_bf16 != nullptr ? 2 : 0)),
+                 "%s_T%d_C%d", name, T, C);
+  const int ctas_per_sm = ps ? (C >= 512 ? 1 : 4) : 8;
+  return with_rows(shuffle_w, [&](auto rows) {
+    if (g_dtype == CRF_DT_F32)
+      return launch_ln_bwd_rows(static_cast<const float*>(g), rows, x, stats, gamma, nullptr, dx, dx_bf16, dgamma,
+                                dbeta, T, C, ctas_per_sm, st);
+    return launch_ln_bwd_rows(static_cast<const __nv_bfloat16*>(g), rows, x, stats, gamma, nullptr, dx, dx_bf16, dgamma,
+                              dbeta, T, C, ctas_per_sm, st);
+  });
 }
 
 int launch_pixel_shuffle_nhwc(const void* src, void* dst, int dtype, int B, int H, int W, int C, int inverse,

@@ -492,10 +492,12 @@ def test_depth_loss_matches_reference_golden():
 
 @pytest.mark.parametrize("B,H,W,C", [(2, 5, 7, 64), (2, 15, 20, 1024), (8, 30, 40, 512), (3, 9, 11, 256), (1, 1, 1, 128)])
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_layernorm_pixel_shuffle_fused(B, H, W, C, dtype):
+@pytest.mark.parametrize("aligned", [True, False])
+def test_layernorm_pixel_shuffle_fused(B, H, W, C, dtype, aligned):
     """The closing LayerNorm of a decoder stage with the following nn.PixelShuffle(2) folded into its store / load
     (crf_layernorm_ps_fwd / _bwd; model_mobileV3_large_newCRFs.py:116-120): bit-identical to LayerNorm kernel +
-    F.pixel_shuffle, forward and backward."""
+    F.pixel_shuffle, forward and backward.  aligned=False hands both backward calls dgamma / dbeta views 4 bytes into
+    a larger buffer, which takes the kernels' scalar-atomic path in place of the 16-byte vector reduction."""
     import ctypes as Cc
     L = _L()
     lib = L.lib()
@@ -524,19 +526,34 @@ def test_layernorm_pixel_shuffle_fused(B, H, W, C, dtype):
         "layernorm_ps.y")
     # backward
     gy = torch.randn(B, 2 * H, 2 * W, C // 4, generator=g).to(DEV).to(dtype)        # NHWC gradient of the shuffled map
+    def zeros_c(aligned):
+        return torch.zeros(C, device=DEV) if aligned else torch.zeros(C + 4, device=DEV)[1:C + 1]
+
     dx = torch.full((T, C), float("nan"), device=DEV)
-    dgam, dbet = torch.zeros(C, device=DEV), torch.zeros(C, device=DEV)
+    dgam, dbet = zeros_c(aligned), zeros_c(aligned)
     L.check(lib.crf_layernorm_ps_bwd(gy.data_ptr(), dt, x.data_ptr(), stats.data_ptr(), gam.data_ptr(), dx.data_ptr(),
                                      dgam.data_ptr(), dbet.data_ptr(), B, H, W, C, 0, st), "crf_layernorm_ps_bwd")
     g_tok = F.pixel_unshuffle(gy.permute(0, 3, 1, 2), 2).permute(0, 2, 3, 1).reshape(T, C).contiguous()
-    dx2 = torch.empty(T, C, device=DEV)
-    dgam2, dbet2 = torch.zeros(C, device=DEV), torch.zeros(C, device=DEV)
-    L.check(lib.crf_layernorm_bwd(g_tok.data_ptr(), dt, x.data_ptr(), stats.data_ptr(), gam.data_ptr(), dx2.data_ptr(),
-                                  dgam2.data_ptr(), dbet2.data_ptr(), T, C, 0, st), "crf_layernorm_bwd")
+
+    def layernorm_bwd(aligned):
+        dx2 = torch.empty(T, C, device=DEV)
+        dgam2, dbet2 = zeros_c(aligned), zeros_c(aligned)
+        L.check(lib.crf_layernorm_bwd(g_tok.data_ptr(), dt, x.data_ptr(), stats.data_ptr(), gam.data_ptr(),
+                                      dx2.data_ptr(), dgam2.data_ptr(), dbet2.data_ptr(), T, C, 0, st), "crf_layernorm_bwd")
+        return dx2, dgam2, dbet2
+
+    dx2, dgam2, dbet2 = layernorm_bwd(aligned)
     torch.cuda.synchronize()
     assert torch.equal(dx, dx2)
     _check(dgam, dgam2, 1e-5, "layernorm_ps.dgamma")
     _check(dbet, dbet2, 1e-5, "layernorm_ps.dbeta")
+    if not aligned:  # the scalar-atomic path against the vector reduction
+        _, dgam3, dbet3 = layernorm_bwd(True)
+        torch.cuda.synchronize()
+        for got, what in ((dgam, "layernorm_ps.dgamma"), (dgam2, "layernorm.dgamma")):
+            _check(got, dgam3, 1e-5, what + " (unaligned)")
+        for got, what in ((dbet, "layernorm_ps.dbeta"), (dbet2, "layernorm.dbeta")):
+            _check(got, dbet3, 1e-5, what + " (unaligned)")
 
 
 def test_colsum_cast_convert():
