@@ -125,3 +125,12 @@ def test_head_width_validation():
         assert (rc == 0) == ok, (C, nH)
         if not ok:
             assert b"head_dim must be 16, 32, 64 or 128" in lib.crf_last_error()
+    # every width in [64, 1024] that is a multiple of 64, with every supported head width that divides it
+    for C in range(64, 1025, 64):
+        for hd in (16, 32, 64, 128):
+            if C % hd == 0:
+                rc = _sizes(lib, ops.make_desc(1, 7, 7, C, C // hd, 0, device=0))[0]
+                assert rc == 0, (C, hd, lib.crf_last_error())
+    for C in (32, 96, 1088):
+        assert _sizes(lib, ops.make_desc(1, 7, 7, C, 1, 0, device=0))[0] != 0, C
+        assert b"multiple of 64" in lib.crf_last_error(), C

@@ -85,7 +85,8 @@ def test_layer_matches_reference_golden(name):
 
 
 @pytest.mark.parametrize("out_bf16", [False, True])
-@pytest.mark.parametrize("B,H,W,C,nH,depth", [(2, 9, 10, 64, 2, 2), (2, 15, 20, 128, 4, 2), (1, 30, 40, 256, 8, 1)])
+@pytest.mark.parametrize("B,H,W,C,nH,depth", [(2, 9, 10, 64, 2, 2), (2, 15, 20, 128, 4, 2), (1, 30, 40, 256, 8, 1),
+                                               (2, 9, 10, 192, 6, 2), (1, 15, 20, 640, 5, 1)])
 def test_layer_with_pixel_shuffle_folded_in(B, H, W, C, nH, depth, out_bf16):
     """crf_layer_args.out_shuffle: the stage-closing LayerNorm writes nn.PixelShuffle(2) of the stage's NCHW output
     (model_mobileV3_large_newCRFs.py:116-120) -- bit-identical to the unshuffled layer call + F.pixel_shuffle, and the
@@ -125,7 +126,8 @@ def test_layer_with_pixel_shuffle_folded_in(B, H, W, C, nH, depth, out_bf16):
 
 
 @pytest.mark.parametrize("with_norm,out_bf16", [(False, False), (True, False), (True, True)])
-@pytest.mark.parametrize("B,H,W,C,nH,depth", [(2, 9, 10, 64, 2, 2), (2, 15, 20, 128, 4, 3), (1, 30, 40, 256, 8, 1)])
+@pytest.mark.parametrize("B,H,W,C,nH,depth", [(2, 9, 10, 64, 2, 2), (2, 15, 20, 128, 4, 3), (1, 30, 40, 256, 8, 1),
+                                               (2, 9, 10, 192, 6, 2), (1, 15, 20, 640, 5, 1)])
 def test_layer_call_equals_block_by_block(B, H, W, C, nH, depth, with_norm, out_bf16):
     """crf_layer_fwd / crf_layer_bwd (one call per BasicCRFLayer incl. the closing norm_crf) against the same layer run
     block by block through crf_block_fwd / crf_block_bwd + the stand-alone LayerNorm: same kernels, same order of
@@ -354,6 +356,26 @@ def test_head_dim_16_block_vs_oracle(H, W, C, nH, shift):
 def test_wide_head_block_vs_oracle(H, W, C, nH, shift):
     """BASELINE.json configs[2], the head_dim = 64 and 128 points (crf_attn_wide.cu: 32-wide slices of a head)."""
     _run_block_vs_oracle(2, H, W, C, nH, shift, seed=400 + C + shift, strided=True, oracle_device=DEV)
+
+
+# Every width the library accepts that is not a power of two.  The width picks the GEMM kernel of each projection (the
+# CTA-pair kernel needs N % 256 == 0, the persistent one N % 128 == 0, else gemm_kernel<64> with C / 64 column tiles),
+# the LayerNorm row-kernel instance (C / 64 channel groups) and, with the head width, the head count.
+_ODD_WIDTHS = [192, 320, 384, 448, 576, 640, 704, 768, 832, 896, 960]
+_WIDTH_CASES = ([(C, 32, p, 2, 15, 20, 3) for C in _ODD_WIDTHS for p in ("bf16", "fp32")]
+                # head widths other than 32 at these widths: odd head counts of 3 ... 15
+                + [(C, hd, p, 2, 15, 20, 3) for C, hd in [(192, 64), (320, 64), (960, 64), (384, 128), (640, 128),
+                                                          (896, 128), (448, 16)] for p in ("bf16", "fp32")]
+                # T = 9600: the CTA-pair GEMMs run several tiles per pair
+                + [(C, 32, "bf16", 8, 30, 40, 0) for C in (576, 768, 960)])
+
+
+@pytest.mark.parametrize("C,hd,precision,B,H,W,shift", _WIDTH_CASES)
+def test_channel_widths_vs_oracle(C, hd, precision, B, H, W, shift):
+    """One block, forward and backward, at a channel width that is not a power of two, against the fp32 oracle: y, dx,
+    dv, all 13 parameter gradients and the per-token-row error, in both precision modes."""
+    _run_block_vs_oracle(B, H, W, C, C // hd, shift, seed=800 + C + hd, strided=True, oracle_device=DEV,
+                         precision=precision, tol=TOL_FP32 if precision == "fp32" else TOL)
 
 
 def test_inference_path_matches_training_path():

@@ -55,7 +55,9 @@ def _rand_bf16(*shape, seed=0, scale=1.0):
 @pytest.mark.parametrize("M,N,K", [(128, 64, 64), (90, 128, 128), (300, 128, 128), (1000, 256, 512), (257, 64, 192),
                                    (4800, 512, 128), (640, 1024, 256), (384, 128, 2048), (200, 256, 4096),
                                    # 152 / 300 tiles on 148 SMs: the K-split work units with the TMA reduce-add
-                                   (2400, 1024, 4096), (2400, 1024, 1024), (9600, 512, 2048)])
+                                   (2400, 1024, 4096), (2400, 1024, 1024), (9600, 512, 2048),
+                                   # a block's N = C projections at C = 64 (mod 128): gemm_kernel<64>, 3 / 15 column tiles
+                                   (600, 192, 192), (600, 192, 768), (600, 960, 960), (600, 960, 3840)])
 def test_gemm_fprop(M, N, K):
     ops, L = _ops(), _L()
     A, W = _rand_bf16(M, K, seed=1), _rand_bf16(N, K, seed=2, scale=K ** -0.5)
@@ -67,7 +69,9 @@ def test_gemm_fprop(M, N, K):
 
 @pytest.mark.parametrize("M,N,K", [(128, 64, 64), (300, 128, 128), (1000, 512, 128), (257, 128, 512),
                                    (640, 256, 1024), (500, 2048, 512), (2400, 1024, 4096), (2400, 1024, 2048),
-                                   (9600, 512, 2048)])
+                                   (9600, 512, 2048),
+                                   # d fc1 / d qk of a block at C = 320 and 576: gemm_kernel<64>, 5 / 9 column tiles
+                                   (600, 320, 1280), (600, 320, 640), (600, 576, 2304), (600, 576, 1152)])
 def test_gemm_dgrad(M, N, K):
     """dX = dY (M,K) @ W (K,N): B operand read MN-major from the (out,in) weight."""
     ops, L = _ops(), _L()
@@ -80,7 +84,9 @@ def test_gemm_dgrad(M, N, K):
 
 @pytest.mark.parametrize("M,N,K,split", [(128, 64, 64, 1), (128, 128, 1000, 1), (512, 128, 1000, 4),
                                          (64, 256, 333, 3), (256, 512, 4800, 16), (1024, 256, 2400, 0),
-                                         (128, 512, 153600, 0), (4096, 1024, 2400, 0), (2048, 512, 9600, 0)])
+                                         (128, 512, 153600, 0), (4096, 1024, 2400, 0), (2048, 512, 9600, 0),
+                                         # the four weight gradients of a block at C = 192 (BN 64 and 256)
+                                         (192, 192, 600, 0), (384, 192, 600, 0), (768, 192, 600, 4), (192, 768, 600, 0)])
 def test_gemm_wgrad(M, N, K, split):
     """dW (M,N) += dY (K,M)^T @ X (K,N): both operands MN-major, split-K over tokens (partials + reduce)."""
     ops, L = _ops(), _L()
@@ -95,7 +101,8 @@ def test_gemm_wgrad(M, N, K, split):
 
 @pytest.mark.parametrize("M,N,K,kind", [(300, 128, 128, "fprop"), (1000, 256, 512, "fprop"), (257, 64, 192, "fprop"),
                                         (300, 128, 128, "dgrad"), (1000, 512, 128, "dgrad"), (90, 64, 1024, "dgrad"),
-                                        (128, 128, 1000, "wgrad"), (512, 128, 5000, "wgrad"), (64, 256, 333, "wgrad")])
+                                        (128, 128, 1000, "wgrad"), (512, 128, 5000, "wgrad"), (64, 256, 333, "wgrad"),
+                                        (600, 192, 192, "fprop"), (600, 320, 1280, "dgrad"), (192, 192, 600, "wgrad")])
 def test_gemm_split3_fp32_emulation(M, N, K, kind):
     """crf_gemm_args.split3 (the fp32 precision mode, csrc/crf_precise.cu): operands stored as [hi | lo] bf16 pairs, the
     product accumulates hi*hi + hi*lo + lo*hi in fp32.  Against a float64 product of the ORIGINAL fp32 matrices: rel
@@ -168,7 +175,11 @@ def test_gemm_bias_residual_with_k_splits(M, N, K):
 
 @pytest.mark.parametrize("M,N,K", [(2400, 4096, 1024), (2400, 1024, 4096), (2400, 1024, 1024), (2400, 2048, 1024),
                                    (9600, 512, 512), (9600, 2048, 512), (9600, 512, 2048), (9600, 1024, 512),
-                                   (1000, 512, 1024), (300, 1024, 2048)])
+                                   (1000, 512, 1024), (300, 1024, 2048),
+                                   # odd numbers of 256-wide column tiles (3 ... 15), the q-scale boundary inside a tile
+                                   # at 5 and 7 tiles, and several rounds of the 74 pairs at T = 9600
+                                   (2400, 768, 768), (2400, 1280, 640), (2400, 1792, 896), (9600, 2304, 576),
+                                   (2400, 3840, 960)])
 @pytest.mark.parametrize("kind", ["fprop", "dgrad"])
 def test_gemm_pair_epilogues(M, N, K, kind):
     """The CTA-pair GEMM (csrc/crf_gemm_pair.cu, 256 x 256 tiles on the two SMs of a TPC) with every epilogue the
@@ -209,16 +220,26 @@ def test_gemm_pair_epilogues(M, N, K, kind):
 
 
 def test_gemm_epilogues():
+    _check_epilogues(333, 256, 128)
+
+
+@pytest.mark.parametrize("M,N,K", [(333, 384, 192), (333, 640, 320),   # persistent kernel, q-scale boundary inside a tile
+                                   (333, 192, 192), (333, 320, 320)])  # gemm_kernel<64> with several column tiles
+def test_gemm_epilogues_inside_tiles(M, N, K):
+    _check_epilogues(M, N, K)
+
+
+def _check_epilogues(M, N, K):
+    """Every fprop epilogue against fp32 PyTorch, with the q scale on the first N / 2 columns."""
     ops, L = _ops(), _L()
-    M, N, K = 333, 256, 128
     A, W = _rand_bf16(M, K, seed=7), _rand_bf16(N, K, seed=8, scale=K ** -0.5)
     bias = torch.randn(N, device=DEV)
     acc = A.float() @ W.float().t()
-    # bf16 store with bias and a scale on the first 128 columns (the q half of the qk projection)
+    # bf16 store with bias and a scale on the first N / 2 columns (the q half of the qk projection)
     out = torch.zeros(M, N, dtype=torch.bfloat16, device=DEV)
-    ops.gemm(A, W, M, N, K, epilogue=L.EPI_STORE_BF16, out0=out, bias=bias, scale=0.25, scale_cols=128)
+    ops.gemm(A, W, M, N, K, epilogue=L.EPI_STORE_BF16, out0=out, bias=bias, scale=0.25, scale_cols=N // 2)
     ref = acc + bias
-    ref[:, :128] *= 0.25
+    ref[:, :N // 2] *= 0.25
     _check(out.float(), ref, 4e-3, "store_bf16")
     # bias + residual, fp32
     res = torch.randn(M, N, device=DEV)
@@ -360,7 +381,10 @@ def test_mlp_fused_fwd(T, C, training):
         _check(y, y_k, 1e-5, "mlp_fused.y vs unfused kernels")   # same products, different K-chunk summation order
 
 
-@pytest.mark.parametrize("C", [64, 128, 512, 1024])
+LN_WIDTHS = list(range(64, 1025, 64))   # every width the library accepts: one row-kernel instance each
+
+
+@pytest.mark.parametrize("C", LN_WIDTHS)
 @pytest.mark.parametrize("layout", ["nchw_view", "contig", "bf16_nchw"])
 def test_ln_fwd(C, layout):
     ops = _ops()
@@ -384,7 +408,7 @@ def test_ln_fwd(C, layout):
     _check(stats[:, 1], (xf.var(-1, unbiased=False) + 1e-5).rsqrt(), 1e-5, "ln_fwd.rstd")
 
 
-@pytest.mark.parametrize("C", [64, 128, 256, 512, 1024])
+@pytest.mark.parametrize("C", LN_WIDTHS)
 def test_ln_bwd(C):
     ops = _ops()
     T = 777
@@ -406,7 +430,7 @@ def test_ln_bwd(C):
     _check(dbeta, beta.grad, 1e-4, "ln_bwd.dbeta")
 
 
-@pytest.mark.parametrize("C", [64, 128, 256, 1024])
+@pytest.mark.parametrize("C", LN_WIDTHS)
 @pytest.mark.parametrize("out_bf16", [False, True])
 def test_layer_norm_standalone(C, out_bf16):
     """functional.layer_norm (the stage-closing norm_crf, newcrf_layers.py:430-431) vs torch's fp32 LayerNorm:
@@ -490,7 +514,8 @@ def test_depth_loss_matches_reference_golden():
                2e-4, f"depth_loss d pred ({tag})")
 
 
-@pytest.mark.parametrize("B,H,W,C", [(2, 5, 7, 64), (2, 15, 20, 1024), (8, 30, 40, 512), (3, 9, 11, 256), (1, 1, 1, 128)])
+@pytest.mark.parametrize("B,H,W,C", [(2, 5, 7, 64), (2, 15, 20, 1024), (8, 30, 40, 512), (3, 9, 11, 256), (1, 1, 1, 128),
+                                     (2, 9, 10, 192), (1, 15, 20, 320), (3, 7, 11, 640), (2, 5, 13, 960)])
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
 @pytest.mark.parametrize("aligned", [True, False])
 def test_layernorm_pixel_shuffle_fused(B, H, W, C, dtype, aligned):
@@ -565,8 +590,12 @@ def test_colsum_cast_convert():
     assert torch.equal(ops.cast_bf16(src), src.to(torch.bfloat16))
     v = torch.randn(2, 128, 9, 10, device=DEV).permute(0, 2, 3, 1)  # NCHW view, like newcrf_layers.py:427
     assert torch.equal(ops.convert_v(v), v.reshape(-1, 128).to(torch.bfloat16))
-    v2 = torch.randn(2, 9, 10, 64, device=DEV)
-    assert torch.equal(ops.convert_v(v2), v2.reshape(-1, 64).to(torch.bfloat16))
+    for Cv in (64, 192, 960):
+        v2 = torch.randn(2, 9, 10, Cv, device=DEV)
+        assert torch.equal(ops.convert_v(v2), v2.reshape(-1, Cv).to(torch.bfloat16)), Cv
+    for Cv in (192, 960):   # NCHW view: the transposing kernel, C / 256 not whole
+        v3 = torch.randn(2, Cv, 9, 10, device=DEV).permute(0, 2, 3, 1)
+        assert torch.equal(ops.convert_v(v3), v3.reshape(-1, Cv).to(torch.bfloat16)), Cv
     torch.cuda.synchronize()
 
 
@@ -630,7 +659,9 @@ def _attn_reference(qk, vb, qk_bias, table, B, H, W, C, nH, shift):
 
 ATTN_CASES = [(1, 7, 7, 64, 2, 0), (1, 14, 14, 64, 2, 0), (2, 9, 10, 64, 2, 0), (2, 9, 10, 64, 2, 3),
               (1, 15, 20, 128, 4, 3), (3, 30, 40, 128, 4, 3), (2, 15, 20, 256, 8, 0), (1, 21, 16, 1024, 32, 3),
-              (2, 9, 10, 64, 4, 3), (1, 15, 20, 128, 8, 0)]   # the last two: head_dim 16
+              (2, 9, 10, 64, 4, 3), (1, 15, 20, 128, 8, 0),   # these two: head_dim 16
+              # head counts that are not powers of two: head_dim 32 at C = 192 / 320, head_dim 16 at C = 192
+              (2, 9, 10, 192, 6, 3), (1, 15, 20, 320, 10, 3), (2, 9, 10, 192, 12, 3)]
 
 
 @pytest.mark.parametrize("B,H,W,C,nH,shift", ATTN_CASES)
@@ -651,7 +682,10 @@ def test_attn_fwd(B, H, W, C, nH, shift):
 
 # head_dim 64 / 128 (crf_attn_wide.cu; BASELINE.json configs[2])
 WIDE_CASES = [(1, 7, 7, 64, 1, 0), (2, 9, 10, 64, 1, 3), (1, 14, 14, 128, 2, 0), (1, 15, 20, 128, 1, 3),
-              (3, 30, 40, 256, 4, 3), (2, 15, 20, 256, 2, 0), (1, 21, 16, 512, 4, 3), (2, 23, 17, 512, 8, 3)]
+              (3, 30, 40, 256, 4, 3), (2, 15, 20, 256, 2, 0), (1, 21, 16, 512, 4, 3), (2, 23, 17, 512, 8, 3),
+              # odd head counts: head_dim 64 at C = 192 / 320 / 960, head_dim 128 at C = 384 / 640 / 896
+              (2, 9, 10, 192, 3, 3), (1, 15, 20, 320, 5, 3), (1, 15, 20, 960, 15, 3),
+              (2, 9, 10, 384, 3, 3), (1, 15, 20, 640, 5, 3), (1, 15, 20, 896, 7, 3)]
 
 
 @pytest.mark.parametrize("B,H,W,C,nH,shift", WIDE_CASES)
