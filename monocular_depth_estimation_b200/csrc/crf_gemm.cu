@@ -27,6 +27,7 @@
 #include <stdlib.h>
 
 #include "crf_gemm_epi.cuh"
+#include "crf_sched.h"
 
 namespace crf {
 
@@ -52,24 +53,20 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
   constexpr int kStageBytes = kATileBytes + kBTileBytes;
   // Bias gradient for free: one extra N=16 MMA per K step against an all-ones B tile puts sum_k A(m,k) into 16
   // spare TMEM columns (every column holds the same sum); needs the next power of two of TMEM columns.
-  const int kc_begin_ = blockIdx.z * chunks_per_split;
-  const int kc_end_ = min(total_chunks, kc_begin_ + chunks_per_split);
+  const int kc_begin = blockIdx.z * chunks_per_split;
+  const int kc_end = min(total_chunks, kc_begin + chunks_per_split);
   // split-operand mode: the column sums of A = hi + lo come from parts 0 (hi) and 2 (lo) only
-  const bool cs_any = chunks_per_part == 0 || kc_begin_ < chunks_per_part || kc_end_ > 2 * chunks_per_part;
+  const bool cs_any = chunks_per_part == 0 || kc_begin < chunks_per_part || kc_end > 2 * chunks_per_part;
   const bool do_colsum = ep.colsum != nullptr && blockIdx.y == 0 && cs_any;
   const uint32_t kTmemCols = ep.colsum != nullptr ? 2u * BN : (BN < 32 ? 32u : static_cast<uint32_t>(BN));
-  constexpr bool kOutF32 = (EPI == CRF_EPI_STORE_F32 || EPI == CRF_EPI_BIAS_RES_F32 || EPI == CRF_EPI_SPLITK_F32);
-  constexpr bool kHasAux = (EPI == CRF_EPI_BIAS_RES_F32 || EPI == CRF_EPI_MUL_DGELU);
-  constexpr bool kHasOut1 = (EPI == CRF_EPI_BIAS_GELU);
-  constexpr int kSlabCols = kOutF32 ? 32 : 64;
+  using TR = EpiTraits<EPI>;
+  constexpr int kSlabCols = TR::kSlabCols;
   constexpr int kNumSlabs = BN / kSlabCols;
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int m0 = blockIdx.x * BM;
   const int n0 = blockIdx.y * BN;
-  const int kc_begin = blockIdx.z * chunks_per_split;
-  const int kc_end = min(total_chunks, kc_begin + chunks_per_split);
   const int nk = kc_end - kc_begin;
   if (nk <= 0) return;  // uniform for the whole CTA
 
@@ -98,8 +95,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
     tma_prefetch_desc(&tmO0);
-    if (kHasOut1) tma_prefetch_desc(&tmO1);
-    if (kHasAux) tma_prefetch_desc(&tmAux);
+    if (TR::kHasOut1) tma_prefetch_desc(&tmO1);
+    if (TR::kHasAux) tma_prefetch_desc(&tmAux);
     for (int s = 0; s < stages; ++s) {
       mbar_init(full_bar(s), 1);
       mbar_init(empty_bar(s), 1);
@@ -189,7 +186,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     const bool tma_red = (EPI == CRF_EPI_SPLITK_F32) && ep.tma_reduce != 0;
     const int out_row0 = (EPI == CRF_EPI_SPLITK_F32 && !tma_red) ? static_cast<int>(blockIdx.z) * ep.m_pad + m0 : m0;
 
-    if (kHasAux && r == 0 && e < kNumSlabs) {
+    if (TR::kHasAux && r == 0 && e < kNumSlabs) {
       mbar_expect_tx(aux_bar(e), kSlabBytes);
       tma_load_2d(x_s + buf * kSlabBytes, &tmAux, aux_bar(e), n0 + e * kSlabCols, m0);
     }
@@ -198,7 +195,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
       const int nc = n0 + s * kSlabCols;
       if (r == 0) bulk_wait_read<0>();  // this group's previous store has drained its slab buffers
       named_bar_sync(1 + e, 128);
-      if (kHasAux) mbar_wait(aux_bar(e), it & 1);
+      if (TR::kHasAux) mbar_wait(aux_bar(e), it & 1);
       uint8_t* o0 = out0_g + buf * kSlabBytes;
       uint8_t* xb = x_g + buf * kSlabBytes;
 #pragma unroll
@@ -213,9 +210,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
       if (r == 0) {
         if (tma_red) tma_reduce_add_2d(&tmO0, out0_s + buf * kSlabBytes, nc, out_row0);
         else if (EPI != CRF_EPI_BIAS_GELU || ep.store_out0) tma_store_2d(&tmO0, out0_s + buf * kSlabBytes, nc, out_row0);
-        if (kHasOut1) tma_store_2d(&tmO1, x_s + buf * kSlabBytes, nc, out_row0);
+        if (TR::kHasOut1) tma_store_2d(&tmO1, x_s + buf * kSlabBytes, nc, out_row0);
         bulk_commit();
-        if (kHasAux && s + 2 < kNumSlabs) {  // the aux slab was consumed before the barrier above: refill it
+        if (TR::kHasAux && s + 2 < kNumSlabs) {  // the aux slab was consumed before the barrier above: refill it
           mbar_expect_tx(aux_bar(e), kSlabBytes);
           tma_load_2d(x_s + buf * kSlabBytes, &tmAux, aux_bar(e), nc + 2 * kSlabCols, m0);
         }
@@ -259,14 +256,13 @@ splitk_reduce_kernel(const float* __restrict__ part, float* __restrict__ out, in
 }
 
 struct Launch {
-  CUtensorMap tmA, tmB, tmO0, tmO1, tmAux;
   int total_chunks, cps, splits, m_pad;
   int tma_reduce = 0;
   int chunks_per_part = 0, a_off = 0, b_off = 0;  // split-operand mode
 };
 
 template <int BN, int EPI>
-int launch_one(const Launch& L, const crf_gemm_args& a, cudaStream_t st) {
+int launch_one(const GemmMaps& m, const Launch& L, const crf_gemm_args& a, cudaStream_t st) {
   constexpr int kStageBytes = kATileBytes + BN * 128;
   // 2 co-resident CTAs/SM when K is short; one deep ring when K is long.
   // wgrad: one CTA per SM streams a long token range -> deep ring.  fprop/dgrad: these are epilogue-bound (GELU,
@@ -279,50 +275,61 @@ int launch_one(const Launch& L, const crf_gemm_args& a, cudaStream_t st) {
   const size_t smem = ring + 1024 + 8 * (2 * stages + 4) + 1024;  // + align slack, barriers, ones tile
   auto kern = gemm_kernel<BN, EPI>;
   CRF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  EpiParams ep{a.bias, a.scale, a.scale_cols, L.m_pad, a.out0 != nullptr ? 1 : 0, a.a_major == 1 ? a.colsum : nullptr,
-               L.tma_reduce};
+  const EpiParams ep = epi_params(a, L.m_pad, L.tma_reduce);
   dim3 grid((a.M + BM - 1) / BM, a.N / BN, L.splits);
-  const double mn = static_cast<double>(a.M) * a.N;
-  const double out_bytes = EPI == CRF_EPI_STORE_BF16 ? 2 * mn
-                           : EPI == CRF_EPI_BIAS_RES_F32 ? 8 * mn
-                           : EPI == CRF_EPI_BIAS_GELU ? (a.out0 != nullptr ? 4 * mn : 2 * mn)
-                           : 4 * mn;
-  KernelTimer tm(st, 2.0 * mn * a.K, (a.split3 ? 2.0 : 1.0) * 2.0 * (static_cast<double>(a.M) + a.N) * a.K + out_bytes,
-                 "gemm%s_%s_epi%d_M%d_N%d_K%d", a.split3 ? "3" : "", a.a_major ? "wgrad" : (a.b_major ? "dgrad" : "fprop"), EPI,
-                 a.M, a.N, a.K);
-  launch_pdl(kern, grid, kThreads, smem, st, L.tmA, L.tmB, L.tmO0, L.tmO1, L.tmAux, a.M, a.N, L.total_chunks, L.cps, stages,
-                                     a.a_major, a.b_major, ep, L.chunks_per_part, L.a_off, L.b_off);
+  KernelTimer tm(st, 2.0 * a.M * a.N * a.K, gemm_bytes(a, EPI), "gemm%s_%s_epi%d_M%d_N%d_K%d", a.split3 ? "3" : "",
+                 a.a_major ? "wgrad" : (a.b_major ? "dgrad" : "fprop"), EPI, a.M, a.N, a.K);
+  launch_pdl(kern, grid, kThreads, smem, st, m.tmA, m.tmB, m.tmO0, m.tmO1, m.tmAux, a.M, a.N, L.total_chunks, L.cps, stages,
+             a.a_major, a.b_major, ep, L.chunks_per_part, L.a_off, L.b_off);
   CRF_CUDA(cudaGetLastError());
   note_launch();
   return 0;
 }
 
-template <int BN>
-int launch_bn(const Launch& L, const crf_gemm_args& a, int epi, cudaStream_t st) {
-  switch (epi) {
-    case CRF_EPI_STORE_F32: return launch_one<BN, CRF_EPI_STORE_F32>(L, a, st);
-    case CRF_EPI_STORE_BF16: return launch_one<BN, CRF_EPI_STORE_BF16>(L, a, st);
-    case CRF_EPI_BIAS_RES_F32: return launch_one<BN, CRF_EPI_BIAS_RES_F32>(L, a, st);
-    case CRF_EPI_BIAS_GELU: return launch_one<BN, CRF_EPI_BIAS_GELU>(L, a, st);
-    case CRF_EPI_MUL_DGELU: return launch_one<BN, CRF_EPI_MUL_DGELU>(L, a, st);
-    case CRF_EPI_SPLITK_F32: return launch_one<BN, CRF_EPI_SPLITK_F32>(L, a, st);
-    default: return set_error("crf_gemm: unknown epilogue %d", epi);
-  }
-}
-
-int launch_bn_dispatch(int BN, const Launch& L, const crf_gemm_args& a, int epi, cudaStream_t st) {
-  switch (BN) {
-    case 256: return launch_bn<256>(L, a, epi, st);
-    case 128: return launch_bn<128>(L, a, epi, st);
-    default: return launch_bn<64>(L, a, epi, st);
-  }
+int launch_tiled(int BN, const GemmMaps& m, const Launch& L, const crf_gemm_args& a, int epi, cudaStream_t st) {
+  return with_epi(epi, [&](auto e) {
+    constexpr int EPI = decltype(e)::value;
+    switch (BN) {
+      case 256: return launch_one<256, EPI>(m, L, a, st);
+      case 128: return launch_one<128, EPI>(m, L, a, st);
+      default: return launch_one<64, EPI>(m, L, a, st);
+    }
+  });
 }
 
 }  // namespace
 
-// Number of K splits a weight-gradient GEMM will use and the fp32 partial-tile workspace it needs.
+int gemm_maps(const crf_gemm_args& a, uint32_t b_rows, GemmMaps* m) {
+  const uint64_t dup = a.split3 ? 2 : 1;  // split-operand matrices are twice as wide: [hi | lo]
+  if (a.a_major == 0 ? make_tmap_bf16(&m->tmA, a.A, a.M, dup * a.K, BM) : make_tmap_bf16(&m->tmA, a.A, a.K, dup * a.M, 64))
+    return 1;
+  if (a.b_major == 0 ? make_tmap_bf16(&m->tmB, a.B, a.N, dup * a.K, b_rows) : make_tmap_bf16(&m->tmB, a.B, a.K, dup * a.N, 64))
+    return 1;
+  m->tmO0 = m->tmO1 = m->tmAux = m->tmA;
+  const int epi = a.epilogue;
+  if (epi == CRF_EPI_BIAS_GELU) {
+    CRF_CHECK(a.out1 != nullptr, "crf_gemm: BIAS_GELU needs out1");
+    if (a.out0 != nullptr && make_tmap_bf16(&m->tmO0, a.out0, a.M, a.N, BM)) return 1;
+    if (make_tmap_bf16(&m->tmO1, a.out1, a.M, a.N, BM)) return 1;
+  } else {
+    CRF_CHECK(a.out0 != nullptr, "crf_gemm: out0 is null");
+    const bool out_f32 = epi == CRF_EPI_STORE_F32 || epi == CRF_EPI_BIAS_RES_F32 || epi == CRF_EPI_SPLITK_F32;
+    if (out_f32 ? make_tmap_f32(&m->tmO0, a.out0, a.M, a.N, BM) : make_tmap_bf16(&m->tmO0, a.out0, a.M, a.N, BM)) return 1;
+  }
+  if (epi == CRF_EPI_BIAS_RES_F32) {
+    CRF_CHECK(a.aux1 != nullptr, "crf_gemm: BIAS_RES_F32 needs aux1 (residual)");
+    if (make_tmap_f32(&m->tmAux, a.aux1, a.M, a.N, BM)) return 1;
+  } else if (epi == CRF_EPI_MUL_DGELU) {
+    CRF_CHECK(a.aux1 != nullptr, "crf_gemm: MUL_DGELU needs aux1 (pre-activation)");
+    if (make_tmap_bf16(&m->tmAux, a.aux1, a.M, a.N, BM)) return 1;
+  }
+  return 0;
+}
+
+// Number of K splits a weight-gradient GEMM will use and the fp32 partial-tile workspace it needs.  The tile width is
+// gemm_tile_n(N) without the cap plan_gemm applies to K-major A: the split-K GEMMs of the library have MN-major A.
 size_t gemm_splitk_workspace_bytes(int M, int N, int K, int device, int* splits_out) {
-  const int BN = (N % 256 == 0) ? 256 : (N % 128 == 0 ? 128 : 64);
+  const int BN = gemm_tile_n(N);
   const int tiles = ((M + BM - 1) / BM) * (N / BN);
   const int chunks = (K + BK - 1) / BK;
   int s = num_sms(device) / tiles;  // about one CTA per SM, each with a deep pipeline over its token range
@@ -342,17 +349,6 @@ int launch_gemm(const crf_gemm_args& a, cudaStream_t st) {
   CRF_CHECK(a.a_major == 1 || a.K % 8 == 0, "crf_gemm: K-major A needs K %% 8 == 0 (K=%d)", a.K);
   CRF_CHECK(a.a_major == 0 || a.M % 8 == 0, "crf_gemm: MN-major A needs M %% 8 == 0 (M=%d)", a.M);
   CRF_CHECK(a.ld_out == a.N, "crf_gemm: outputs must be dense (ld_out == N)");
-  if (!a.split3) {  // token-major projections: CTA-pair kernel, else the persistent kernel where the shape is eligible
-    const int rc2 = launch_gemm_pair(a, st);
-    if (rc2 >= 0) return rc2;
-    const int rc = launch_gemm_persistent(a, st);
-    if (rc >= 0) return rc;
-  }
-  int BN = (a.N % 256 == 0) ? 256 : (a.N % 128 == 0 ? 128 : 64);
-  if (a.a_major == 0 && BN > 128) BN = 128;
-
-  Launch L{};
-  const int dup = a.split3 ? 2 : 1;  // split-operand matrices are twice as wide: [hi | lo]
   if (a.split3) {
     CRF_CHECK((a.a_major == 1 || a.K % BK == 0) && (a.b_major == 1 || a.K % BK == 0),
               "crf_gemm: split3 with a K-major operand needs K %% 64 == 0 (K=%d)", a.K);
@@ -360,16 +356,14 @@ int launch_gemm(const crf_gemm_args& a, cudaStream_t st) {
     CRF_CHECK(a.epilogue == CRF_EPI_STORE_F32 || a.epilogue == CRF_EPI_BIAS_RES_F32 || a.epilogue == CRF_EPI_SPLITK_F32,
               "crf_gemm: split3 supports the fp32 epilogues only");
   }
-  if (a.a_major == 0) {
-    if (make_tmap_bf16(&L.tmA, a.A, a.M, static_cast<uint64_t>(dup) * a.K, BM)) return 1;
-  } else {
-    if (make_tmap_bf16(&L.tmA, a.A, a.K, static_cast<uint64_t>(dup) * a.M, 64)) return 1;
-  }
-  if (a.b_major == 0) {
-    if (make_tmap_bf16(&L.tmB, a.B, a.N, static_cast<uint64_t>(dup) * a.K, BN)) return 1;
-  } else {
-    if (make_tmap_bf16(&L.tmB, a.B, a.K, static_cast<uint64_t>(dup) * a.N, 64)) return 1;
-  }
+  const GemmPlan plan = plan_gemm(a.M, a.N, a.K, a.a_major, a.epilogue, a.split3);
+  GemmMaps m;
+  // the pair and persistent kernels load 128 rows of B per CTA and K step
+  if (gemm_maps(a, plan.kernel == kGemmTiled ? plan.bn : 128, &m)) return 1;
+  if (plan.kernel == kGemmPair) return launch_gemm_pair(a, m, st);
+  if (plan.kernel == kGemmPersistent) return launch_gemm_persistent(a, m, st);
+
+  Launch L{};
   L.total_chunks = (a.K + BK - 1) / BK;
   if (a.split3) {
     L.chunks_per_part = L.total_chunks;
@@ -380,13 +374,10 @@ int launch_gemm(const crf_gemm_args& a, cudaStream_t st) {
   L.splits = 1;
   L.cps = L.total_chunks;
   L.m_pad = (a.M + BM - 1) / BM * BM;
-  L.tmO1 = L.tmA;  // placeholders for unused maps (never dereferenced by the kernel)
-  L.tmAux = L.tmA;
-  int epi = a.epilogue;
+  const int epi = a.epilogue;
 
   if (epi == CRF_EPI_SPLITK_F32) {
     // out0 (M,N) f32 += A^T B.  One split: in-place accumulate (residual = out0).  Otherwise partials + reduce.
-    CRF_CHECK(a.out0 != nullptr, "crf_gemm: out0 is null");
     int splits = 1;
     gemm_splitk_workspace_bytes(a.M, a.N, a.split3 ? 3 * a.K : a.K, a.device, &splits);
     if (a.split_k > 0 && a.split_k < splits) splits = a.split_k;
@@ -399,9 +390,8 @@ int launch_gemm(const crf_gemm_args& a, cudaStream_t st) {
     crf_gemm_args b = a;
     b.bias = nullptr;
     if (splits <= 1) {
-      if (make_tmap_f32(&L.tmO0, a.out0, a.M, a.N, BM)) return 1;
-      L.tmAux = L.tmO0;
-      return launch_bn_dispatch(BN, L, b, CRF_EPI_BIAS_RES_F32, st);
+      m.tmAux = m.tmO0;
+      return launch_tiled(plan.bn, m, L, b, CRF_EPI_BIAS_RES_F32, st);
     }
     L.cps = (L.total_chunks + splits - 1) / splits;
     L.splits = (L.total_chunks + L.cps - 1) / L.cps;  // no empty split
@@ -410,11 +400,10 @@ int launch_gemm(const crf_gemm_args& a, cudaStream_t st) {
     // depends on it).  CRF_WGRAD_DETERMINISTIC=1 keeps the partial tiles + fixed-order reduce kernel.
     if (!deterministic) {
       L.tma_reduce = 1;
-      if (make_tmap_f32(&L.tmO0, a.out0, a.M, a.N, BM)) return 1;
-      return launch_bn_dispatch(BN, L, b, epi, st);
+      return launch_tiled(plan.bn, m, L, b, epi, st);
     }
-    if (make_tmap_f32(&L.tmO0, a.workspace, static_cast<uint64_t>(L.splits) * L.m_pad, a.N, BM)) return 1;
-    if (launch_bn_dispatch(BN, L, b, epi, st)) return 1;
+    if (make_tmap_f32(&m.tmO0, a.workspace, static_cast<uint64_t>(L.splits) * L.m_pad, a.N, BM)) return 1;
+    if (launch_tiled(plan.bn, m, L, b, epi, st)) return 1;
     const int64_t total4 = static_cast<int64_t>(a.M) * a.N / 4;
     KernelTimer tm(st, 0.0, 4.0 * a.M * a.N * (L.splits + 2), "splitk_reduce_M%d_N%d_S%d", a.M, a.N, L.splits);
     launch_pdl(splitk_reduce_kernel, static_cast<unsigned>((total4 + 255) / 256), 256, 0, st, 
@@ -423,29 +412,7 @@ int launch_gemm(const crf_gemm_args& a, cudaStream_t st) {
     note_launch();
     return 0;
   }
-
-  const bool out_f32 = (epi == CRF_EPI_STORE_F32 || epi == CRF_EPI_BIAS_RES_F32);
-  if (epi == CRF_EPI_BIAS_GELU) {
-    CRF_CHECK(a.out1 != nullptr, "crf_gemm: BIAS_GELU needs out1");
-    if (a.out0 != nullptr) {
-      if (make_tmap_bf16(&L.tmO0, a.out0, a.M, a.N, BM)) return 1;
-    } else {
-      L.tmO0 = L.tmA;
-    }
-    if (make_tmap_bf16(&L.tmO1, a.out1, a.M, a.N, BM)) return 1;
-  } else {
-    CRF_CHECK(a.out0 != nullptr, "crf_gemm: out0 is null");
-    if (out_f32 ? make_tmap_f32(&L.tmO0, a.out0, a.M, a.N, BM) : make_tmap_bf16(&L.tmO0, a.out0, a.M, a.N, BM))
-      return 1;
-  }
-  if (epi == CRF_EPI_BIAS_RES_F32) {
-    CRF_CHECK(a.aux1 != nullptr, "crf_gemm: BIAS_RES_F32 needs aux1 (residual)");
-    if (make_tmap_f32(&L.tmAux, a.aux1, a.M, a.N, BM)) return 1;
-  } else if (epi == CRF_EPI_MUL_DGELU) {
-    CRF_CHECK(a.aux1 != nullptr, "crf_gemm: MUL_DGELU needs aux1 (pre-activation)");
-    if (make_tmap_bf16(&L.tmAux, a.aux1, a.M, a.N, BM)) return 1;
-  }
-  return launch_bn_dispatch(BN, L, a, epi, st);
+  return launch_tiled(plan.bn, m, L, a, epi, st);
 }
 
 }  // namespace crf

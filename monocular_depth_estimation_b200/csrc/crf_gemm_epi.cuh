@@ -1,6 +1,8 @@
 // Epilogue building blocks shared by the GEMM kernels: per-thread processing of 32 accumulator columns of one row
 // (bias, scale, residual, exact-erf GELU, GELU derivative) and the swizzled slab stores that feed the TMA stores.
 #pragma once
+#include <type_traits>
+
 #include "crf_host.h"
 #include "crf_ptx.cuh"
 
@@ -89,5 +91,44 @@ struct EpiTraits {
   static constexpr bool kHasOut1 = (EPI == CRF_EPI_BIAS_GELU);
   static constexpr int kSlabCols = kOutF32 ? 32 : 64;
 };
+
+// Calls f(std::integral_constant<int, EPI>()) for a GEMM epilogue (the kernels are instantiated per epilogue) and
+// returns its result.
+template <typename F>
+int with_epi(int epi, F&& f) {
+  switch (epi) {
+    case CRF_EPI_STORE_F32: return f(std::integral_constant<int, CRF_EPI_STORE_F32>());
+    case CRF_EPI_STORE_BF16: return f(std::integral_constant<int, CRF_EPI_STORE_BF16>());
+    case CRF_EPI_BIAS_RES_F32: return f(std::integral_constant<int, CRF_EPI_BIAS_RES_F32>());
+    case CRF_EPI_BIAS_GELU: return f(std::integral_constant<int, CRF_EPI_BIAS_GELU>());
+    case CRF_EPI_MUL_DGELU: return f(std::integral_constant<int, CRF_EPI_MUL_DGELU>());
+    case CRF_EPI_SPLITK_F32: return f(std::integral_constant<int, CRF_EPI_SPLITK_F32>());
+    default: return set_error("crf_gemm: unknown epilogue %d", epi);
+  }
+}
+
+// m_pad and tma_reduce: the tiled kernel's split-K (0 for the other kernels and epilogues)
+inline EpiParams epi_params(const crf_gemm_args& a, int m_pad, int tma_reduce) {
+  EpiParams ep;
+  ep.bias = a.bias;
+  ep.scale = a.scale;
+  ep.scale_cols = a.scale_cols;
+  ep.m_pad = m_pad;
+  ep.store_out0 = a.out0 != nullptr ? 1 : 0;
+  ep.colsum = a.a_major == 1 ? a.colsum : nullptr;
+  ep.tma_reduce = tma_reduce;
+  return ep;
+}
+
+// Algorithmic HBM bytes of a GEMM with epilogue epi (KernelTimer): both operands once (twice as wide with split3), the
+// outputs once, the aux input once.
+inline double gemm_bytes(const crf_gemm_args& a, int epi) {
+  const double mn = static_cast<double>(a.M) * a.N;
+  const double out_bytes = epi == CRF_EPI_STORE_BF16 ? 2 * mn
+                           : epi == CRF_EPI_BIAS_RES_F32 ? 8 * mn
+                           : epi == CRF_EPI_BIAS_GELU ? (a.out0 != nullptr ? 4 * mn : 2 * mn)
+                           : 4 * mn;
+  return (a.split3 ? 2.0 : 1.0) * 2.0 * (static_cast<double>(a.M) + a.N) * a.K + out_bytes;
+}
 
 }  // namespace crf

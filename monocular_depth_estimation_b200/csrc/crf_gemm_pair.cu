@@ -206,87 +206,30 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 }
 
 template <int EPI>
-int launch_pair(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmO0, const CUtensorMap& tmO1,
-                const CUtensorMap& tmAux, const crf_gemm_args& a, cudaStream_t st) {
+int launch_pair(const GemmMaps& m, const crf_gemm_args& a, cudaStream_t st) {
   auto kern = gemm_pair_kernel<EPI>;
   CRF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
   const int tiles = ((a.M + PM - 1) / PM) * (a.N / PN);
   const int max_pairs = num_sms(a.device) / 2;
   int pairs = max_pairs;
   if (pairs > tiles) pairs = tiles;
-  EpiParams ep{a.bias, a.scale, a.scale_cols, 0, a.out0 != nullptr ? 1 : 0, nullptr, 0};
-  const double mn = static_cast<double>(a.M) * a.N;
-  const double out_bytes = EPI == CRF_EPI_STORE_BF16 ? 2 * mn
-                           : EPI == CRF_EPI_BIAS_RES_F32 ? 8 * mn
-                           : EPI == CRF_EPI_BIAS_GELU ? (a.out0 != nullptr ? 4 * mn : 2 * mn)
-                           : 4 * mn;
-  KernelTimer tm(st, 2.0 * mn * a.K, 2.0 * (static_cast<double>(a.M) + a.N) * a.K + out_bytes,
-                 "gemm2_%s_epi%d_M%d_N%d_K%d", a.b_major ? "dgrad" : "fprop", EPI, a.M, a.N, a.K);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(2 * pairs);
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // see launch_pdl (crf_host.h)
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  CRF_CUDA(cudaLaunchKernelEx(&cfg, kern, tmA, tmB, tmO0, tmO1, tmAux, a.M, a.N, a.K, a.b_major, ep));
+  KernelTimer tm(st, 2.0 * a.M * a.N * a.K, gemm_bytes(a, EPI), "gemm2_%s_epi%d_M%d_N%d_K%d",
+                 a.b_major ? "dgrad" : "fprop", EPI, a.M, a.N, a.K);
+  CRF_CUDA(launch_pdl_cluster(2, kern, 2 * pairs, kThreads, kSmemBytes, st, m.tmA, m.tmB, m.tmO0, m.tmO1, m.tmAux, a.M, a.N,
+                              a.K, a.b_major, epi_params(a, 0, 0)));
   note_launch();
   return 0;
 }
 
 }  // namespace
 
-// fprop / dgrad (A K-major) with N a multiple of 256 and enough work for CTA pairs.  Returns -1 if not eligible.
-int launch_gemm_pair(const crf_gemm_args& a, cudaStream_t st) {
-  // verified (tests/test_gpu_stages.py, block parity) and measured on B200: 15-30 % faster than the single-CTA kernel on
-  // every C >= 512 projection (profiles/r02_gemm_pair.md)
-  if (a.a_major != 0 || a.N % PN != 0 || a.epilogue == CRF_EPI_SPLITK_F32 || a.split3) return -1;
-  if (a.K < 512 || a.N < 512) return -1;
-  CUtensorMap tmA, tmB, tmO0, tmO1, tmAux;
-  if (make_tmap_bf16(&tmA, a.A, a.M, a.K, 128)) return 1;
-  if (a.b_major == 0) {
-    if (make_tmap_bf16(&tmB, a.B, a.N, a.K, 128)) return 1;
-  } else {
-    if (make_tmap_bf16(&tmB, a.B, a.K, a.N, 64)) return 1;
-  }
-  tmO1 = tmA;
-  tmAux = tmA;
-  const int epi = a.epilogue;
-  const bool out_f32 = (epi == CRF_EPI_STORE_F32 || epi == CRF_EPI_BIAS_RES_F32);
-  if (epi == CRF_EPI_BIAS_GELU) {
-    CRF_CHECK(a.out1 != nullptr, "crf_gemm: BIAS_GELU needs out1");
-    if (a.out0 != nullptr) {
-      if (make_tmap_bf16(&tmO0, a.out0, a.M, a.N, 128)) return 1;
-    } else {
-      tmO0 = tmA;
-    }
-    if (make_tmap_bf16(&tmO1, a.out1, a.M, a.N, 128)) return 1;
-  } else {
-    CRF_CHECK(a.out0 != nullptr, "crf_gemm: out0 is null");
-    if (out_f32 ? make_tmap_f32(&tmO0, a.out0, a.M, a.N, 128) : make_tmap_bf16(&tmO0, a.out0, a.M, a.N, 128)) return 1;
-  }
-  if (epi == CRF_EPI_BIAS_RES_F32) {
-    CRF_CHECK(a.aux1 != nullptr, "crf_gemm: BIAS_RES_F32 needs aux1 (residual)");
-    if (make_tmap_f32(&tmAux, a.aux1, a.M, a.N, 128)) return 1;
-  } else if (epi == CRF_EPI_MUL_DGELU) {
-    CRF_CHECK(a.aux1 != nullptr, "crf_gemm: MUL_DGELU needs aux1 (pre-activation)");
-    if (make_tmap_bf16(&tmAux, a.aux1, a.M, a.N, 128)) return 1;
-  }
-  switch (epi) {
-    case CRF_EPI_STORE_F32: return launch_pair<CRF_EPI_STORE_F32>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    case CRF_EPI_STORE_BF16: return launch_pair<CRF_EPI_STORE_BF16>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    case CRF_EPI_BIAS_RES_F32: return launch_pair<CRF_EPI_BIAS_RES_F32>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    case CRF_EPI_BIAS_GELU: return launch_pair<CRF_EPI_BIAS_GELU>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    case CRF_EPI_MUL_DGELU: return launch_pair<CRF_EPI_MUL_DGELU>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    default: return set_error("crf_gemm: unknown epilogue %d", epi);
-  }
+// fprop / dgrad (A K-major) with N a multiple of 256 and enough work for CTA pairs (plan_gemm, crf_sched.h).
+int launch_gemm_pair(const crf_gemm_args& a, const GemmMaps& m, cudaStream_t st) {
+  return with_epi(a.epilogue, [&](auto e) {
+    constexpr int EPI = decltype(e)::value;
+    if constexpr (EPI == CRF_EPI_SPLITK_F32) return set_error("crf_gemm: the CTA-pair kernel has no split-K epilogue");
+    else return launch_pair<EPI>(m, a, st);
+  });
 }
 
 }  // namespace crf

@@ -233,8 +233,7 @@ gemm_persistent_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_con
 }
 
 template <int EPI>
-int launch_p(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmO0, const CUtensorMap& tmO1,
-             const CUtensorMap& tmAux, const crf_gemm_args& a, cudaStream_t st) {
+int launch_p(const GemmMaps& m, const crf_gemm_args& a, cudaStream_t st) {
   auto kern = gemm_persistent_kernel<EPI>;
   constexpr int kSmemBytes = Plan<EPI>::kSmemBytes;
   CRF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
@@ -253,15 +252,10 @@ int launch_p(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& 
   if (splits > 1) CRF_CUDA(cudaMemsetAsync(a.out0, 0, static_cast<size_t>(a.M) * a.N * sizeof(float), st));
   int grid = sms;
   if (grid > tiles * splits) grid = tiles * splits;
-  EpiParams ep{a.bias, a.scale, a.scale_cols, 0, a.out0 != nullptr ? 1 : 0, nullptr};
-  const double mn = static_cast<double>(a.M) * a.N;
-  const double out_bytes = EPI == CRF_EPI_STORE_BF16 ? 2 * mn
-                           : EPI == CRF_EPI_BIAS_RES_F32 ? 8 * mn
-                           : EPI == CRF_EPI_BIAS_GELU ? (a.out0 != nullptr ? 4 * mn : 2 * mn)
-                           : 4 * mn;
-  KernelTimer tm(st, 2.0 * mn * a.K, 2.0 * (static_cast<double>(a.M) + a.N) * a.K + out_bytes,
-                 "gemm_%s_epi%d_M%d_N%d_K%d", a.b_major ? "dgrad" : "fprop", EPI, a.M, a.N, a.K);
-  launch_pdl(kern, grid, kThreads, kSmemBytes, st, tmA, tmB, tmO0, tmO1, tmAux, a.M, a.N, a.K, a.b_major, ep, splits);
+  KernelTimer tm(st, 2.0 * a.M * a.N * a.K, gemm_bytes(a, EPI), "gemm_%s_epi%d_M%d_N%d_K%d",
+                 a.b_major ? "dgrad" : "fprop", EPI, a.M, a.N, a.K);
+  launch_pdl(kern, grid, kThreads, kSmemBytes, st, m.tmA, m.tmB, m.tmO0, m.tmO1, m.tmAux, a.M, a.N, a.K, a.b_major,
+             epi_params(a, 0, 0), splits);
   CRF_CUDA(cudaGetLastError());
   note_launch();
   return 0;
@@ -269,47 +263,13 @@ int launch_p(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& 
 
 }  // namespace
 
-// fprop / dgrad (A K-major), N a multiple of 128, no split-K.  Returns -1 if the shape is not eligible.
-int launch_gemm_persistent(const crf_gemm_args& a, cudaStream_t st) {
-  if (a.a_major != 0 || a.N % BN != 0 || a.epilogue == CRF_EPI_SPLITK_F32) return -1;
-  CUtensorMap tmA, tmB, tmO0, tmO1, tmAux;
-  if (make_tmap_bf16(&tmA, a.A, a.M, a.K, BM)) return 1;
-  if (a.b_major == 0) {
-    if (make_tmap_bf16(&tmB, a.B, a.N, a.K, BN)) return 1;
-  } else {
-    if (make_tmap_bf16(&tmB, a.B, a.K, a.N, 64)) return 1;
-  }
-  tmO1 = tmA;
-  tmAux = tmA;
-  const int epi = a.epilogue;
-  const bool out_f32 = (epi == CRF_EPI_STORE_F32 || epi == CRF_EPI_BIAS_RES_F32);
-  if (epi == CRF_EPI_BIAS_GELU) {
-    CRF_CHECK(a.out1 != nullptr, "crf_gemm: BIAS_GELU needs out1");
-    if (a.out0 != nullptr) {
-      if (make_tmap_bf16(&tmO0, a.out0, a.M, a.N, BM)) return 1;
-    } else {
-      tmO0 = tmA;
-    }
-    if (make_tmap_bf16(&tmO1, a.out1, a.M, a.N, BM)) return 1;
-  } else {
-    CRF_CHECK(a.out0 != nullptr, "crf_gemm: out0 is null");
-    if (out_f32 ? make_tmap_f32(&tmO0, a.out0, a.M, a.N, BM) : make_tmap_bf16(&tmO0, a.out0, a.M, a.N, BM)) return 1;
-  }
-  if (epi == CRF_EPI_BIAS_RES_F32) {
-    CRF_CHECK(a.aux1 != nullptr, "crf_gemm: BIAS_RES_F32 needs aux1 (residual)");
-    if (make_tmap_f32(&tmAux, a.aux1, a.M, a.N, BM)) return 1;
-  } else if (epi == CRF_EPI_MUL_DGELU) {
-    CRF_CHECK(a.aux1 != nullptr, "crf_gemm: MUL_DGELU needs aux1 (pre-activation)");
-    if (make_tmap_bf16(&tmAux, a.aux1, a.M, a.N, BM)) return 1;
-  }
-  switch (epi) {
-    case CRF_EPI_STORE_F32: return launch_p<CRF_EPI_STORE_F32>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    case CRF_EPI_STORE_BF16: return launch_p<CRF_EPI_STORE_BF16>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    case CRF_EPI_BIAS_RES_F32: return launch_p<CRF_EPI_BIAS_RES_F32>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    case CRF_EPI_BIAS_GELU: return launch_p<CRF_EPI_BIAS_GELU>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    case CRF_EPI_MUL_DGELU: return launch_p<CRF_EPI_MUL_DGELU>(tmA, tmB, tmO0, tmO1, tmAux, a, st);
-    default: return set_error("crf_gemm: unknown epilogue %d", epi);
-  }
+// fprop / dgrad (A K-major), N a multiple of 128, no split-K (plan_gemm, crf_sched.h).
+int launch_gemm_persistent(const crf_gemm_args& a, const GemmMaps& m, cudaStream_t st) {
+  return with_epi(a.epilogue, [&](auto e) {
+    constexpr int EPI = decltype(e)::value;
+    if constexpr (EPI == CRF_EPI_SPLITK_F32) return set_error("crf_gemm: the persistent kernel has no split-K epilogue");
+    else return launch_p<EPI>(m, a, st);
+  });
 }
 
 }  // namespace crf

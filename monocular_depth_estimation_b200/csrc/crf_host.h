@@ -70,26 +70,52 @@ long long launch_count();
 
 // Kernel launch with the programmatic-stream-serialization attribute (PDL): the kernel may be scheduled while the
 // previous kernel of the stream is still draining; every kernel launched through here begins with pdl_prologue()
-// (crf_ptx.cuh), which waits for the previous grid before anything else runs.
+// (crf_ptx.cuh), which waits for the previous grid before anything else runs.  cluster_x > 1 launches clusters of
+// that many CTAs along x.
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+inline cudaError_t launch_pdl_cluster(unsigned cluster_x, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
+                                      cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchAttribute attr[2];
+  int n = 0;
+  if (cluster_x > 1) {
+    attr[n].id = cudaLaunchAttributeClusterDimension;
+    attr[n].val.clusterDim.x = cluster_x;
+    attr[n].val.clusterDim.y = 1;
+    attr[n].val.clusterDim.z = 1;
+    ++n;
+  }
+  attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[n].val.programmaticStreamSerializationAllowed = 1;
+  ++n;
   cfg.attrs = attr;
-  cfg.numAttrs = 1;
+  cfg.numAttrs = n;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+}
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+  return launch_pdl_cluster(1, kern, grid, block, smem, st, static_cast<Args&&>(args)...);
 }
 
 // ---- internal launchers (stream-ordered, no allocation) ----
+// launch_gemm validates the arguments, picks the kernel with plan_gemm (crf_sched.h), builds the tensor maps with
+// gemm_maps and launches the CTA-pair kernel (crf_gemm_pair.cu), the persistent kernel (crf_gemm_persist.cu) or the
+// tiled kernel (crf_gemm.cu).
 int launch_gemm(const crf_gemm_args& a, cudaStream_t st);
-int launch_gemm_persistent(const crf_gemm_args& a, cudaStream_t st);  // -1: shape not eligible
-int launch_gemm_pair(const crf_gemm_args& a, cudaStream_t st);        // cta_group::2 tiles (crf_gemm_pair.cu); -1: not eligible
+// TMA maps of one GEMM, in the kernels' parameter order.  Maps an epilogue does not use are copies of tmA (never read).
+struct GemmMaps {
+  CUtensorMap tmA, tmB, tmO0, tmO1, tmAux;
+};
+// Checks that the epilogue has its outputs and aux input and builds the maps: a K-major operand in boxes of 128 rows (A)
+// or b_rows rows (B), an MN-major one in boxes of 64 K-rows, both twice as wide with split3; outputs and aux in boxes
+// of 128 rows.
+int gemm_maps(const crf_gemm_args& a, uint32_t b_rows, GemmMaps* m);
+int launch_gemm_pair(const crf_gemm_args& a, const GemmMaps& m, cudaStream_t st);
+int launch_gemm_persistent(const crf_gemm_args& a, const GemmMaps& m, cudaStream_t st);
 // crf_precise.cu: the fp32 precision mode (crf_block_desc.precision == CRF_PREC_FP32)
 size_t precise_saved_bytes(const crf_block_desc& d);
 size_t precise_bwd_bytes(const crf_block_desc& d);
