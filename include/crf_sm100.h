@@ -309,6 +309,27 @@ int crf_colsum_bf16(const void* g, float* out, int T, int N, int device, void* s
 /* f32 -> bf16 contiguous */
 int crf_cast_bf16(const float* src, void* dst, int64_t n, int device, void* stream);
 
+/* Training-mode BatchNorm2d + activation over a channels-last bf16 map x, viewed as (T, C) rows (T = B H W >= 2,
+ * C % 8 == 0), two kernels each way.  Results follow torch's act(F.batch_norm(x, ..., training=True)) with fp32
+ * parameters: the BN output is rounded to bf16 before the activation; only the fp32 summation order differs.
+ *   crf_bn_fwd: y = act(bf16(w (x - mean) invstd + b)) (bf16, like x); writes save_mean / save_invstd (fp32, C), updates
+ *     running_mean / running_var (unbiased variance) with `momentum` and adds 1 to the int64 num_batches_tracked.
+ *   crf_bn_bwd: dx (bf16) from dy (bf16) and the saved statistics, with the BN output recomputed from x; writes
+ *     dweight / dbias (fp32, C).
+ * workspace: at least crf_bn_workspace_bytes(T, C, device) bytes, 16-byte aligned, contents don't-care.  tickets: at
+ * least C / 8 int32 counters, zero before the first call; every call leaves them zero again (CUDA-graph replay safe).
+ * One tickets buffer must not serve two calls in flight at once.  x, y, dy, dx: 16-byte aligned, row-contiguous. */
+#define CRF_ACT_NONE 0
+#define CRF_ACT_RELU 1
+#define CRF_ACT_HARDSWISH 2
+size_t crf_bn_workspace_bytes(int T, int C, int device);
+int crf_bn_fwd(const void* x, void* y, const float* weight, const float* bias, float* running_mean, float* running_var,
+               long long* num_batches_tracked, float* save_mean, float* save_invstd, int T, int C, float eps,
+               float momentum, int act, void* workspace, size_t workspace_bytes, int* tickets, int device, void* stream);
+int crf_bn_bwd(const void* x, const void* dy, const float* weight, const float* bias, const float* save_mean,
+               const float* save_invstd, void* dx, float* dweight, float* dbias, int T, int C, int act, void* workspace,
+               size_t workspace_bytes, int* tickets, int device, void* stream);
+
 /* Window-attention core (everything between the qk projection and the output projection).
  *   qk   bf16 (T, 2C): q already multiplied by scale (cols [0,C)), k (cols [C,2C))
  *   vb   bf16 (T, C)

@@ -23,6 +23,8 @@ EPI_BIAS_GELU = 3
 EPI_MUL_DGELU = 4
 EPI_SPLITK_F32 = 5
 
+ACT_NONE, ACT_RELU, ACT_HARDSWISH = 0, 1, 2   # crf_bn_fwd / crf_bn_bwd activation
+
 # every symbol include/crf_sm100.h declares (checked by tests/test_abi.py)
 EXPORTED_SYMBOLS = (
     "crf_last_error", "crf_abi_version", "crf_kernel_launches", "crf_timing_enable", "crf_timing_report", "crf_block_sizes", "crf_block_fwd", "crf_block_bwd", "crf_convert_v",
@@ -30,6 +32,7 @@ EXPORTED_SYMBOLS = (
     "crf_window_gather", "crf_window_scatter", "crf_shift_mask", "crf_gemm", "crf_mlp_fwd", "crf_gemm_workspace_bytes", "crf_ln_fwd", "crf_ln_bwd", "crf_dgrad_ln_bwd",
     "crf_layernorm_fwd", "crf_layernorm_bwd", "crf_layernorm_ps_fwd", "crf_layernorm_ps_bwd", "crf_depth_loss_fwd", "crf_depth_loss_bwd", "crf_pixel_shuffle_nhwc",
     "crf_colsum_bf16", "crf_cast_bf16", "crf_attn_fwd", "crf_attn_bwd", "crf_adam_step",
+    "crf_bn_workspace_bytes", "crf_bn_fwd", "crf_bn_bwd",
 )
 
 
@@ -136,8 +139,13 @@ def _declare(lib):
     lib.crf_adam_step.argtypes = [C.POINTER(AdamTensor), i32, i32, f64, f64, f64, f64, f64, vp, i32, vp]
     lib.crf_attn_fwd.argtypes = [C.POINTER(BlockDesc), vp, vp, vp, f32, vp, vp, i32, vp, vp, vp]
     lib.crf_attn_bwd.argtypes = [C.POINTER(BlockDesc), vp, vp, vp, f32, vp, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp]
+    lib.crf_bn_workspace_bytes.restype = sz
+    lib.crf_bn_workspace_bytes.argtypes = [i32, i32, i32]
+    lib.crf_bn_fwd.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, f32, f32, i32, vp, sz, vp, i32, vp]
+    lib.crf_bn_bwd.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, sz, vp, i32, vp]
     for name in EXPORTED_SYMBOLS:
-        if name not in ("crf_last_error", "crf_kernel_launches", "crf_timing_report", "crf_gemm_workspace_bytes"):
+        if name not in ("crf_last_error", "crf_kernel_launches", "crf_timing_report", "crf_gemm_workspace_bytes",
+                        "crf_bn_workspace_bytes"):
             getattr(lib, name).restype = i32
     lib.crf_kernel_launches.restype = C.c_longlong
     lib.crf_kernel_launches.argtypes = []

@@ -619,6 +619,19 @@ int crf_cast_bf16(const float* src, void* dst, int64_t n, int device, void* stre
   CRF_CHECK(guard.ok, "cannot select device %d", device);
   return launch_cast_bf16(src, dst, n, static_cast<cudaStream_t>(stream));
 }
+size_t crf_bn_workspace_bytes(int T, int C, int device) { return bn_workspace_bytes(T, C, device); }
+int crf_bn_fwd(const void* x, void* y, const float* weight, const float* bias, float* running_mean, float* running_var,
+               long long* num_batches_tracked, float* save_mean, float* save_invstd, int T, int C, float eps,
+               float momentum, int act, void* workspace, size_t workspace_bytes, int* tickets, int device, void* stream) {
+  return launch_bn_fwd(x, y, weight, bias, running_mean, running_var, num_batches_tracked, save_mean, save_invstd, T, C,
+                       eps, momentum, act, workspace, workspace_bytes, tickets, device, static_cast<cudaStream_t>(stream));
+}
+int crf_bn_bwd(const void* x, const void* dy, const float* weight, const float* bias, const float* save_mean,
+               const float* save_invstd, void* dx, float* dweight, float* dbias, int T, int C, int act, void* workspace,
+               size_t workspace_bytes, int* tickets, int device, void* stream) {
+  return launch_bn_bwd(x, dy, weight, bias, save_mean, save_invstd, dx, dweight, dbias, T, C, act, workspace,
+                       workspace_bytes, tickets, device, static_cast<cudaStream_t>(stream));
+}
 
 int crf_attn_fwd(const crf_block_desc* d, const void* qk, const void* vb, const float* qk_bias, float scale,
                  const float* rpb_table, const float* mask, int mask_windows, void* o, float* lse, void* stream) {

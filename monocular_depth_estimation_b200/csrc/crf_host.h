@@ -154,6 +154,15 @@ int launch_pixel_shuffle_nhwc(const void* src, void* dst, int dtype, int B, int 
 int launch_adam_step(const crf_adam_tensor* tensors, int n_tensors, int chunk_elems, double lr, double b1, double b2,
                      double eps, double wd, float* step, cudaStream_t st);
 int launch_colsum_bf16(const void* g, float* out, int T, int N, cudaStream_t st);
+// crf_bn.cu: training-mode BatchNorm + activation on channels-last bf16 maps (include/crf_sm100.h: crf_bn_fwd / _bwd)
+size_t bn_workspace_bytes(int T, int C, int device);
+int launch_bn_fwd(const void* x, void* y, const float* weight, const float* bias, float* running_mean,
+                  float* running_var, long long* num_batches_tracked, float* save_mean, float* save_invstd, int T, int C,
+                  float eps, float momentum, int act, void* ws, size_t ws_bytes, int* tickets, int device,
+                  cudaStream_t st);
+int launch_bn_bwd(const void* x, const void* dy, const float* weight, const float* bias, const float* save_mean,
+                  const float* save_invstd, void* dx, float* dweight, float* dbias, int T, int C, int act, void* ws,
+                  size_t ws_bytes, int* tickets, int device, cudaStream_t st);
 int launch_cast_bf16(const float* src, void* dst, int64_t n, cudaStream_t st);
 int launch_cast4_bf16(const float* const src[4], void* const dst[4], const long long n[4], cudaStream_t st);
 int launch_convert_tokens(const void* src, int dtype, int64_t sb, int64_t st_, int64_t sc, int B, int T_img, int C,

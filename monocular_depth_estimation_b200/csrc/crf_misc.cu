@@ -8,6 +8,7 @@
 #include <algorithm>
 
 #include "crf_host.h"
+#include "crf_colreduce.cuh"
 #include "crf_ptx.cuh"
 #include "crf_window.cuh"
 
@@ -278,54 +279,34 @@ ln_bwd_kernel(const TG* __restrict__ g, const float* __restrict__ x, const float
 }
 
 // ------------------------------------------------------------------------------------------------
-// out[n] += sum_t g[t,n], g bf16 (T,N).  Thread owns eight adjacent columns (one 16-byte load per row) and keeps eight
-// rows in flight (128 B per thread, 32 KB per CTA); a CTA covers up to 2048 columns x a row chunk, the row lanes are
-// combined through shared memory, then two vector reductions per thread of row lane 0.  Two CTAs per SM: the atomics at
-// the end are per CTA, so more CTAs cost more than they hide (6 CTAs per SM: 2.5x slower at N >= 256, measured).
+// out[n] += sum_t g[t,n], g bf16 (T,N), on the shared column reduction (crf_colreduce.cuh): eight rows in flight (128 B
+// per thread, 32 KB per CTA); a CTA covers up to 2048 columns x a row chunk, then two vector reductions per thread of
+// row lane 0.  Two CTAs per SM: the atomics at the end are per CTA, so more CTAs cost more than they hide (6 CTAs per
+// SM: 2.5x slower at N >= 256, measured).
 // ------------------------------------------------------------------------------------------------
+struct ColSumOp {
+  static constexpr int kAcc = 1;
+  static constexpr int kRows = 8;
+  using Regs = uint4;
+  const __nv_bfloat16* __restrict__ g;
+  __device__ __forceinline__ uint4 load(int64_t off) const { return __ldg(reinterpret_cast<const uint4*>(g + off)); }
+  __device__ __forceinline__ void add(const uint4& w, float (&s)[1][8]) const {
+    float v[8];
+    unpack_bf16x8(w, v);
+#pragma unroll
+    for (int k = 0; k < 8; ++k) s[0][k] += v[k];
+  }
+};
+
 __global__ void __launch_bounds__(256)
 colsum_bf16_kernel(const __nv_bfloat16* __restrict__ g, float* __restrict__ out, int T, int N, int rows_per_cta) {
   pdl_prologue();
-  __shared__ __align__(16) float red[256][8];
   const int c = (blockIdx.x * blockDim.x + threadIdx.x) * 8;
   const int r0 = blockIdx.y * rows_per_cta;
-  const int r1 = min(T, r0 + rows_per_cta);
-  float s[8];
-#pragma unroll
-  for (int k = 0; k < 8; ++k) s[k] = 0.f;
-  if (c < N) {
-    const int by = blockDim.y;
-    const int64_t step = static_cast<int64_t>(by) * N;
-    const __nv_bfloat16* p = g + static_cast<int64_t>(r0 + threadIdx.y) * N + c;
-    int r = r0 + threadIdx.y;
-    for (; r + 7 * by < r1; r += 8 * by, p += 8 * step) {
-      uint4 w[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) w[u] = __ldg(reinterpret_cast<const uint4*>(p + u * step));
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        s[0] += bf16_lo(w[u].x); s[1] += bf16_hi(w[u].x); s[2] += bf16_lo(w[u].y); s[3] += bf16_hi(w[u].y);
-        s[4] += bf16_lo(w[u].z); s[5] += bf16_hi(w[u].z); s[6] += bf16_lo(w[u].w); s[7] += bf16_hi(w[u].w);
-      }
-    }
-    for (; r < r1; r += by, p += step) {
-      const uint4 w = __ldg(reinterpret_cast<const uint4*>(p));
-      s[0] += bf16_lo(w.x); s[1] += bf16_hi(w.x); s[2] += bf16_lo(w.y); s[3] += bf16_hi(w.y);
-      s[4] += bf16_lo(w.z); s[5] += bf16_hi(w.z); s[6] += bf16_lo(w.w); s[7] += bf16_hi(w.w);
-    }
-  }
-  const int tid = threadIdx.y * blockDim.x + threadIdx.x;
-  *reinterpret_cast<float4*>(&red[tid][0]) = make_float4(s[0], s[1], s[2], s[3]);
-  *reinterpret_cast<float4*>(&red[tid][4]) = make_float4(s[4], s[5], s[6], s[7]);
-  __syncthreads();
+  float s[1][8];
+  colreduce_cta(ColSumOp{g}, c, N, r0, min(T, r0 + rows_per_cta), s);
   if (threadIdx.y == 0 && c < N) {
-    float4 a = make_float4(s[0], s[1], s[2], s[3]), b = make_float4(s[4], s[5], s[6], s[7]);
-    for (int y = 1; y < blockDim.y; ++y) {
-      const float4 p = *reinterpret_cast<const float4*>(&red[y * blockDim.x + threadIdx.x][0]);
-      const float4 q = *reinterpret_cast<const float4*>(&red[y * blockDim.x + threadIdx.x][4]);
-      a.x += p.x; a.y += p.y; a.z += p.z; a.w += p.w;
-      b.x += q.x; b.y += q.y; b.z += q.z; b.w += q.w;
-    }
+    const float4 a = make_float4(s[0][0], s[0][1], s[0][2], s[0][3]), b = make_float4(s[0][4], s[0][5], s[0][6], s[0][7]);
     if ((reinterpret_cast<uintptr_t>(out) & 15) == 0) {
       red_add_f32x4(out + c, a);
       red_add_f32x4(out + c + 4, b);

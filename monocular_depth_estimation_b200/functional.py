@@ -462,3 +462,57 @@ def window_attention(x, v, qk_w, qk_b, table, proj_w, proj_b, num_heads, scale, 
     if not x.is_cuda:
         raise RuntimeError("monocular_depth_estimation_b200 runs on CUDA (sm_100a) only; there is no CPU path")
     return _WindowAttentionFn.apply(x, v, mask, num_heads, float(scale), qk_w, qk_b, table, proj_w, proj_b)
+
+
+_ACT_CODES = {None: L.ACT_NONE, "relu": L.ACT_RELU, "hardswish": L.ACT_HARDSWISH}
+
+
+class _BatchNormActFn(torch.autograd.Function):
+    """Training-mode BatchNorm2d + activation over a channels-last bf16 map on the library (crf_bn_fwd / crf_bn_bwd):
+    two kernels each way.  Saves x and the batch statistics only; the BN output the activation's backward needs is
+    recomputed from them."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias, running_mean, running_var, num_batches_tracked, tickets, eps, momentum, act):
+        B, Cd, H, W = x.shape
+        T, dev = B * H * W, x.device
+        xd = x.detach()
+        w, b = weight.detach(), bias.detach()
+        y = torch.empty_like(xd)                        # channels-last, like x
+        stats = torch.empty(2, Cd, dtype=torch.float32, device=dev)   # save_mean, save_invstd
+        ws_bytes = L.lib().crf_bn_workspace_bytes(T, Cd, dev.index)
+        ws = _alloc_bytes(ws_bytes, dev)
+        L.check(L.lib().crf_bn_fwd(xd.data_ptr(), y.data_ptr(), w.data_ptr(), b.data_ptr(), running_mean.data_ptr(),
+                                   running_var.data_ptr(), num_batches_tracked.data_ptr(), stats[0].data_ptr(),
+                                   stats[1].data_ptr(), T, Cd, float(eps), float(momentum), act, ws.data_ptr(),
+                                   ws_bytes, tickets.data_ptr(), dev.index, _stream_ptr(dev)), "crf_bn_fwd")
+        _check_guard(ws, ws_bytes, "crf_bn_fwd workspace")
+        ctx.save_for_backward(xd, w, b, stats)
+        ctx.tickets, ctx.act = tickets, act
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        xd, w, b, stats = ctx.saved_tensors
+        B, Cd, H, W = xd.shape
+        T, dev = B * H * W, xd.device
+        dy = dy.to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
+        dx = torch.empty_like(xd)
+        dwb = torch.empty(2, Cd, dtype=torch.float32, device=dev)
+        ws_bytes = L.lib().crf_bn_workspace_bytes(T, Cd, dev.index)
+        ws = _alloc_bytes(ws_bytes, dev)
+        L.check(L.lib().crf_bn_bwd(xd.data_ptr(), dy.data_ptr(), w.data_ptr(), b.data_ptr(), stats[0].data_ptr(),
+                                   stats[1].data_ptr(), dx.data_ptr(), dwb[0].data_ptr(), dwb[1].data_ptr(), T, Cd,
+                                   ctx.act, ws.data_ptr(), ws_bytes, ctx.tickets.data_ptr(), dev.index,
+                                   _stream_ptr(dev)), "crf_bn_bwd")
+        _check_guard(ws, ws_bytes, "crf_bn_bwd workspace")
+        return dx, dwb[0], dwb[1], None, None, None, None, None, None, None
+
+
+def batch_norm_act(x, weight, bias, running_mean, running_var, num_batches_tracked, tickets, eps, momentum, act=None):
+    """act(F.batch_norm(x, running_mean, running_var, weight, bias, training=True, momentum, eps)) for a CUDA bf16
+    channels-last (B, C, H, W) map, C % 8 == 0, B H W >= 2, fp32 parameters and running statistics; act is None, "relu"
+    or "hardswish".  Updates the running statistics and adds 1 to num_batches_tracked on the device.  tickets: int32,
+    at least C / 8 zeros, owned by the caller and used by one call at a time."""
+    return _BatchNormActFn.apply(x, weight, bias, running_mean, running_var, num_batches_tracked, tickets, eps,
+                                 momentum, _ACT_CODES[act])

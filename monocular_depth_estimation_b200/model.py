@@ -42,14 +42,82 @@ class Decoder(nn.Module):
         return F.interpolate(d, scale_factor=4, mode="bilinear", align_corners=False)
 
 
+_ACTS = {"relu": nn.ReLU, "hardswish": nn.Hardswish}
+_ACT_FNS = {"relu": F.relu, "hardswish": F.hardswish}
+
+
+class BatchNormAct2d(nn.BatchNorm2d):
+    """nn.BatchNorm2d followed by an activation (act: None, "relu" or "hardswish"), with nn.BatchNorm2d's parameters,
+    buffers and state_dict.  In training mode on a CUDA bf16 channels-last map with C % 8 == 0 it runs on the library's
+    BatchNorm kernels (functional.batch_norm_act: two launches each way, only x and the statistics saved for the
+    backward); every other case runs act(nn.BatchNorm2d.forward(x)) unchanged."""
+
+    def __init__(self, num_features, eps=1e-5, momentum=0.1, affine=True, track_running_stats=True, act=None,
+                 device=None, dtype=None):
+        super().__init__(num_features, eps, momentum, affine, track_running_stats, device, dtype)
+        if act not in (None, *_ACTS):
+            raise ValueError(f"act must be None, 'relu' or 'hardswish' (got {act!r})")
+        self.act = act
+        self._tickets = None   # the kernels' per-launch counters (not state: always zero between launches)
+
+    @classmethod
+    def from_batchnorm(cls, bn, act=None):
+        """A BatchNormAct2d that holds bn's own parameter and buffer tensors (shared, not copied)."""
+        m = cls(bn.num_features, bn.eps, bn.momentum, bn.affine, bn.track_running_stats, act=act, device="meta")
+        m._parameters.update(bn._parameters)
+        m._buffers.update(bn._buffers)
+        m.train(bn.training)
+        return m
+
+    def _library(self, x):
+        return (self.training and self.track_running_stats and self.affine and isinstance(self.momentum, float)
+                and x.is_cuda and x.dtype == torch.bfloat16 and x.dim() == 4
+                and x.is_contiguous(memory_format=torch.channels_last) and x.data_ptr() % 16 == 0
+                and x.shape[1] % 8 == 0 and x.shape[0] * x.shape[2] * x.shape[3] >= 2
+                and self.weight.dtype == torch.float32 and self.running_mean.dtype == torch.float32)
+
+    def forward(self, x):
+        if self._library(x):
+            from .functional import batch_norm_act
+            if self._tickets is None or self._tickets.device != x.device:
+                self._tickets = torch.zeros(self.num_features // 8, dtype=torch.int32, device=x.device)
+            return batch_norm_act(x, self.weight, self.bias, self.running_mean, self.running_var,
+                                  self.num_batches_tracked, self._tickets, self.eps, self.momentum, self.act)
+        y = super().forward(x)
+        return y if self.act is None else _ACT_FNS[self.act](y, inplace=True)   # as torchvision's inplace modules
+
+    def extra_repr(self):
+        return super().extra_repr() + f", act={self.act}"
+
+
+def fuse_batchnorm_act(features):
+    """Replaces, inside every torchvision Conv2dNormActivation of `features`, the BatchNorm2d (index 1) by a
+    BatchNormAct2d holding the same tensors and the ReLU / Hardswish after it (index 2) by nn.Identity.  Keys, shapes and
+    dtypes of the state_dict stay torchvision's."""
+    from torchvision.ops.misc import Conv2dNormActivation
+    for mod in features.modules():
+        if not isinstance(mod, Conv2dNormActivation) or type(mod[1]) is not nn.BatchNorm2d:
+            continue
+        act = None
+        if len(mod) > 2:
+            act = next((k for k, cls in _ACTS.items() if type(mod[2]) is cls), None)
+            if act is None:
+                continue
+            mod[2] = nn.Identity()
+        mod[1] = BatchNormAct2d.from_batchnorm(mod[1], act)
+    return features
+
+
 class Encoder(nn.Module):
-    """torchvision MobileNetV3-large feature stack; keeps every intermediate map (18 tensors incl. the input)."""
+    """torchvision MobileNetV3-large feature stack; keeps every intermediate map (18 tensors incl. the input).  Its 46
+    BatchNorm layers, with the activation that follows each, are BatchNormAct2d modules."""
 
     def __init__(self, pretrained=False):
         super().__init__()
         import torchvision.models as tvm
         weights = tvm.MobileNet_V3_Large_Weights.IMAGENET1K_V1 if pretrained else None
         self.original_model = tvm.mobilenet_v3_large(weights=weights)
+        fuse_batchnorm_act(self.original_model.features)
 
     def forward(self, x):
         feats = [x]
