@@ -330,6 +330,26 @@ int crf_bn_bwd(const void* x, const void* dy, const float* weight, const float* 
                const float* save_invstd, void* dx, float* dweight, float* dbias, int T, int C, int act, void* workspace,
                size_t workspace_bytes, int* tickets, int device, void* stream);
 
+/* Depthwise convolution nn.Conv2d(C, C, k, stride, padding=k // 2, groups=C, bias=False) over a channels-last bf16 map
+ * x viewed as (B, H, W, C), k = 3 or 5, stride = 1 or 2, C % 8 == 0; the output is (B, Ho, Wo, C) with
+ * Ho = (H - 1) / stride + 1, Wo = (W - 1) / stride + 1.  Results follow torch's conv2d under bf16 autocast: the fp32
+ * weight (C, 1, k, k), contiguous, is rounded to bf16 on load; only the fp32 summation order differs.  No atomics: every
+ * result is bit-reproducible from run to run.
+ *   crf_dwconv_fwd: y (bf16): each output one fp32 sum of bf16 products in a fixed tap order, rounded once.
+ *   crf_dwconv_bwd: dx (bf16, like x) and dweight (fp32 (C, 1, k, k), contiguous: summed in fp32 partials and double,
+ *     rounded to bf16 and widened, as cuDNN's bf16 weight gradient cast back to fp32) from dy (bf16, like y).  Either
+ *     of dx and dweight may be NULL when that gradient is not needed; workspace and tickets serve dweight only.
+ * workspace: at least crf_dwconv_workspace_bytes(B, H, W, C, k, stride, device) bytes, 16-byte aligned, contents
+ * don't-care.  tickets: at least k * C / 8 int32 counters, zero before the first call; every call leaves them zero
+ * again (CUDA-graph replay safe).  One tickets buffer must not serve two calls in flight at once.  x, y, dy, dx: 16-byte
+ * aligned, contiguous. */
+size_t crf_dwconv_workspace_bytes(int B, int H, int W, int C, int k, int stride, int device);
+int crf_dwconv_fwd(const void* x, const float* weight, void* y, int B, int H, int W, int C, int k, int stride, int device,
+                   void* stream);
+int crf_dwconv_bwd(const void* x, const float* weight, const void* dy, void* dx, float* dweight, int B, int H, int W,
+                   int C, int k, int stride, void* workspace, size_t workspace_bytes, int* tickets, int device,
+                   void* stream);
+
 /* Window-attention core (everything between the qk projection and the output projection).
  *   qk   bf16 (T, 2C): q already multiplied by scale (cols [0,C)), k (cols [C,2C))
  *   vb   bf16 (T, C)

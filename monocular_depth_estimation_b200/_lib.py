@@ -33,6 +33,7 @@ EXPORTED_SYMBOLS = (
     "crf_layernorm_fwd", "crf_layernorm_bwd", "crf_layernorm_ps_fwd", "crf_layernorm_ps_bwd", "crf_depth_loss_fwd", "crf_depth_loss_bwd", "crf_pixel_shuffle_nhwc",
     "crf_colsum_bf16", "crf_cast_bf16", "crf_attn_fwd", "crf_attn_bwd", "crf_adam_step",
     "crf_bn_workspace_bytes", "crf_bn_fwd", "crf_bn_bwd",
+    "crf_dwconv_workspace_bytes", "crf_dwconv_fwd", "crf_dwconv_bwd",
 )
 
 
@@ -143,9 +144,13 @@ def _declare(lib):
     lib.crf_bn_workspace_bytes.argtypes = [i32, i32, i32]
     lib.crf_bn_fwd.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, f32, f32, i32, vp, sz, vp, i32, vp]
     lib.crf_bn_bwd.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, sz, vp, i32, vp]
+    lib.crf_dwconv_workspace_bytes.restype = sz
+    lib.crf_dwconv_workspace_bytes.argtypes = [i32, i32, i32, i32, i32, i32, i32]
+    lib.crf_dwconv_fwd.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp]
+    lib.crf_dwconv_bwd.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, sz, vp, i32, vp]
     for name in EXPORTED_SYMBOLS:
         if name not in ("crf_last_error", "crf_kernel_launches", "crf_timing_report", "crf_gemm_workspace_bytes",
-                        "crf_bn_workspace_bytes"):
+                        "crf_bn_workspace_bytes", "crf_dwconv_workspace_bytes"):
             getattr(lib, name).restype = i32
     lib.crf_kernel_launches.restype = C.c_longlong
     lib.crf_kernel_launches.argtypes = []

@@ -632,6 +632,19 @@ int crf_bn_bwd(const void* x, const void* dy, const float* weight, const float* 
   return launch_bn_bwd(x, dy, weight, bias, save_mean, save_invstd, dx, dweight, dbias, T, C, act, workspace,
                        workspace_bytes, tickets, device, static_cast<cudaStream_t>(stream));
 }
+size_t crf_dwconv_workspace_bytes(int B, int H, int W, int C, int k, int stride, int device) {
+  return dwconv_workspace_bytes(B, H, W, C, k, stride, device);
+}
+int crf_dwconv_fwd(const void* x, const float* weight, void* y, int B, int H, int W, int C, int k, int stride, int device,
+                   void* stream) {
+  return launch_dwconv_fwd(x, weight, y, B, H, W, C, k, stride, device, static_cast<cudaStream_t>(stream));
+}
+int crf_dwconv_bwd(const void* x, const float* weight, const void* dy, void* dx, float* dweight, int B, int H, int W,
+                   int C, int k, int stride, void* workspace, size_t workspace_bytes, int* tickets, int device,
+                   void* stream) {
+  return launch_dwconv_bwd(x, weight, dy, dx, dweight, B, H, W, C, k, stride, workspace, workspace_bytes, tickets,
+                           device, static_cast<cudaStream_t>(stream));
+}
 
 int crf_attn_fwd(const crf_block_desc* d, const void* qk, const void* vb, const float* qk_bias, float scale,
                  const float* rpb_table, const float* mask, int mask_windows, void* o, float* lse, void* stream) {

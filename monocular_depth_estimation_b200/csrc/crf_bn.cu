@@ -6,10 +6,7 @@
 // expressions follow ATen's channels-last kernels (Normalization.cuh) and its ReLU / Hardswish backward.  What remains
 // different from torch is the fp32 summation order of the reductions.
 //
-// The two reductions run on the shared column reduction (crf_colreduce.cuh).  Every CTA writes its per-column partial
-// sums to the workspace and takes a ticket from its column group's counter; the last CTA of a group sums the partials in
-// double, in a fixed order, and finalises the group's channels.  It resets the counter, so the next launch (or CUDA-graph
-// replay) starts from zero; no CTA waits for another.
+// The two reductions run on the shared column reduction and its ticketed finalisation (crf_colreduce.cuh).
 #include <algorithm>
 
 #include "crf_host.h"
@@ -100,79 +97,6 @@ struct BwdOp {
     }
   }
 };
-
-// part[(a * gridDim.y + blockIdx.y) * C + c]: accumulator a of the CTA's row block
-template <int NACC>
-__device__ __forceinline__ void store_partials(float* __restrict__ part, const float (&s)[NACC][8], int c, int C) {
-  if (threadIdx.y != 0 || c >= C) return;
-#pragma unroll
-  for (int a = 0; a < NACC; ++a) {
-    float* dst = part + (static_cast<int64_t>(a) * gridDim.y + blockIdx.y) * C + c;
-    *reinterpret_cast<float4*>(dst) = make_float4(s[a][0], s[a][1], s[a][2], s[a][3]);
-    *reinterpret_cast<float4*>(dst + 4) = make_float4(s[a][4], s[a][5], s[a][6], s[a][7]);
-  }
-}
-
-// True in the CTA that arrives last of its column group (blockIdx.x); that CTA resets the group's counter.
-__device__ __forceinline__ bool last_of_column_group(int* tickets) {
-  __shared__ bool last;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0 && threadIdx.y == 0) {
-    last = atomicAdd(tickets + blockIdx.x, 1) == static_cast<int>(gridDim.y) - 1;
-    if (last) tickets[blockIdx.x] = 0;
-  }
-  __syncthreads();
-  if (last) __threadfence();
-  return last;
-}
-
-// In the last CTA of a column group: sums each column's NACC partials over the grid's row blocks in double -- thread
-// slices take every slices-th row block, then slice 0 adds the slices in order -- and calls f(c, sums) once per column.
-template <int NACC, typename F>
-__device__ __forceinline__ void finalize_columns(const float* part, int C, F&& f) {
-  __shared__ double red[256][NACC];
-  const int c0 = blockIdx.x * blockDim.x * 8;
-  const int ncol = min(static_cast<int>(blockDim.x) * 8, C - c0);
-  const int nthr = blockDim.x * blockDim.y;
-  const int slices = nthr / ncol;  // >= 4: at most 64 columns per group
-  const int tid = threadIdx.y * blockDim.x + threadIdx.x;
-  const int col = tid % ncol, sl = tid / ncol;
-  double acc[NACC];
-#pragma unroll
-  for (int a = 0; a < NACC; ++a) acc[a] = 0.0;
-  if (sl < slices) {
-    const int gy = gridDim.y;
-    const float* p = part + c0 + col;
-    auto at = [&](int a, int y) { return __ldcg(p + (static_cast<int64_t>(a) * gy + y) * C); };
-    int y = sl;
-    for (; y + 7 * slices < gy; y += 8 * slices) {  // eight row blocks' loads in flight, added in row-block order
-      float v[8][NACC];
-#pragma unroll
-      for (int u = 0; u < 8; ++u)
-#pragma unroll
-        for (int a = 0; a < NACC; ++a) v[u][a] = at(a, y + u * slices);
-#pragma unroll
-      for (int u = 0; u < 8; ++u)
-#pragma unroll
-        for (int a = 0; a < NACC; ++a) acc[a] += v[u][a];
-    }
-    for (; y < gy; y += slices) {
-#pragma unroll
-      for (int a = 0; a < NACC; ++a) acc[a] += at(a, y);
-    }
-  }
-#pragma unroll
-  for (int a = 0; a < NACC; ++a) red[tid][a] = acc[a];
-  __syncthreads();
-  if (tid < ncol) {
-    for (int s = 1; s < slices; ++s) {
-#pragma unroll
-      for (int a = 0; a < NACC; ++a) acc[a] += red[s * ncol + tid][a];
-    }
-    f(c0 + tid, acc);
-  }
-}
 
 __global__ void __launch_bounds__(256)
 bn_stats_kernel(const __nv_bfloat16* __restrict__ x, int T, int C, int rows_per_cta, float* __restrict__ part,

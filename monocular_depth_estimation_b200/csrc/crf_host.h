@@ -163,6 +163,12 @@ int launch_bn_fwd(const void* x, void* y, const float* weight, const float* bias
 int launch_bn_bwd(const void* x, const void* dy, const float* weight, const float* bias, const float* save_mean,
                   const float* save_invstd, void* dx, float* dweight, float* dbias, int T, int C, int act, void* ws,
                   size_t ws_bytes, int* tickets, int device, cudaStream_t st);
+// crf_dwconv.cu: depthwise 3x3 / 5x5 convolutions on channels-last bf16 maps (include/crf_sm100.h: crf_dwconv_*)
+size_t dwconv_workspace_bytes(int B, int H, int W, int C, int k, int stride, int device);
+int launch_dwconv_fwd(const void* x, const float* weight, void* y, int B, int H, int W, int C, int k, int stride,
+                      int device, cudaStream_t st);
+int launch_dwconv_bwd(const void* x, const float* weight, const void* dy, void* dx, float* dweight, int B, int H, int W,
+                      int C, int k, int stride, void* ws, size_t ws_bytes, int* tickets, int device, cudaStream_t st);
 int launch_cast_bf16(const float* src, void* dst, int64_t n, cudaStream_t st);
 int launch_cast4_bf16(const float* const src[4], void* const dst[4], const long long n[4], cudaStream_t st);
 int launch_convert_tokens(const void* src, int dtype, int64_t sb, int64_t st_, int64_t sc, int B, int T_img, int C,

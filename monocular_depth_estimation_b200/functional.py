@@ -516,3 +516,50 @@ def batch_norm_act(x, weight, bias, running_mean, running_var, num_batches_track
     at least C / 8 zeros, owned by the caller and used by one call at a time."""
     return _BatchNormActFn.apply(x, weight, bias, running_mean, running_var, num_batches_tracked, tickets, eps,
                                  momentum, _ACT_CODES[act])
+
+
+class _DepthwiseConvFn(torch.autograd.Function):
+    """Depthwise conv2d (groups == C, k = 3 or 5, stride 1 or 2, padding k // 2, no bias) over a channels-last bf16 map
+    on the library (crf_dwconv_fwd / crf_dwconv_bwd), with the fp32 weight rounded to bf16 inside the kernels as
+    autocast's cast would.  One kernel forward; backward one per requested gradient.  Saves x and the weight only."""
+
+    @staticmethod
+    def forward(ctx, x, weight, stride, tickets):
+        B, Cd, H, W = x.shape
+        k = weight.shape[-1]
+        dev = x.device
+        xd, w = x.detach(), weight.detach()
+        Ho, Wo = (H - 1) // stride + 1, (W - 1) // stride + 1
+        y = torch.empty(B, Cd, Ho, Wo, dtype=torch.bfloat16, device=dev, memory_format=torch.channels_last)
+        L.check(L.lib().crf_dwconv_fwd(xd.data_ptr(), w.data_ptr(), y.data_ptr(), B, H, W, Cd, k, stride, dev.index,
+                                       _stream_ptr(dev)), "crf_dwconv_fwd")
+        ctx.save_for_backward(xd, w)
+        ctx.stride, ctx.tickets = stride, tickets
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        xd, w = ctx.saved_tensors
+        B, Cd, H, W = xd.shape
+        k, dev = w.shape[-1], xd.device
+        dy = dy.to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
+        dx = torch.empty_like(xd) if ctx.needs_input_grad[0] else None
+        dw = torch.empty_strided(w.shape, w.stride(), dtype=torch.float32, device=dev) if ctx.needs_input_grad[1] else None
+        ws_bytes = L.lib().crf_dwconv_workspace_bytes(B, H, W, Cd, k, ctx.stride, dev.index) if dw is not None else 0
+        ws = _alloc_bytes(ws_bytes, dev) if dw is not None else None
+        L.check(L.lib().crf_dwconv_bwd(xd.data_ptr(), w.data_ptr(), dy.data_ptr(),
+                                       None if dx is None else dx.data_ptr(), None if dw is None else dw.data_ptr(),
+                                       B, H, W, Cd, k, ctx.stride, None if ws is None else ws.data_ptr(), ws_bytes,
+                                       ctx.tickets.data_ptr(), dev.index, _stream_ptr(dev)), "crf_dwconv_bwd")
+        if ws is not None:
+            _check_guard(ws, ws_bytes, "crf_dwconv_bwd workspace")
+        return dx, dw, None, None
+
+
+def depthwise_conv(x, weight, stride, tickets):
+    """F.conv2d(x, weight, None, stride, weight.shape[-1] // 2, groups=C) as torch computes it under bf16 autocast, for a
+    CUDA bf16 channels-last (B, C, H, W) map x with C % 8 == 0 and an fp32 (C, 1, k, k) weight with k = 3 or 5 laid out
+    (k k, -, k, 1) (contiguous or channels-last); stride 1 or 2.  Returns a bf16 channels-last map; the weight gradient is
+    fp32 with the weight's strides.  tickets: int32, at least k C / 8 zeros, owned by the caller and used by one call at
+    a time."""
+    return _DepthwiseConvFn.apply(x, weight, stride, tickets)

@@ -108,9 +108,66 @@ def fuse_batchnorm_act(features):
     return features
 
 
+class DepthwiseConv2d(nn.Conv2d):
+    """nn.Conv2d with groups == in_channels == out_channels, with nn.Conv2d's parameters and state_dict.  Under CUDA bf16
+    autocast, on a bf16 channels-last map, for the geometries of the library's depthwise kernels (k = 3 or 5, stride 1
+    or 2, padding k // 2, no bias, C % 8 == 0) it runs on them (functional.depthwise_conv: one launch forward, one per
+    gradient backward, bit-reproducible); every other case runs nn.Conv2d.forward unchanged."""
+
+    def __init__(self, *args, **kwargs):
+        super().__init__(*args, **kwargs)
+        if not (self.groups == self.in_channels == self.out_channels):
+            raise ValueError("DepthwiseConv2d needs groups == in_channels == out_channels")
+        self._tickets = None   # the weight-gradient kernel's per-launch counters (not state: zero between launches)
+
+    @classmethod
+    def from_conv(cls, conv):
+        """A DepthwiseConv2d that holds conv's own parameters (shared, not copied)."""
+        m = cls(conv.in_channels, conv.out_channels, conv.kernel_size, conv.stride, conv.padding, conv.dilation,
+                conv.groups, conv.bias is not None, conv.padding_mode, device="meta")
+        m._parameters.update(conv._parameters)
+        m.train(conv.training)
+        return m
+
+    def _library(self, x):
+        k, w = self.kernel_size[0], self.weight
+        return (torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") == torch.bfloat16
+                and x.is_cuda and x.dtype == torch.bfloat16 and x.dim() == 4
+                and x.is_contiguous(memory_format=torch.channels_last) and x.data_ptr() % 16 == 0
+                and x.shape[1] == self.in_channels and self.in_channels % 8 == 0
+                and self.kernel_size == (k, k) and k in (3, 5) and self.stride in ((1, 1), (2, 2))
+                and self.padding == (k // 2, k // 2) and self.dilation == (1, 1) and self.bias is None
+                and self.padding_mode == "zeros" and w.dtype == torch.float32 and w.device == x.device
+                and w.stride() in ((k * k, k * k, k, 1), (k * k, 1, k, 1)) and w.data_ptr() % 16 == 0)
+
+    def forward(self, x):
+        if self._library(x):
+            from .functional import depthwise_conv
+            if self._tickets is None or self._tickets.device != x.device:
+                self._tickets = torch.zeros(self.kernel_size[0] * self.in_channels // 8, dtype=torch.int32,
+                                            device=x.device)
+            return depthwise_conv(x, self.weight, self.stride[0], self._tickets)
+        return super().forward(x)
+
+
+def fuse_depthwise(features):
+    """Replaces the convolution (index 0) of every torchvision Conv2dNormActivation of `features` whose convolution is
+    depthwise (groups == in_channels == out_channels > 1) by a DepthwiseConv2d holding the same weight.  Keys, shapes and
+    dtypes of the state_dict stay torchvision's."""
+    from torchvision.ops.misc import Conv2dNormActivation
+    for mod in features.modules():
+        if not isinstance(mod, Conv2dNormActivation) or type(mod[0]) is not nn.Conv2d:
+            continue
+        c = mod[0]
+        if c.groups == c.in_channels == c.out_channels > 1:
+            mod[0] = DepthwiseConv2d.from_conv(c)
+    return features
+
+
 class Encoder(nn.Module):
     """torchvision MobileNetV3-large feature stack; keeps every intermediate map (18 tensors incl. the input).  Its 46
-    BatchNorm layers, with the activation that follows each, are BatchNormAct2d modules."""
+    BatchNorm layers, with the activation that follows each, are BatchNormAct2d modules; its 15 depthwise convolutions
+    are DepthwiseConv2d modules."""
 
     def __init__(self, pretrained=False):
         super().__init__()
@@ -118,6 +175,7 @@ class Encoder(nn.Module):
         weights = tvm.MobileNet_V3_Large_Weights.IMAGENET1K_V1 if pretrained else None
         self.original_model = tvm.mobilenet_v3_large(weights=weights)
         fuse_batchnorm_act(self.original_model.features)
+        fuse_depthwise(self.original_model.features)
 
     def forward(self, x):
         feats = [x]
